@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the DVB-S2 decode stage (BASELINE.json metric: decoded information Gbit/s, QPSK 1/2 normal).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--esn0 DB] [--pool F]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--esn0 DB] [--pool F] [--dump-outputs DIR]
 
 One "step" = R passes of the hot path (LDPC + BCH + descramble, from int8 LLRs) over a pool of F synthetic
 FECFRAMEs (defaults F = 16384, R = 5: 81920 frames per step, so that the driver's 20 steps time more than two
@@ -15,6 +15,13 @@ data-path collective; timing is barrier-bracketed and the max over ranks is used
 also drives ONE handle configured with all N devices (the in-process dispatcher the SDR++ plugin would use,
 reference batch seam module_dvbs2_demod.cpp:343-367) through decode_batch and submit/collect while the other
 ranks idle, checks its output bytes against the single-device result and reports `dispatcher`.
+
+`--dump-outputs DIR` writes, after the timed steps, what rank 0's last timed launch returned, as float32 / float64
+.npy files of at most DUMP_BYTES in all: the BBFRAME bytes of a fixed, seeded sample of DUMP_FRAMES frames
+(bbframe_bytes.npy, rows in the order of frame_index.npy) and the result records (tag.npy, ldpc_iters.npy,
+bch_corr.npy, flags.npy) of every frame, or of a seeded sample of DUMP_RECORDS frames when the pool is larger
+(record_index.npy). The inputs are generated from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 
 `--impl reference` times the reference's own CPU code (oracle/_ref, compiled from /root/reference
 unmodified; else the oracle port) on the host cores with the same pool generator and metric.
@@ -38,6 +45,14 @@ MODCOD, SHORT, RATE_ENUM = 4, False, 3  # QPSK 1/2 normal
 MAX_TRIALS = 25
 LLR_SCALE = 4.0  # "L4" generator of SURVEY.md 8d: rint(4 * true channel LLR), clamped to +-127
 HBM_BYTES_PER_FRAME = 64800 + 32208 // 8 + 16  # algorithmic: LLRs in, BBFRAME + result record out
+DUMP_FRAMES = 2048  # BBFRAMEs written by --dump-outputs: 2048 x 4026 bytes as float32 = 33 MB
+DUMP_RECORDS = 1 << 19  # result records written by --dump-outputs: 32 bytes each with their index = 16.8 MB
+DUMP_BYTES = 64 << 20
+
+
+def sorted_sample(n, k, seed):
+    """all of range(n) when it has at most k entries, else k of them drawn without replacement, ascending"""
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
 
 
 def load_peaks():
@@ -307,7 +322,12 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--parity-frames", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed launch's outputs as .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path; --impl reference has no device outputs")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -334,13 +354,11 @@ def main():
             if s >= args.warmup:
                 t_all += last["seconds"]
                 frames_all += last["frames"]
-            if s >= args.warmup and t_all > 120:
-                break
         v = frames_all * kbch / t_all / 1e9
         config = dict(config, frames_per_step_per_gpu=last["frames"], frames_per_launch=None, launches_per_step=None,
                       cache="n/a (host)", parallelism="%d host processes, 16 frames per SSE4.1 call" % procs)
         line = {"impl": "reference", "metric": "decoded_info_gbit_s", "value": v, "unit": "Gbit/s", "n_gpus": args.gpus,
-                "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * t_all / max(1, args.steps),
+                "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * t_all / args.steps,
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int8", "data": "synthetic",
                 "config": config, "frames_per_s": frames_all / t_all,
                 "cpu_baseline": {"value": v, "unit": "Gbit/s", "cores": last["cores"], "kind": last["kind"], "sample": last["sample"],
@@ -402,6 +420,17 @@ def main():
     iters = res["ldpc_iters"].astype(np.int32)
     mean_it = float(np.where(iters < 0, MAX_TRIALS, iters).mean())
     fer = float((res["bch_corr"] < 0).mean())
+    dump = None
+    if rank == 0 and args.dump_outputs:   # taken now: the parity and latency legs below reuse d_bb
+        frame_index = sorted_sample(args.pool, DUMP_FRAMES, 0)
+        record_index = sorted_sample(args.pool, DUMP_RECORDS, 1)
+        rec = res[record_index]
+        dump = {"frame_index": frame_index.astype(np.float64),
+                "bbframe_bytes": d_bb[torch.from_numpy(frame_index).to(dev)].cpu().numpy().astype(np.float32),
+                "record_index": record_index.astype(np.float64),
+                "tag": rec["tag"].astype(np.float64), "ldpc_iters": rec["ldpc_iters"].astype(np.float32),
+                "bch_corr": rec["bch_corr"].astype(np.float32), "flags": rec["flags"].astype(np.float64)}
+        assert sum(a.nbytes for a in dump.values()) <= DUMP_BYTES
 
     # ---- parity of what was just timed (outside the timed region): the slowest frames of the last launch and
     #      random ones, GPU result vs CPU oracle
@@ -435,12 +464,16 @@ def main():
         dec_e.decode_batch_raw(h_in, e2e_frames, h_bb, h_res)
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(2, min(args.steps, 8))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         dec_e.decode_batch_raw(h_in, e2e_frames, h_bb, h_res)
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
     sampler.stop()
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     # ---- what the host side can deliver at all: the same input bytes from page-locked memory, copies only, every rank at
     #      once (under torchrun the ranks share the host's memory controllers and PCIe root complexes)
     pin = torch.from_numpy(host_copy).pin_memory()
