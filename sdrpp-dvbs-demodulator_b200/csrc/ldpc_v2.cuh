@@ -16,9 +16,10 @@
 //   * link addresses are  min(x, x - 720)  in unsigned arithmetic (one VIADDMNMX.U32) instead of compare/select;
 //   * there is no "one frame finished" code path: a frame's results are written out the moment it stops and its
 //     lane simply keeps computing until the pair is done;
-//   * parity LLRs are never transposed: thread j is the only consumer of column j of the q x 360 parity matrix,
-//     which is CONTIGUOUS in the input frame (v[K + q j + i], layered_decoder.hh:124-126), so the first pass reads
-//     it straight from the input;
+//   * column j of the q x 360 parity matrix is CONTIGUOUS in the input frame (v[K + q j + i],
+//     layered_decoder.hh:124-126) and thread j is its only consumer; the pair load transposes it once, with
+//     coalesced loads and stores, into the workspace words every pass reads (layer-major, one word per row);
+//   * the next pair is claimed when the first frame of the current one stops, and its frames are prefetched into L2;
 //   * LDPCDecoder::bad is screened: after every pass thread j tests row (q-1, j), whose parity LLRs it still holds
 //     in registers; only when all 360 rows of that layer pass for a live frame does the full bit-plane test run.
 //     Any bad row makes bad() true (layered_decoder.hh:28-45), so the screen never changes a result.
@@ -241,42 +242,14 @@ __device__ __forceinline__ void harvest_planes(const uint4* src, int n360, uint3
 
 // The full LDPCDecoder::bad (layered_decoder.hh:28-45) for both frames of the pair: a row is bad when its sign product
 // is not positive, i.e. odd parity of hard decisions or any zero LLR.  Hard decisions are gathered into bit planes
-// (parity part from the workspace after a pass, straight from the input before the first one), each layer's 360
-// checks are then 12 words of rotate-and-XOR.  Returns bit f set when frame f is bad.  All threads of the CTA call it.
-template <bool STREAMED, int THREADS>
-__device__ __noinline__ int full_test(const LdpcParams2& p, bool after_pass, const uint16_t* wpty, uint32_t* HP, uint32_t* HD,
-                                      const uint4* vdata4, const int8_t* inA, const int8_t* inB, int* s_bad) {
-    const int tid = threadIdx.x, q = p.q, K = p.K;
+// (parity part from the workspace, where load_pair staged it before the first pass), each layer's 360 checks are then
+// 12 words of rotate-and-XOR.  Returns bit f set when frame f is bad.  All threads of the CTA call it.
+template <int THREADS>
+__device__ __noinline__ int full_test(const LdpcParams2& p, const uint16_t* wpty, uint32_t* HP, uint32_t* HD,
+                                      const uint4* vdata4, int* s_bad) {
+    const int tid = threadIdx.x, q = p.q;
     uint32_t nzacc = 0xFFFFFFFFu;
-    if (after_pass) {
-        harvest_planes<true, THREADS>(reinterpret_cast<const uint4*>(wpty), q, HP, q, tid, nzacc);
-    } else {
-        // parity planes straight from the input: one ballot per layer and frame (a frame that is a codeword before
-        // the first pass is the only way to get here); thread r < 360 reads column r: pty[i][r] = v[K + q r + i]
-        const int wid = tid >> 5, lane = tid & 31;
-        if (wid < 12) {
-            const bool row = tid < 360;
-            const unsigned wl = __activemask();     // (the CTA's last warp is a partial one)
-            const int8_t* ca = inA + K + (size_t)q * (row ? tid : 0);
-            const int8_t* cb = inB + K + (size_t)q * (row ? tid : 0);
-            for (int i = 0; i < q; ++i) {
-                uint32_t w = 0x8181u;
-                if (row) {
-                    const uint32_t a = STREAMED ? (uint8_t)__ldcg(ca + i) : (uint8_t)__ldg(ca + i);
-                    const uint32_t b = STREAMED ? (uint8_t)__ldcg(cb + i) : (uint8_t)__ldg(cb + i);
-                    w = (a | (b << 8)) ^ 0x8080u;
-                }
-                const unsigned ba = __ballot_sync(wl, !(w & 0x80u));
-                const unsigned bb = __ballot_sync(wl, !(w & 0x8000u));
-                if (lane == 0) {
-                    __stcg(&HP[i * kBitWords + wid], ba);
-                    __stcg(&HP[(q + i) * kBitWords + wid], bb);
-                }
-                if ((w & 0xFFu) == 0x80u) nzacc &= ~0x00800080u;
-                if ((w & 0xFF00u) == 0x8000u) nzacc &= ~0x80008000u;
-            }
-        }
-    }
+    harvest_planes<true, THREADS>(reinterpret_cast<const uint4*>(wpty), q, HP, q, tid, nzacc);
     harvest_planes<false, THREADS>(vdata4, p.ngroups, HD, p.ngroups, tid, nzacc);
     if (tid < 2) s_bad[tid] = 0;
     __syncthreads();
@@ -316,10 +289,10 @@ __device__ __noinline__ int full_test(const LdpcParams2& p, bool after_pass, con
 
 // Results of the frames that stop here (bit f of fin): iteration count, MSB-first hard decisions of the K systematic
 // bits (module_dvbs2_demod.cpp:357-360) straight from the LLR pairs (8 pairs = one uint4 give one byte of each frame),
-// optionally the posterior LLRs (what BBFrameLDPC::decode leaves in place).
+// optionally the posterior LLRs (what BBFrameLDPC::decode leaves in place; before the first pass the staged input).
 template <int THREADS>
-__device__ __noinline__ void emit_results(const LdpcParams2& p, int fin, const int (&res)[2], int fa, int fb, bool after_pass,
-                                          const uint16_t* wpty, const uint4* vdata4, const int8_t* inA, const int8_t* inB) {
+__device__ __noinline__ void emit_results(const LdpcParams2& p, int fin, const int (&res)[2], int fa, int fb,
+                                          const uint16_t* wpty, const uint4* vdata4) {
     const int tid = threadIdx.x, q = p.q, K = p.K, N = p.N, R = p.R;
     const int kbytes = K / 8;
     for (int b = tid; b < kbytes; b += THREADS) {
@@ -336,17 +309,81 @@ __device__ __noinline__ void emit_results(const LdpcParams2& p, int fin, const i
             int8_t* lo = p.llr_out + (size_t)fr * N;
             const uint8_t* vb = reinterpret_cast<const uint8_t*>(vdata4) + f;
             for (int x = tid; x < K; x += THREADS) lo[x] = (int8_t)(vb[2 * x] ^ 0x80u);
-            if (after_pass) {
-                for (int x = tid; x < R; x += THREADS) {
-                    const int jj = x / q, ii = x - jj * q;
-                    lo[K + x] = (int8_t)((__ldcg(&wpty[360 * ii + jj]) >> (8 * f)) ^ 0x80u);
-                }
-            } else {
-                const int8_t* in = f ? inB : inA;
-                for (int x = tid; x < R; x += THREADS) lo[K + x] = in[K + x];
+            for (int x = tid; x < R; x += THREADS) {
+                const int jj = x / q, ii = x - jj * q;
+                lo[K + x] = (int8_t)((__ldcg(&wpty[360 * ii + jj]) >> (8 * f)) ^ 0x80u);
             }
         }
     }
+}
+
+// 8 LLRs of frame A and the same 8 of frame B -> 8 LLR pairs in offset binary (A in the even bytes)
+__device__ __forceinline__ uint4 interleave8(uint2 a, uint2 b) {
+    uint4 o;
+    o.x = prmt(a.x, b.x, 0x5140) ^ 0x80808080u;
+    o.y = prmt(a.x, b.x, 0x7362) ^ 0x80808080u;
+    o.z = prmt(a.y, b.y, 0x5140) ^ 0x80808080u;
+    o.w = prmt(a.y, b.y, 0x7362) ^ 0x80808080u;
+    return o;
+}
+template <bool STREAMED>
+__device__ __forceinline__ uint2 ld_in8(const int8_t* frame, int x) {   // 8 bytes at frame + 8 x (frames are 8-byte aligned)
+    const uint2* s = reinterpret_cast<const uint2*>(frame) + x;
+    // streamed: the copy engine is still writing other frames of this buffer -> L2-coherent loads
+    return STREAMED ? __ldcg(s) : __ldg(s);
+}
+
+// Pair load.  Parity part: pty[i][j] = v[K + q j + i] (column j of the q x 360 parity matrix is contiguous in the
+// frame, layered_decoder.hh:124-126), and every pass reads it as wpty[i * 360 + j] (packed offset-binary pair, A in the
+// low byte), i.e. transposed.  Both frames' parity bytes are read with coalesced 8-byte loads into vdata (which the
+// systematic part fills only afterwards), interleaved, and written out transposed with coalesced 16-bit stores: a
+// strided gather of single bytes straight from the frames would touch a sector per lane and per layer.  vdata holds
+// 2K bytes, the parity pairs of the frame 2R: below rate 1/2 this goes in chunks of columns, a multiple of 8 columns
+// each so that every chunk starts 8-byte aligned.  Then the systematic LLRs -> vdata (A in even bytes, B in odd).
+// All threads of the CTA call it; the caller's barrier publishes vdata, the ones in here publish wpty.
+template <bool STREAMED, int THREADS>
+__device__ __noinline__ void load_pair(const LdpcParams2& p, const int8_t* inA, const int8_t* inB, uint16_t* vdata,
+                                       uint16_t* wpty) {
+    static_assert(THREADS % 360 == 0, "a whole number of threads per column");
+    const int tid = threadIdx.x, q = p.q, K = p.K;
+    uint4* v4 = reinterpret_cast<uint4*>(vdata);
+    const int8_t* ptA = inA + K;
+    const int8_t* ptB = inB + K;
+    const int cols = min(360, (K / q) & ~7);
+    const int jj = tid % 360, i0 = tid / 360;          // this thread's column in a chunk and first layer
+    for (int j0 = 0; j0 < 360; j0 += cols) {
+        const int nc = min(cols, 360 - j0);
+        const int b8 = q * j0 / 8;
+        for (int x = tid; x < q * nc / 8; x += THREADS) v4[x] = interleave8(ld_in8<STREAMED>(ptA, b8 + x), ld_in8<STREAMED>(ptB, b8 + x));
+        __syncthreads();
+        if (jj < nc)
+            for (int i = i0; i < q; i += THREADS / 360) __stcg(&wpty[i * 360 + j0 + jj], vdata[jj * q + i]);
+        __syncthreads();
+    }
+    for (int x = tid; x < K / 8; x += THREADS) v4[x] = interleave8(ld_in8<STREAMED>(inA, x), ld_in8<STREAMED>(inB, x));
+}
+
+// Take the next pair from the launch's counter ahead of time (the caller keeps it for its next round) and prefetch
+// both of its frames into L2, so that its load_pair reads from L2 instead of HBM.  Streamed input is prefetched only
+// when the copy engine has already delivered it; there is no waiting here.  cp.async.bulk.prefetch wants a 16-byte
+// aligned address and size; a short frame (16 200 bytes) of odd index starts 8 bytes off, so the range is widened to
+// 16-byte boundaries -- at most 15 bytes either side, inside the same mapped page as the frame's own bytes.
+// The last grid's worth of pairs is left to be handed out when a CTA is actually free (kNoPair): a pair claimed
+// ahead starts only after the slower frame of the current pair, which at the end of a launch lengthens its drain.
+constexpr unsigned kNoPair = 0xFFFFFFFFu;   // no pair claimed ahead
+template <bool STREAMED>
+__device__ __noinline__ unsigned claim_next_pair(const LdpcParams2& p, unsigned npairs) {
+    if (*reinterpret_cast<const volatile unsigned*>(p.work_counter) + gridDim.x >= npairs) return kNoPair;
+    const unsigned np = atomicAdd(p.work_counter, 1u);
+    if (np < npairs) {
+        const unsigned f0 = 2u * np, nf = min(2u, (unsigned)p.nframes - f0);
+        if (!STREAMED || *reinterpret_cast<const volatile unsigned*>(p.arrived) >= f0 + nf) {
+            const size_t b = reinterpret_cast<size_t>(p.llr_in + (size_t)f0 * p.N);
+            const size_t lo = b & ~(size_t)15, hi = (b + (size_t)nf * p.N + 15) & ~(size_t)15;
+            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(lo), "r"((unsigned)(hi - lo)) : "memory");
+        }
+    }
+    return np;
 }
 
 // Streamed input: block until the copy engine has delivered `need` frames.  Returns false when the host never
@@ -416,11 +453,15 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
 
     // zero the bit planes once: bytes 45..51 of every 360-bit group are never written and must read as 0
     for (int x = tid; x < 2 * (p.ngroups + q) * kBitWords; x += kThreads) __stcg(&HD[x], 0u);
+    __shared__ unsigned int s_next;   // pair claimed (and prefetched) while the current one still ran, or kNoPair
+    if (tid == 0) s_next = kNoPair;
 
     for (;;) {
         __syncthreads();
         if (tid == 0) {
-            unsigned np = atomicAdd(p.work_counter, 1u);
+            unsigned np = s_next;
+            if (np == kNoPair) np = atomicAdd(p.work_counter, 1u);
+            s_next = kNoPair;
             if (STREAMED && np < (unsigned)npairs) {
                 // the copy engine raises *arrived behind every piece of frames it has delivered (same stream, so the
                 // data is in memory before the count); pairs are handed out in frame order, so every waiter waits
@@ -445,33 +486,15 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
         }
         const int8_t* inA = p.llr_in + (size_t)fa * N;
         const int8_t* inB = p.llr_in + (size_t)(hasB ? fb : fa) * N;
-        // column j of the parity part: pty[i][j] = v[K + q j + i], contiguous in i
-        const int8_t* colA = inA + K + (size_t)q * j;
-        const int8_t* colB = inB + K + (size_t)q * j;
-        auto in_pair = [&](int i) -> uint32_t {   // parity LLR pair of row (i, j) from the input, packed offset binary
-            const uint32_t a = STREAMED ? (uint8_t)__ldcg(colA + i) : (uint8_t)__ldg(colA + i);
-            const uint32_t b = STREAMED ? (uint8_t)__ldcg(colB + i) : (uint8_t)__ldg(colB + i);
-            return (a | (b << 8)) ^ 0x8080u;
-        };
 
-        // ---- load: systematic LLRs -> shared (A in even bytes, B in odd), offset binary
-        for (int x = tid; x < K / 8; x += kThreads) {
-            // streamed: the copy engine is still writing other frames of this buffer -> L2-coherent loads
-            uint2 a = STREAMED ? __ldcg(reinterpret_cast<const uint2*>(inA) + x) : __ldg(reinterpret_cast<const uint2*>(inA) + x);
-            uint2 b = STREAMED ? __ldcg(reinterpret_cast<const uint2*>(inB) + x) : __ldg(reinterpret_cast<const uint2*>(inB) + x);
-            uint4 o;
-            o.x = prmt(a.x, b.x, 0x5140) ^ 0x80808080u;
-            o.y = prmt(a.x, b.x, 0x7362) ^ 0x80808080u;
-            o.z = prmt(a.y, b.y, 0x5140) ^ 0x80808080u;
-            o.w = prmt(a.y, b.y, 0x7362) ^ 0x80808080u;
-            reinterpret_cast<uint4*>(vdata)[x] = o;
-        }
+        // ---- load: parity LLR pairs -> workspace (transposed), systematic LLRs -> shared, offset binary
+        load_pair<STREAMED, kThreads>(p, inA, inB, vdata, wpty);
         uint32_t pown = 0, psec = 0;      // unpacked parity LLRs of the row being worked on
         {
-            const uint32_t last = in_pair(q - 1);
+            const uint32_t last = __ldcg(wpty + (q - 1) * 360 + j);
             X[j + 1] = (uint16_t)last;
             pown = unpack_lo(last);
-            psec = unpack_lo(in_pair(q - 2));
+            psec = unpack_lo(__ldcg(wpty + (q - 2) * 360 + j));
         }
         if (tid == 0) X[0] = 0xFFFFu;
 
@@ -521,7 +544,7 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
             //      screen found nothing for a frame that is still iterating
             int bad = (__syncthreads_or(scr & 1) ? 1 : 0) | (__syncthreads_or(scr & 2) ? 2 : 0);
             if (live & ~bad)
-                bad = full_test<STREAMED, kThreads>(p, n > 0, wpty, HP, HD, reinterpret_cast<const uint4*>(vdata), inA, inB, s_bad);
+                bad = full_test<kThreads>(p, wpty, HP, HD, reinterpret_cast<const uint4*>(vdata), s_bad);
             // ---- while (bad() && --trials >= 0) update();  (layered_decoder.hh:127-128), per frame
             int fin = 0;
             for (int f = 0; f < 2; ++f) {
@@ -534,7 +557,10 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
                 }
             }
             if (fin) {
-                emit_results<kThreads>(p, fin, res, fa, fb, n > 0, wpty, reinterpret_cast<const uint4*>(vdata), inA, inB);
+                emit_results<kThreads>(p, fin, res, fa, fb, wpty, reinterpret_cast<const uint4*>(vdata));
+                // the first frame of the pair to stop: take the next pair now and start its frames towards L2 (the
+                // other frame near the threshold runs more passes, which hide the HBM latency); not near the launch's end
+                if (tid == 0 && s_next == kNoPair) s_next = claim_next_pair<STREAMED>(p, (unsigned)npairs);
                 live &= ~fin;
                 // the other frame goes on: nobody may start the next pass (it overwrites the LLRs and the parity
                 // words in the workspace) while a slower warp is still reading them out
@@ -543,26 +569,21 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
             if (!live) break;
 
             // ---- LDPCDecoder::update (layered_decoder.hh:46-74): one pass over all layers.  The first pass (all
-            //      messages zero, parity LLRs straight from the input) is its own instantiation of the loop.
+            //      messages zero, row levels from the table) is its own instantiation of the loop.
             auto pass = [&](auto first_tag) {
                 constexpr bool FIRST = decltype(first_tag)::value;
                 uint32_t mw[MW];
                 uint4 nxt[SG];
-                uint32_t pnext = 0, pnext_b = 0;   // parity LLR pair of the next layer's own parity bit (FIRST: raw bytes of A, B)
+                uint32_t pnext = 0;    // parity LLR pair of the next layer's own parity bit
                 uint32_t pprev = 0;
 #pragma unroll
                 for (int x = 0; x < MW; ++x) mw[x] = 0;
                 // running pointers: this thread's message record and own parity LLR pair of the layer being worked on
                 uint4* rp = wmsg + j;
                 uint16_t* pp = wpty + j;
-                const int8_t* ca = colA;
-                const int8_t* cb = colB;
                 psec = unpack_lo(lds_u16(xaddr));    // X[j] = pty[q-1][j-1]; thread 0 reads the +127 stand-in of the missing link
-                if (FIRST) {
-                    pnext = STREAMED ? (uint8_t)__ldcg(ca) : (uint8_t)__ldg(ca);
-                    pnext_b = STREAMED ? (uint8_t)__ldcg(cb) : (uint8_t)__ldg(cb);
-                } else {
-                    pnext = __ldcg(pp);
+                pnext = __ldcg(pp);
+                if (!FIRST) {
 #pragma unroll
                     for (int s = 0; s < SG; ++s) nxt[s] = __ldcg(rp + s * 360);
                 }
@@ -585,14 +606,10 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
                         keep = nxt[SG - 1].w;
                     }
                     // pty[q-1][j] was updated in layer 0 by thread j+1 (at least one barrier ago: layer_sync)
-                    const uint32_t pw = FIRST ? ((pnext | (pnext_b << 8)) ^ 0x8080u) : pnext;
-                    pown = unpack_lo(i == q - 1 ? lds_u16(xaddr + 2) : pw);   // X[j + 1]
+                    pown = unpack_lo(i == q - 1 ? lds_u16(xaddr + 2) : pnext);   // X[j + 1]
                     if (i + 1 < q) {   // prefetch the next layer's row while this one computes
-                        if (FIRST) {
-                            pnext = STREAMED ? (uint8_t)__ldcg(ca + 1) : (uint8_t)__ldg(ca + 1);
-                            pnext_b = STREAMED ? (uint8_t)__ldcg(cb + 1) : (uint8_t)__ldg(cb + 1);
-                        } else {
-                            pnext = __ldcg(pp + 360);
+                        pnext = __ldcg(pp + 360);
+                        if (!FIRST) {
 #pragma unroll
                             for (int s = 0; s < SG; ++s) nxt[s] = __ldcg(rp + (SG + s) * 360);
                         }
@@ -632,8 +649,6 @@ __global__ void __launch_bounds__(kThreads, OCC) ldpc_v2_kernel(const __grid_con
                     psec = pown;
                     rp += SG * 360;
                     pp += 360;
-                    ca += 1;
-                    cb += 1;
                 }
                 // after the last layer: pprev = pty[q-2][j] (stored above), pown = pty[q-1][j], both final for this pass
                 psec = pprev;

@@ -150,11 +150,15 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
     }
     const int npairs = (p.nframes + 1) >> 1;
     for (int x = tid; x < 2 * (p.ngroups + q) * kBitWords; x += T) __stcg(&HD[x], 0u);
+    __shared__ unsigned int s_next;   // pair claimed (and prefetched) while the current one still ran, or kNoPair
+    if (tid == 0) s_next = kNoPair;
 
     for (;;) {
         __syncthreads();
         if (tid == 0) {
-            unsigned np = atomicAdd(p.work_counter, 1u);
+            unsigned np = s_next;
+            if (np == kNoPair) np = atomicAdd(p.work_counter, 1u);
+            s_next = kNoPair;
             if (STREAMED && np < (unsigned)npairs) {
                 if (!wait_arrived(p.arrived, min(2u * np + 2u, (unsigned)p.nframes), p.wait_budget)) np |= 0x80000000u;
                 __threadfence();
@@ -176,30 +180,14 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
         }
         const int8_t* inA = p.llr_in + (size_t)fa * N;
         const int8_t* inB = p.llr_in + (size_t)(hasB ? fb : fa) * N;
-        const int8_t* colA = inA + K + (size_t)q * j;
-        const int8_t* colB = inB + K + (size_t)q * j;
-        auto in_pair = [&](int i) -> uint32_t {
-            const uint32_t a = STREAMED ? (uint8_t)__ldcg(colA + i) : (uint8_t)__ldg(colA + i);
-            const uint32_t b = STREAMED ? (uint8_t)__ldcg(colB + i) : (uint8_t)__ldg(colB + i);
-            return (a | (b << 8)) ^ 0x8080u;
-        };
 
-        for (int x = tid; x < K / 8; x += T) {
-            uint2 a = STREAMED ? __ldcg(reinterpret_cast<const uint2*>(inA) + x) : __ldg(reinterpret_cast<const uint2*>(inA) + x);
-            uint2 b = STREAMED ? __ldcg(reinterpret_cast<const uint2*>(inB) + x) : __ldg(reinterpret_cast<const uint2*>(inB) + x);
-            uint4 o;
-            o.x = prmt(a.x, b.x, 0x5140) ^ 0x80808080u;
-            o.y = prmt(a.x, b.x, 0x7362) ^ 0x80808080u;
-            o.z = prmt(a.y, b.y, 0x5140) ^ 0x80808080u;
-            o.w = prmt(a.y, b.y, 0x7362) ^ 0x80808080u;
-            reinterpret_cast<uint4*>(vdata)[x] = o;
-        }
+        load_pair<STREAMED, T>(p, inA, inB, vdata, wpty);
         // this half's parity LLR of row (q-1, j): h = 0 pty[q-1][j], h = 1 pty[q-2][j] (for the screen before pass 1)
         uint32_t preg;
         {
-            const uint32_t last = in_pair(q - 1);
-            if (h == 0) X[j + 1] = (uint16_t)last;
-            preg = unpack_lo(h == 0 ? last : in_pair(q - 2));
+            const uint32_t w = __ldcg(wpty + (q - 1 - h) * 360 + j);
+            if (h == 0) X[j + 1] = (uint16_t)w;
+            preg = unpack_lo(w);
         }
         if (tid == 0) X[0] = 0xFFFFu;
 
@@ -248,7 +236,7 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
         for (int n = 0;; ++n) {
             int bad = (__syncthreads_or(scr & 1) ? 1 : 0) | (__syncthreads_or(scr & 2) ? 2 : 0);
             if (live & ~bad)
-                bad = full_test<STREAMED, T>(p, n > 0, wpty, HP, HD, reinterpret_cast<const uint4*>(vdata), inA, inB, s_bad);
+                bad = full_test<T>(p, wpty, HP, HD, reinterpret_cast<const uint4*>(vdata), s_bad);
             int fin = 0;
             for (int f = 0; f < 2; ++f) {
                 if (!(live >> f & 1)) continue;
@@ -260,7 +248,8 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
                 }
             }
             if (fin) {
-                emit_results<T>(p, fin, res, fa, fb, n > 0, wpty, reinterpret_cast<const uint4*>(vdata), inA, inB);
+                emit_results<T>(p, fin, res, fa, fb, wpty, reinterpret_cast<const uint4*>(vdata));
+                if (tid == 0 && s_next == kNoPair) s_next = claim_next_pair<STREAMED>(p, (unsigned)npairs);   // as ldpc_v2_kernel
                 live &= ~fin;
                 // the other frame goes on: nobody may start the next pass (it overwrites the LLRs and the parity
                 // words in the workspace) while a slower warp is still reading them out
@@ -272,20 +261,15 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
                 constexpr bool FIRST = decltype(first_tag)::value;
                 uint32_t mw[MW];
                 uint4 nxt[SG];
-                uint32_t pnext = 0, pnext_b = 0;
+                uint32_t pnext = 0;
 #pragma unroll
                 for (int x = 0; x < MW; ++x) mw[x] = 0;
                 uint4* rp = wmsg + slot_t;
                 uint16_t* pp = wpty + j;
-                const int8_t* ca = colA;
-                const int8_t* cb = colB;
                 // h = 1 starts with pty[q-1][j-1] (X[j]; thread 0's is the +127 stand-in of the missing link)
                 if (h == 1) preg = unpack_lo(lds_u16(xaddr));
-                if (FIRST) {
-                    pnext = STREAMED ? (uint8_t)__ldcg(ca) : (uint8_t)__ldg(ca);
-                    pnext_b = STREAMED ? (uint8_t)__ldcg(cb) : (uint8_t)__ldg(cb);
-                } else {
-                    pnext = __ldcg(pp);
+                pnext = __ldcg(pp);
+                if (!FIRST) {
 #pragma unroll
                     for (int s = 0; s < SG; ++s) nxt[s] = __ldcg(rp + s * 720);
                 }
@@ -302,16 +286,11 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
                         }
                         keep = nxt[SG - 1].w;
                     }
-                    if (h == 0) {   // the row's own parity bit
-                        const uint32_t pw = FIRST ? ((pnext | (pnext_b << 8)) ^ 0x8080u) : pnext;
-                        preg = unpack_lo(i == q - 1 ? lds_u16(xaddr + 2) : pw);   // X[j + 1]
-                    }
+                    if (h == 0)     // the row's own parity bit
+                        preg = unpack_lo(i == q - 1 ? lds_u16(xaddr + 2) : pnext);   // X[j + 1]
                     if (i + 1 < q) {
-                        if (FIRST) {
-                            pnext = STREAMED ? (uint8_t)__ldcg(ca + 1) : (uint8_t)__ldg(ca + 1);
-                            pnext_b = STREAMED ? (uint8_t)__ldcg(cb + 1) : (uint8_t)__ldg(cb + 1);
-                        } else {
-                            pnext = __ldcg(pp + 360);
+                        pnext = __ldcg(pp + 360);
+                        if (!FIRST) {
 #pragma unroll
                             for (int s = 0; s < SG; ++s) nxt[s] = __ldcg(rp + (SG + s) * 720);
                         }
@@ -353,8 +332,6 @@ __global__ void __launch_bounds__(kLdpcThreads2, 1) ldpc_v2l_kernel(const __grid
                     if (h == 1 && i + 1 < q) preg = other;
                     rp += 2 * SG * 360;
                     pp += 360;
-                    ca += 1;
-                    cb += 1;
                 }
                 // after the last layer: h = 0 holds pty[q-1][j], h = 1 pty[q-2][j] (stored above), both final
                 if (h == 0) {
