@@ -1,6 +1,8 @@
 // K3/K4/K5 -- see bch_decoder.cuh.
 #include "bch_decoder.cuh"
 
+#include <algorithm>
+
 namespace s2 {
 namespace {
 
@@ -291,10 +293,12 @@ __global__ void __launch_bounds__(kWarps * 32) bch_kernel(const __grid_constant_
     }
 }
 
+// gridDim.y is at most 65535: each block row takes frames blockIdx.y, blockIdx.y + gridDim.y, ...
 __global__ void descramble_kernel(uint8_t* frames, int stride, int nframes, int kbytes, const uint8_t* prbs) {
-    int x = blockIdx.x * blockDim.x + threadIdx.x;
-    int f = blockIdx.y;
-    if (x < kbytes && f < nframes) frames[(size_t)f * stride + x] ^= prbs[x];
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= kbytes) return;
+    const uint8_t p = prbs[x];
+    for (int f = blockIdx.y; f < nframes; f += gridDim.y) frames[(size_t)f * stride + x] ^= p;
 }
 
 }  // namespace
@@ -312,7 +316,7 @@ int bch_launch(const BchArgs& a, cudaStream_t stream) {
 int descramble_launch(uint8_t* frames, int stride, int nframes, int kbch, const uint8_t* prbs, cudaStream_t stream) {
     if (nframes <= 0) return 0;
     int kbytes = kbch / 8;
-    dim3 grid((kbytes + 255) / 256, nframes);
+    dim3 grid((kbytes + 255) / 256, std::min(nframes, 65535));
     descramble_kernel<<<grid, 256, 0, stream>>>(frames, stride, nframes, kbytes, prbs);
     return (int)cudaGetLastError();
 }

@@ -159,19 +159,21 @@ __global__ void __launch_bounds__(kChainThreads) plsync_chain_kernel(const PlSyn
     }
 }
 
-// blockIdx.y < max_frames: frame k -> out; blockIdx.y == max_frames: what stays behind -> front of the next work buffer
+// k < max_frames: frame k -> out; k == max_frames: what stays behind -> front of the next work buffer.  k runs from
+// blockIdx.y in steps of gridDim.y, which is at most 65535.
 __global__ void __launch_bounds__(256) plsync_copy_kernel(const PlSyncArgs a, int pend_before_upper) {
-    const int k = blockIdx.y;
     const int nfr = a.st->nframes;
-    if (k < a.max_frames) {
-        if (k >= nfr) return;
-        const float2* src = a.work + a.starts[k];
-        float2* dst = a.out + (size_t)k * a.rfs;
-        for (int i = blockIdx.x * 256 + threadIdx.x; i < a.rfs; i += gridDim.x * 256) dst[i] = src[i];
-    } else {
-        const float2* src = a.work + a.starts[a.max_frames];
-        const int n = a.st->pend;
-        for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) a.work_next[i] = src[i];
+    for (int k = blockIdx.y; k <= a.max_frames; k += gridDim.y) {
+        if (k < a.max_frames) {
+            if (k >= nfr) continue;
+            const float2* src = a.work + a.starts[k];
+            float2* dst = a.out + (size_t)k * a.rfs;
+            for (int i = blockIdx.x * 256 + threadIdx.x; i < a.rfs; i += gridDim.x * 256) dst[i] = src[i];
+        } else {
+            const float2* src = a.work + a.starts[a.max_frames];
+            const int n = a.st->pend;
+            for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) a.work_next[i] = src[i];
+        }
     }
 }
 
@@ -272,7 +274,7 @@ int plsync_launch(const PlSyncArgs& a, int pend_upper_bound, cudaStream_t stream
     if (a.append && a.count > 0) plsync_append_kernel<<<std::min((a.count + 255) / 256, 1184), 256, 0, stream>>>(a);
     if (lmax >= kPlHeader) plsync_metric_kernel<<<(lmax - kPlHeader + 1 + kMetricThreads - 1) / kMetricThreads, kMetricThreads, 0, stream>>>(a);
     plsync_chain_kernel<<<1, kChainThreads, 0, stream>>>(a);
-    plsync_copy_kernel<<<dim3(16, a.max_frames + 1), 256, 0, stream>>>(a, pend_upper_bound);
+    plsync_copy_kernel<<<dim3(16, std::min(a.max_frames + 1, 65535)), 256, 0, stream>>>(a, pend_upper_bound);
     return (int)cudaGetLastError();
 }
 
