@@ -32,6 +32,7 @@ extern "C" {
 #define DVBS2FEC_FLAG_BCH_FAIL 2u  /* BBFrameBCH::decode returned -1 */
 #define DVBS2FEC_FLAG_BBHEADER_CRC_FAIL 4u /* CRC-8 over the 80 BBHEADER bits is non-zero: BBFrameTSParser::work would
                                               drop this frame (dvbs2/bbframe_ts_parser.cpp:66-80,121-134) */
+#define DVBS2FEC_FLAG_DUMMY 8u     /* VCM calls: the frame is a DUMMY PLFRAME (modcod 0); nothing was decoded */
 
 typedef struct dvbs2fec_handle dvbs2fec_handle;
 
@@ -120,13 +121,43 @@ int dvbs2fec_decode_batch_device(dvbs2fec_handle* h, const int8_t* d_llr, int n,
  * without a host copy of the symbols (S2BBToSoft::process onwards, module_dvbs2_demod.cpp:334-366) */
 int dvbs2fec_decode_plframes_device(dvbs2fec_handle* h, const float* d_plframes, int n, uint8_t* d_bb_out,
                                     dvbs2fec_result* d_results, void* cuda_stream);
-/* number of kernel launches the last decode_batch* call on this handle enqueued */
+/* number of kernel launches the last decode_batch* / decode_*vcm* call on this handle enqueued */
 int dvbs2fec_last_launch_count(const dvbs2fec_handle* h);
 /* measurement aid: with profiling on, every kernel launch of decode_batch_device is bracketed by CUDA
  * events on its stream; kernel_times() waits for them and returns the summed device time per kernel
- * (ms) and the number of launches since the previous call. */
+ * (ms) and the number of launches since the previous call.  VCM calls count their gather into demap_ms and their
+ * scatter into bch_ms. */
 int dvbs2fec_set_profiling(dvbs2fec_handle* h, int on);
 int dvbs2fec_kernel_times(dvbs2fec_handle* h, float* demap_ms, float* ldpc_ms, float* bch_ms, int* launches);
+
+/* ---- VCM / ACM: frames of different MODCOD, frame size and pilot setting in one call ----
+ * desc holds four int32 per frame, laid out like the results of dvbs2fec_plhdr_process so that they can be passed
+ * straight in: modcod (0..28), shortframes, pilots, and a fourth field that is ignored.  modcod 0 is a DUMMY PLFRAME:
+ * 90 + 36 * 90 = 3330 symbols, no LLRs, no BBFRAME bytes; its result has ldpc_iters = 0, bch_corr = 0 and
+ * DVBS2FEC_FLAG_DUMMY.  Any other frame without an LDPC code (modcod outside 0..28, short frames at rate 9/10) fails
+ * the whole call with DVBS2FEC_EINVAL before anything is written; the error text names the frame.
+ * Frames are packed back to back in input order: dvbs2fec_plframe_symbols(frame) complex floats, nldpc(frame) LLR
+ * bytes and kbch(frame) / 8 BBFRAME bytes each (no alignment: normal 1/4 is 2001 bytes).  One result per frame,
+ * tag = the frame's index in the call. */
+
+/* n + 1 prefix offsets of that layout into each non-NULL array: sym_off in complex samples, llr_off and bb_off in
+ * bytes.  Needs no handle or device. */
+int dvbs2fec_vcm_layout(int n, const int32_t* desc, int64_t* sym_off, int64_t* llr_off, int64_t* bb_off);
+/* dvbs2fec_decode_batch / dvbs2fec_decode_plframes for a VCM batch: host buffers, synchronous.  desc is in host memory
+ * in all four calls (the host groups the frames by LDPC code and sizes the launches from it).  The calls use the
+ * handle's max_trials and dvbs2fec_set_pl_scrambling setting (the PL descrambling sequence restarts at every frame),
+ * run on the handle's first device, need no dvbs2fec_set_modcod and leave the configured MODCOD as it was.  A call
+ * runs in chunks of at most max_batch frames; inside a chunk the frames of each LDPC code are decoded by one launch. */
+int dvbs2fec_decode_vcm(dvbs2fec_handle* h, int n, const int32_t* desc, const int8_t* llr, uint8_t* bb_out,
+                        dvbs2fec_result* results);
+int dvbs2fec_decode_plframes_vcm(dvbs2fec_handle* h, int n, const int32_t* desc, const float* plframes, uint8_t* bb_out,
+                                 dvbs2fec_result* results);
+/* the same on device buffers, enqueued on `cuda_stream` and not synchronised, sharing the scratch and the ordering of
+ * dvbs2fec_decode_batch_device */
+int dvbs2fec_decode_vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const int8_t* d_llr, uint8_t* d_bb_out,
+                               dvbs2fec_result* d_results, void* cuda_stream);
+int dvbs2fec_decode_plframes_vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const float* d_plframes,
+                                        uint8_t* d_bb_out, dvbs2fec_result* d_results, void* cuda_stream);
 
 /* ---- frame-batching queue between PL sync and the decoder (replaces simd_packer,
  *      module_dvbs2_demod.cpp:343-347): frames come back in submission order ---- */

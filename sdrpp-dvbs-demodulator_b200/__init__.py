@@ -24,7 +24,7 @@ LIB_PATH = os.path.join(_HERE, "libdvbs2fec.so")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include", "dvbs2fec.h")
 
 EINVAL, ENODEV, ECUDA, EAGAIN, ENOSPC = -22, -19, -5, -11, -28
-FLAG_LDPC_FAIL, FLAG_BCH_FAIL, FLAG_BBHEADER_CRC_FAIL = 1, 2, 4
+FLAG_LDPC_FAIL, FLAG_BCH_FAIL, FLAG_BBHEADER_CRC_FAIL, FLAG_DUMMY = 1, 2, 4, 8
 
 # reference dvbs2_code_rate_t numbering (dvbs2/dvbs2.h:11-25)
 RATE_NAMES = {0: "1/4", 1: "1/3", 2: "2/5", 3: "1/2", 4: "3/5", 5: "2/3", 6: "3/4", 7: "4/5", 8: "5/6", 10: "8/9", 11: "9/10"}
@@ -180,6 +180,11 @@ def lib():
     L.dvbs2fec_pll_set_state.argtypes = [vp, C.c_float, C.c_float]
     L.dvbs2fec_pll_set_sequential.argtypes = [vp, C.c_int]
     L.dvbs2fec_pll_process_multi_device.argtypes = [C.c_int, vp, C.c_int, C.c_int, vp, vp, vp]
+    L.dvbs2fec_vcm_layout.argtypes = [C.c_int, vp, vp, vp, vp]
+    L.dvbs2fec_decode_vcm.argtypes = [vp, C.c_int, vp, vp, vp, vp]
+    L.dvbs2fec_decode_plframes_vcm.argtypes = [vp, C.c_int, vp, vp, vp, vp]
+    L.dvbs2fec_decode_vcm_device.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp]
+    L.dvbs2fec_decode_plframes_vcm_device.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -219,6 +224,20 @@ def modulate(modcod, shortframes, pilots, code_bits):
     out = np.zeros(info["plframe_symbols"] * 2, np.float32)
     _check(lib().dvbs2fec_modulate(modcod, int(shortframes), int(pilots), _ptr(bits), _ptr(out)))
     return out.view(np.complex64)
+
+
+def _vcm_desc(desc):
+    """frame descriptors as dvbs2fec_plhdr_process returns them: int32 [n][4] = modcod, shortframes, pilots, (ignored)"""
+    return np.ascontiguousarray(desc, np.int32).reshape(-1, 4)
+
+
+def vcm_layout(desc):
+    """packed layout of a VCM batch: (sym_off, llr_off, bb_off), n + 1 int64 prefix offsets each -- complex samples of
+    the PLFRAMEs, LLR bytes, BBFRAME bytes.  Raises DVBS2FecError (EINVAL) on a descriptor without a code."""
+    d = _vcm_desc(desc)
+    offs = [np.zeros(len(d) + 1, np.int64) for _ in range(3)]
+    _check(lib().dvbs2fec_vcm_layout(len(d), _ptr(d), *[_ptr(o) for o in offs]))
+    return tuple(offs)
 
 
 class DVBS2Decoder:
@@ -349,6 +368,39 @@ class DVBS2Decoder:
     def decode_plframes_device(self, d_plframes_ptr, n, d_bb_ptr, d_res_ptr, stream_ptr=0):
         """PLFRAME symbols on the device (plframe_symbols complex floats per frame) -> BBFRAMEs on the device"""
         _check(lib().dvbs2fec_decode_plframes_device(self._h, d_plframes_ptr, n, d_bb_ptr, d_res_ptr, stream_ptr))
+
+    # ---- VCM / ACM batches: any MODCOD, frame size and pilot setting per frame (no setDemodParams needed) ----
+    def decode_vcm(self, desc, llr):
+        """desc: int32 [n][4] (modcod 0 = DUMMY PLFRAME); llr: the frames' LLRs packed back to back (vcm_layout).
+        -> (packed BBFRAME bytes, bb_off [n + 1], results [n])"""
+        d = _vcm_desc(desc)
+        _, llr_off, bb_off = vcm_layout(d)
+        x = np.ascontiguousarray(llr, np.int8).reshape(-1)
+        assert x.size == llr_off[-1], (x.size, llr_off[-1])
+        bb = np.zeros(bb_off[-1], np.uint8)
+        res = np.zeros(len(d), RESULT_DTYPE)
+        _check(lib().dvbs2fec_decode_vcm(self._h, len(d), _ptr(d), _ptr(x), _ptr(bb), _ptr(res)))
+        return bb, bb_off, res
+
+    def decode_plframes_vcm(self, desc, plframes):
+        """desc as decode_vcm; plframes: the PLFRAMEs packed back to back (complex64, vcm_layout's sym_off)"""
+        d = _vcm_desc(desc)
+        sym_off, _, bb_off = vcm_layout(d)
+        x = np.ascontiguousarray(plframes).view(np.float32).reshape(-1)
+        assert x.size == 2 * sym_off[-1], (x.size, 2 * sym_off[-1])
+        bb = np.zeros(bb_off[-1], np.uint8)
+        res = np.zeros(len(d), RESULT_DTYPE)
+        _check(lib().dvbs2fec_decode_plframes_vcm(self._h, len(d), _ptr(d), _ptr(x), _ptr(bb), _ptr(res)))
+        return bb, bb_off, res
+
+    def decode_vcm_device(self, desc, d_llr_ptr, d_bb_ptr, d_res_ptr, stream_ptr=0):
+        """desc in host memory, the rest device pointers (vcm_layout sizes them); enqueues on ``stream_ptr`` and returns"""
+        d = _vcm_desc(desc)
+        _check(lib().dvbs2fec_decode_vcm_device(self._h, len(d), _ptr(d), d_llr_ptr, d_bb_ptr, d_res_ptr, stream_ptr))
+
+    def decode_plframes_vcm_device(self, desc, d_plframes_ptr, d_bb_ptr, d_res_ptr, stream_ptr=0):
+        d = _vcm_desc(desc)
+        _check(lib().dvbs2fec_decode_plframes_vcm_device(self._h, len(d), _ptr(d), d_plframes_ptr, d_bb_ptr, d_res_ptr, stream_ptr))
 
     def set_profiling(self, on):
         _check(lib().dvbs2fec_set_profiling(self._h, int(on)))

@@ -29,6 +29,7 @@
 #include "ldpc_decoder.cuh"
 #include "s2_codes.h"
 #include "ts_parser.cuh"
+#include "vcm.cuh"
 
 using namespace s2;
 
@@ -124,10 +125,18 @@ struct Slot {
     PinBuf<uint8_t> h_in;
     PinBuf<uint8_t> h_bb;
     PinBuf<dvbs2fec_result> h_res;
+    // VCM calls: the chunk's input as it arrives (host entries), its packed output (host entries), the frame records
+    DevBuf<uint8_t> vin;
+    DevBuf<uint8_t> vbb;
+    DevBuf<dvbs2fec_result> vres;
+    DevBuf<VcmFrame> vmeta;
+    PinBuf<VcmFrame> h_vmeta;
+    bool vmeta_copying = false;          // device entry: `armed` marks the end of the last copy out of h_vmeta
     // pending copy-out of a staged batch
     uint8_t* user_bb = nullptr;
     dvbs2fec_result* user_res = nullptr;
     int pending = 0;
+    size_t bb_bytes = 0;
     bool staged_out = true;
     uint64_t tag_base = 0;
 };
@@ -137,6 +146,14 @@ struct CodeDev {  // per (device, LDPC code)
 };
 struct BchTabDev {
     DevBuf<uint16_t> crc, basis;
+};
+
+struct CodeTables {  // what the kernels of one LDPC code need; ldpc.links points into links
+    LdpcDev ldpc{};
+    BchDev bch{};
+    int grid = 0;
+    int hard_stride = 0;
+    std::vector<uint32_t> links;
 };
 
 struct DevCtx {
@@ -158,7 +175,14 @@ struct DevCtx {
     BchDev bchd{};
     DemapDev demap{};
     int grid = 0;
-    ~DevCtx() { ldpc_release(ldpc); }
+    // VCM calls: prepared codes by code index, demap records by (modcod, short, pilots) -- see vcm.cuh
+    std::map<int, CodeTables> vcm_codes;
+    DevBuf<DemapDev> vcm_demap;
+    bool vcm_demap_ok[kVcmConfigs] = {};
+    ~DevCtx() {
+        ldpc_release(ldpc);
+        for (auto& kv : vcm_codes) ldpc_release(kv.second.ldpc);
+    }
 };
 
 }  // namespace
@@ -241,17 +265,14 @@ static int ts_args(dvbs2fec_ts_parser* p, const uint8_t* d_bb, int cnt, uint8_t*
 
 namespace {
 
-int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
-    CU(cudaSetDevice(d.device));
-    const LdpcCode& c = *h->code;
-    // --- LDPC
+// LDPC code c on device d into L (ldpc_prepare) and its grid; links = host link words of c, kept alive by the caller
+int prepare_ldpc(DevCtx& d, const LdpcCode& c, const uint32_t* links, LdpcDev& L, int& grid) {
     CodeDev& cd = d.codes[c.index];
     if (!cd.row_level.p) {
         CU(cd.row_level.reserve(c.row_level.size()));
         CU(cudaMemcpy(cd.row_level.p, c.row_level.data(), c.row_level.size(), cudaMemcpyHostToDevice));
         CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
     }
-    LdpcDev& L = d.ldpc;
     L.N = c.N; L.K = c.K; L.R = c.R; L.q = c.q;
     L.ngroups = c.K / kGroup;
     L.max_cnt = c.max_cnt;
@@ -261,7 +282,7 @@ int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
     L.chains = !L.v2 && ldpc_chains_pay_off(c.index);
     L.occ3 = ldpc_ctas_wanted3(c.index);
     if (!L.sg) return fail(DVBS2FEC_EINVAL, "no LDPC kernel for %d links per row", c.max_cnt);
-    L.links = h->h_links.data();
+    L.links = links;
     L.layer_off = c.layer_off.data();
     L.layer_nlev = c.layer_nlev.data();
     L.row_level = cd.row_level.p;
@@ -269,8 +290,12 @@ int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
     int per_sm = ldpc_max_ctas_per_sm(L);
     if (per_sm <= 0) return fail(DVBS2FEC_ENODEV, "LDPC kernel does not fit on device %d (%s)", d.device,
                                  cudaGetErrorString(cudaGetLastError()));
-    d.grid = d.sms * per_sm;
-    // --- BCH
+    grid = d.sms * per_sm;
+    return 0;
+}
+
+// BCH, GF and BB scrambler tables of code c on device d into B
+int prepare_bch(DevCtx& d, const LdpcCode& c, BchDev& B) {
     const int m = c.bch_m, t = c.bch_t, fi = (m == 16);
     const GfHost& gf = gf_host(m);
     if (!d.gf_log[fi].p) {
@@ -297,14 +322,15 @@ int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
         CU(cudaMemcpy(d.prbs.p, seq.data(), seq.size(), cudaMemcpyHostToDevice));
         CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
     }
-    BchDev& B = d.bchd;
     B.gf.m = m; B.gf.N = gf.N; B.gf.log = d.gf_log[fi].p; B.gf.exp = d.gf_exp[fi].p;
     B.t = t; B.nbch = c.K; B.kbch = c.kbch;
     B.prefix = gf.N - c.K;
     B.crc = bt.crc.p; B.basis = bt.basis.p; B.prbs = d.prbs.p;
-    // --- demapper
-    const ModcodCfg& mc = h->mc;
-    DemapDev& D = d.demap;
+    return 0;
+}
+
+// demapper record of configuration mc (code c, plsyms complex samples per PLFRAME) on device d into D
+int prepare_demap(DevCtx& d, const ModcodCfg& mc, const LdpcCode& c, int plsyms, const uint8_t* rn, DemapDev& D) {
     ConstellationHost ch = make_constellation(mc.constellation, mc.g1, mc.g2);
     D.constellation = (int)mc.constellation;
     D.bits = mc.bits;
@@ -312,14 +338,14 @@ int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
     D.nsym = c.N / mc.bits;
     D.reversed_cols = (mc.constellation == PSK8 && mc.rate == R3_5);
     D.pilots = mc.pilots;
-    D.plframe_syms = h->plsyms;
+    D.plframe_syms = plsyms;
     D.amp = ch.amp; D.prescale = ch.prescale; D.sca = ch.sca;
     for (int i = 0; i < 32; ++i) {
         D.pts[2 * i] = i < ch.states ? ch.re[i] : 0.f;
         D.pts[2 * i + 1] = i < ch.states ? ch.im[i] : 0.f;
     }
     D.lut = nullptr;
-    D.rn = h->pl_codenum >= 0 ? d.pl_rn.p : nullptr;
+    D.rn = rn;
     if (mc.constellation != APSK32) {
         int key = (mc.constellation == APSK16) ? mc.modcod : (int)mc.constellation;  // 16APSK: one LUT per gamma
         DevBuf<uint32_t>& lut = d.luts[key];
@@ -332,6 +358,14 @@ int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
         D.lut = lut.p;
     }
     return 0;
+}
+
+int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
+    CU(cudaSetDevice(d.device));
+    const LdpcCode& c = *h->code;
+    if (int rc = prepare_ldpc(d, c, h->h_links.data(), d.ldpc, d.grid)) return rc;
+    if (int rc = prepare_bch(d, c, d.bchd)) return rc;
+    return prepare_demap(d, h->mc, c, h->plsyms, h->pl_codenum >= 0 ? d.pl_rn.p : nullptr, d.demap);
 }
 
 // kind of input: 0 = LLRs, 1 = PLFRAME symbols, 2 = LUT coordinates of the payload symbols
@@ -361,14 +395,13 @@ int reserve_slot(dvbs2fec_handle* h, DevCtx& d, Slot& s, int nframes, int kind, 
     return 0;
 }
 
-// enqueue demap (optional) + LDPC + BCH/descramble for n frames already on the device
-int enqueue_chain(dvbs2fec_handle* h, DevCtx& d, Slot& s, const float* d_sym, const int8_t* d_llr, int n,
-                  uint8_t* d_bb, dvbs2fec_result* d_res, cudaStream_t st, int* launches, uint64_t tag_base = 0,
-                  const unsigned int* arrived = nullptr, const uint8_t* d_idx = nullptr) {
-    const int8_t* llr = d_llr;
-    // kernel-time spans for dvbs2fec_kernel_times; several threads (one per GPU, the queue worker) may add some
+// kernel-time spans for dvbs2fec_kernel_times (kind 0 demap, 1 LDPC, 2 BCH); several threads (one per GPU, the queue
+// worker) may add some
+struct SpanMark {
+    dvbs2fec_handle* h;
+    cudaStream_t st;
     dvbs2fec_handle::Span cur{0, nullptr, nullptr};
-    auto mark = [&](int kind, bool begin) {
+    void operator()(int kind, bool begin) {
         if (!h->profiling) return;
         if (begin) {
             cur = dvbs2fec_handle::Span{kind, nullptr, nullptr};
@@ -380,7 +413,15 @@ int enqueue_chain(dvbs2fec_handle* h, DevCtx& d, Slot& s, const float* d_sym, co
             std::lock_guard<std::mutex> lk(h->span_mu);
             h->spans.push_back(cur);
         }
-    };
+    }
+};
+
+// enqueue demap (optional) + LDPC + BCH/descramble for n frames already on the device
+int enqueue_chain(dvbs2fec_handle* h, DevCtx& d, Slot& s, const float* d_sym, const int8_t* d_llr, int n,
+                  uint8_t* d_bb, dvbs2fec_result* d_res, cudaStream_t st, int* launches, uint64_t tag_base = 0,
+                  const unsigned int* arrived = nullptr, const uint8_t* d_idx = nullptr) {
+    const int8_t* llr = d_llr;
+    SpanMark mark{h, st};
     if (d_sym || d_idx) {
         mark(0, true);
         int e = d_sym ? demap_launch(d.demap, d_sym, n, s.llr.p, st) : demap_idx_launch(d.demap, d_idx, n, s.llr.p, st);
@@ -471,12 +512,34 @@ bool is_pinned(const void* p) {
 int finish_slot(dvbs2fec_handle* h, Slot& s) {
     if (!s.pending) return 0;
     CU(cudaEventSynchronize(s.done));
-    const size_t kb = h->code->kbch / 8;
-    if (s.user_bb && s.staged_out) memcpy(s.user_bb, s.h_bb.p, (size_t)s.pending * kb);
+    if (s.user_bb && s.staged_out) memcpy(s.user_bb, s.h_bb.p, s.bb_bytes);
     if (s.user_res && s.staged_out) memcpy(s.user_res, s.h_res.p, (size_t)s.pending * sizeof(dvbs2fec_result));
     s.pending = 0;
     return 0;
 }
+
+// Error exit of the synchronous entry points: nothing asynchronous may outlive the call -- copies into the caller's
+// buffers that were already enqueued are waited for, and no slot keeps a pointer to them (a later call would copy into
+// freed memory).
+struct HostSlotsAbort {
+    DevCtx& d;
+    bool armed = true;
+    ~HostSlotsAbort() {
+        if (!armed) return;
+        char keep[sizeof(g_err)];
+        memcpy(keep, g_err, sizeof keep);
+        for (int k = 0; k < kSlots; ++k) {
+            Slot& s = d.slot[k];
+            cudaStreamSynchronize(s.copy);
+            cudaStreamSynchronize(s.stream);
+            s.pending = 0;
+            s.user_bb = nullptr;
+            s.user_res = nullptr;
+        }
+        cudaGetLastError();
+        memcpy(g_err, keep, sizeof keep);
+    }
+};
 
 // frames [0, n) of one device's share, host buffers in and out
 int run_device_share(dvbs2fec_handle* h, DevCtx& d, const int8_t* llr, const float* sym, const uint8_t* idx, int n, uint8_t* bb,
@@ -497,27 +560,7 @@ int run_device_share(dvbs2fec_handle* h, DevCtx& d, const int8_t* llr, const flo
     const bool pin_in = is_pinned(in);
     const bool pin_out = (!bb || is_pinned(bb)) && (!res || is_pinned(res));
     int which = 0, rc = 0;
-    // Error exit: nothing asynchronous may outlive the call -- copies into the caller's buffers that were already
-    // enqueued are waited for, and no slot keeps a pointer to them (a later call would copy into freed memory).
-    struct Abort {
-        DevCtx& d;
-        bool armed = true;
-        ~Abort() {
-            if (!armed) return;
-            char keep[sizeof(g_err)];
-            memcpy(keep, g_err, sizeof keep);
-            for (int k = 0; k < kSlots; ++k) {
-                Slot& s = d.slot[k];
-                cudaStreamSynchronize(s.copy);
-                cudaStreamSynchronize(s.stream);
-                s.pending = 0;
-                s.user_bb = nullptr;
-                s.user_res = nullptr;
-            }
-            cudaGetLastError();
-            memcpy(g_err, keep, sizeof keep);
-        }
-    } abort_guard{d};
+    HostSlotsAbort abort_guard{d};
     for (int f0 = 0; f0 < n; f0 += chunk, which ^= 1) {
         Slot& s = d.slot[which];
         const int m = std::min(chunk, n - f0);
@@ -549,6 +592,7 @@ int run_device_share(dvbs2fec_handle* h, DevCtx& d, const int8_t* llr, const flo
         CU(cudaEventRecord(s.done, s.stream));
         s.tag_base = tag0 + f0;
         s.pending = m;
+        s.bb_bytes = (size_t)m * kb;
     }
     for (int k = 0; k < kSlots; ++k)
         if ((rc = finish_slot(h, d.slot[k]))) return rc;
@@ -720,6 +764,369 @@ void drain_queue(dvbs2fec_handle* h) {
     h->flush_req = false;
 }
 
+// ---------------------------------------------------------------- VCM / ACM batches (vcm.cuh)
+struct VcmDesc {   // one frame of a call; code -1: DUMMY PLFRAME
+    int cfg, code, plsyms, nsym, N, kb;
+};
+struct VcmGroup {  // the frames of one LDPC code inside a chunk, in input order
+    int code, cnt, p0;                  // p0: first record in group order
+    size_t llr_off, hard_off, bb_off;   // byte offsets of the group in the chunk's scratch
+};
+struct VcmChunk {
+    int f0, f1;
+    bool fast;                          // one code, no dummy frame: nothing to reorder
+    int nsym_max, n_max;
+    std::vector<VcmGroup> groups;       // largest first
+};
+struct VcmPlan {
+    std::vector<VcmDesc> fr;
+    std::vector<int64_t> sym_off, llr_off, bb_off;   // [n + 1]
+    std::vector<VcmFrame> rec;                       // [n]
+    std::vector<VcmChunk> chunks;
+    size_t llr_bytes = 0, hard_bytes = 0, bb_bytes = 0, workspace = 0, in_max = 0, out_max = 0;   // per chunk, maximum
+    int max_chunk = 0;
+};
+
+constexpr int kDummySyms = 90 + 36 * 90;   // DUMMY PLFRAME: header + 36 slots
+
+size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// validates every descriptor and fills the layout; nothing else is touched on error
+int vcm_parse(int n, const int32_t* desc, VcmPlan& P) {
+    if (n < 0) return fail(DVBS2FEC_EINVAL, "frame count %d is negative", n);
+    if (n > 0 && !desc) return fail(DVBS2FEC_EINVAL, "desc is NULL");
+    P.fr.resize(n);
+    P.sym_off.assign(n + 1, 0);
+    P.llr_off.assign(n + 1, 0);
+    P.bb_off.assign(n + 1, 0);
+    for (int i = 0; i < n; ++i) {
+        const int modcod = desc[4 * i];
+        const bool sh = desc[4 * i + 1] != 0, pi = desc[4 * i + 2] != 0;
+        VcmDesc& f = P.fr[i];
+        if (modcod == 0) {
+            f = VcmDesc{0, -1, kDummySyms, 0, 0, 0};
+        } else {
+            ModcodCfg mc;
+            if (modcod < 0 || modcod > 28 || !modcod_config(modcod, sh, pi, &mc) || mc.code < 0)
+                return fail(DVBS2FEC_EINVAL, "frame %d: MODCOD %d with %s frames has no LDPC code", i, modcod,
+                            sh ? "short" : "normal");
+            const LdpcCode& c = ldpc_code(mc.code);
+            const int nsym = c.N / mc.bits;
+            f = VcmDesc{modcod * 4 + sh * 2 + pi, mc.code, 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0), nsym, c.N,
+                        c.kbch / 8};
+        }
+        P.sym_off[i + 1] = P.sym_off[i] + f.plsyms;
+        P.llr_off[i + 1] = P.llr_off[i] + f.N;
+        P.bb_off[i + 1] = P.bb_off[i] + f.kb;
+    }
+    return 0;
+}
+
+// Prepares every code and (symbol input) demap record the call uses, then splits it into chunks of at most chunk
+// frames and lays out each chunk's groups and frame records.
+int vcm_plan(dvbs2fec_handle* h, DevCtx& d, VcmPlan& P, bool sym, int chunk) {
+    CU(cudaSetDevice(d.device));
+    const int n = (int)P.fr.size();
+    bool code_seen[kNumCodes] = {}, cfg_seen[kVcmConfigs] = {};
+    for (const VcmDesc& f : P.fr)
+        if (f.code >= 0) code_seen[f.code] = cfg_seen[f.cfg] = true;
+    for (int ci = 0; ci < kNumCodes; ++ci) {
+        if (!code_seen[ci]) continue;
+        if (!d.vcm_codes.count(ci)) {
+            const LdpcCode& c = ldpc_code(ci);
+            CodeTables& T = d.vcm_codes[ci];
+            for (const LayerLink& l : c.links) T.links.push_back(((uint32_t)l.group << 16) | l.shift);
+            T.hard_stride = ((c.K / 8) + 15) & ~15;
+            int rc = prepare_ldpc(d, c, T.links.data(), T.ldpc, T.grid);
+            if (!rc) rc = prepare_bch(d, c, T.bch);
+            if (rc) {
+                ldpc_release(T.ldpc);
+                d.vcm_codes.erase(ci);
+                return rc;
+            }
+        }
+        const CodeTables& T = d.vcm_codes[ci];
+        P.workspace = std::max(P.workspace, (size_t)T.grid * ldpc_workspace_bytes(T.ldpc));
+    }
+    if (sym) {
+        CU(d.vcm_demap.reserve(kVcmConfigs));
+        for (int cfg = 0; cfg < kVcmConfigs; ++cfg) {
+            if (!cfg_seen[cfg] || d.vcm_demap_ok[cfg]) continue;
+            ModcodCfg mc;
+            modcod_config(cfg / 4, (cfg & 2) != 0, (cfg & 1) != 0, &mc);
+            const LdpcCode& c = ldpc_code(mc.code);
+            const int nsym = c.N / mc.bits;
+            DemapDev D{};
+            if (int rc = prepare_demap(d, mc, c, 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0), nullptr, D)) return rc;
+            CU(cudaMemcpy(d.vcm_demap.p + cfg, &D, sizeof D, cudaMemcpyHostToDevice));
+            CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+            d.vcm_demap_ok[cfg] = true;
+        }
+    }
+    P.rec.resize(n);
+    for (int f0 = 0; f0 < n; f0 += chunk) {
+        VcmChunk c{f0, std::min(n, f0 + chunk), false, 0, 0, {}};
+        int gi[kNumCodes];
+        std::fill(gi, gi + kNumCodes, -1);
+        bool dummy = false;
+        for (int f = c.f0; f < c.f1; ++f) {
+            const int code = P.fr[f].code;
+            if (code < 0) {
+                dummy = true;
+                continue;
+            }
+            if (gi[code] < 0) {
+                gi[code] = (int)c.groups.size();
+                c.groups.push_back(VcmGroup{code, 0, 0, 0, 0, 0});
+            }
+            ++c.groups[gi[code]].cnt;
+        }
+        std::stable_sort(c.groups.begin(), c.groups.end(), [](const VcmGroup& a, const VcmGroup& b) { return a.cnt > b.cnt; });
+        c.fast = c.groups.size() == 1 && !dummy;
+        size_t lo = 0, ho = 0, bo = 0;
+        int p = 0;
+        for (size_t g = 0; g < c.groups.size(); ++g) {
+            VcmGroup& G = c.groups[g];
+            const LdpcCode& lc = ldpc_code(G.code);
+            gi[G.code] = (int)g;
+            G.p0 = p;
+            G.llr_off = lo;
+            G.hard_off = ho;
+            G.bb_off = bo;
+            lo += align256((size_t)G.cnt * lc.N);
+            ho += (size_t)G.cnt * d.vcm_codes[G.code].hard_stride;
+            bo += align256((size_t)G.cnt * (lc.kbch / 8));
+            p += G.cnt;
+        }
+        int fill[kNumCodes] = {};
+        for (int f = c.f0; f < c.f1; ++f) {
+            const VcmDesc& D = P.fr[f];
+            VcmFrame& r = P.rec[f];
+            r.in_off = sym ? P.sym_off[f] : P.llr_off[f];
+            r.bb_dst = P.bb_off[f];
+            r.cfg = D.cfg;
+            r.nbytes = D.N;
+            r.kb = D.kb;
+            r.pos = -1;
+            r.llr_off = r.bb_src = 0;
+            if (D.code < 0) continue;
+            const VcmGroup& G = c.groups[gi[D.code]];
+            const int i = fill[D.code]++;
+            r.pos = G.p0 + i;
+            r.llr_off = (long long)(G.llr_off + (size_t)i * D.N);
+            r.bb_src = (long long)(G.bb_off + (size_t)i * D.kb);
+            c.nsym_max = std::max(c.nsym_max, D.nsym);
+            c.n_max = std::max(c.n_max, D.N);
+        }
+        if (sym || !c.fast) P.llr_bytes = std::max(P.llr_bytes, lo);   // a fast chunk of LLRs is decoded where it lies
+        P.hard_bytes = std::max(P.hard_bytes, ho);
+        P.bb_bytes = std::max(P.bb_bytes, bo);
+        P.in_max = std::max(P.in_max, sym ? (size_t)(P.sym_off[c.f1] - P.sym_off[c.f0]) * 8 : (size_t)(P.llr_off[c.f1] - P.llr_off[c.f0]));
+        P.out_max = std::max(P.out_max, (size_t)(P.bb_off[c.f1] - P.bb_off[c.f0]));
+        P.max_chunk = std::max(P.max_chunk, c.f1 - c.f0);
+        P.chunks.push_back(std::move(c));
+    }
+    return 0;
+}
+
+// scratch of slot s for the plan; host: also the staging of the chunk's input and output, records per chunk
+int vcm_reserve(Slot& s, const VcmPlan& P, bool host) {
+    CU(s.llr.reserve(P.llr_bytes));
+    CU(s.hard.reserve(P.hard_bytes));
+    CU(s.iters.reserve(P.max_chunk));
+    CU(s.bb.reserve(P.bb_bytes));
+    CU(s.res.reserve(P.max_chunk));
+    CU(s.workspace.reserve(P.workspace));
+    CU(s.counter.reserve(kNumCodes));
+    const size_t nrec = host ? (size_t)P.max_chunk : P.rec.size();
+    CU(s.vmeta.reserve(nrec));
+    CU(s.h_vmeta.reserve(nrec));
+    if (host) {
+        CU(s.vin.reserve(P.in_max));
+        CU(s.vbb.reserve(P.out_max));
+        CU(s.vres.reserve(P.max_chunk));
+        CU(s.h_in.reserve(P.in_max));
+        CU(s.h_bb.reserve(P.out_max));
+        CU(s.h_res.reserve(P.max_chunk));
+    }
+    return 0;
+}
+
+// Enqueues one chunk on st.  in: the input, in_off - in_shift indexes it (complex samples or bytes); rec: the chunk's
+// records on the device; bb_out / res_out: BBFRAMEs at bb_off - bb_shift and the records of frames f0.. (may be null).
+// Launches: demap or gather (unless the chunk is a fast one of LLRs, or all dummy), LDPC and BCH per code, scatter
+// (unless fast): 2k + 2 for k codes, 2 / 3 for a fast chunk of LLRs / symbols, 1 for a chunk of dummy frames.
+int vcm_chunk(dvbs2fec_handle* h, DevCtx& d, Slot& s, const VcmPlan& P, const VcmChunk& c, bool sym, const void* in,
+              long long in_shift, const VcmFrame* rec, uint8_t* bb_out, long long bb_shift, dvbs2fec_result* res_out,
+              cudaStream_t st, int* launches) {
+    SpanMark mark{h, st};
+    const int m = c.f1 - c.f0;
+    const int8_t* llr = s.llr.p;
+    if (!c.groups.empty()) {
+        int e = 0;
+        if (sym) {
+            mark(0, true);
+            e = demap_vcm_launch(d.vcm_demap.p, h->pl_codenum >= 0 ? d.pl_rn.p : nullptr, static_cast<const float*>(in), in_shift,
+                                 rec, m, c.nsym_max, s.llr.p, st);
+            mark(0, false);
+            ++*launches;
+        } else if (!c.fast) {
+            mark(0, true);
+            e = vcm_gather_launch(static_cast<const int8_t*>(in), in_shift, rec, m, c.n_max, s.llr.p, st);
+            mark(0, false);
+            ++*launches;
+        } else {
+            llr = static_cast<const int8_t*>(in) + (P.llr_off[c.f0] - in_shift);
+        }
+        if (e) return fail(DVBS2FEC_ECUDA, "VCM demap / gather launch: %s", cudaGetErrorString((cudaError_t)e));
+        CU(cudaMemsetAsync(s.counter.p, 0, c.groups.size() * sizeof(unsigned int), st));
+    }
+    for (size_t g = 0; g < c.groups.size(); ++g) {
+        const VcmGroup& G = c.groups[g];
+        const CodeTables& T = d.vcm_codes.at(G.code);
+        LdpcArgs la{};
+        la.code = T.ldpc;
+        la.llr_in = llr + G.llr_off;
+        la.nframes = G.cnt;
+        la.max_trials = h->max_trials;
+        la.hard_out = s.hard.p + G.hard_off;
+        la.hard_stride = T.hard_stride;
+        la.iters_out = s.iters.p + G.p0;
+        la.workspace = s.workspace.p;
+        la.work_counter = s.counter.p + g;
+        mark(1, true);
+        int e = ldpc_launch(la, std::min(T.grid, (G.cnt + 1) / 2), st);
+        mark(1, false);
+        if (e) return fail(DVBS2FEC_ECUDA, "ldpc launch: %s", cudaGetErrorString((cudaError_t)e));
+        ++*launches;
+        BchArgs ba{};
+        ba.code = T.bch;
+        ba.hard = s.hard.p + G.hard_off;
+        ba.hard_stride = T.hard_stride;
+        ba.nframes = G.cnt;
+        ba.ldpc_iters = s.iters.p + G.p0;
+        ba.descramble = 1;
+        if (c.fast) {   // input order: straight into the caller's buffers
+            ba.tag_base = (unsigned long long)c.f0;
+            ba.bb_out = bb_out ? bb_out + (P.bb_off[c.f0] - bb_shift) : nullptr;
+            ba.results = res_out;
+        } else {
+            ba.bb_out = s.bb.p + G.bb_off;
+            ba.results = s.res.p + G.p0;
+        }
+        mark(2, true);
+        e = bch_launch(ba, st);
+        mark(2, false);
+        if (e) return fail(DVBS2FEC_ECUDA, "bch launch: %s", cudaGetErrorString((cudaError_t)e));
+        ++*launches;
+    }
+    if (!c.fast) {
+        mark(2, true);
+        int e = vcm_scatter_launch(rec, m, s.bb.p, s.res.p, bb_out, bb_shift, res_out, (unsigned long long)c.f0, st);
+        mark(2, false);
+        if (e) return fail(DVBS2FEC_ECUDA, "VCM scatter launch: %s", cudaGetErrorString((cudaError_t)e));
+        ++*launches;
+    }
+    return 0;
+}
+
+// host buffers: chunk by chunk through the two synchronous slots, like run_device_share (no streamed input)
+int vcm_host(dvbs2fec_handle* h, int n, const int32_t* desc, const void* in, bool sym, uint8_t* bb, dvbs2fec_result* res) {
+    if (!h) return fail(DVBS2FEC_EINVAL, "handle is NULL");
+    VcmPlan P;
+    if (int rc = vcm_parse(n, desc, P)) return rc;
+    if (!in && (sym ? P.sym_off[n] : P.llr_off[n]) > 0) return fail(DVBS2FEC_EINVAL, "input is NULL");
+    if (h->devs.empty()) return fail(DVBS2FEC_ENODEV, "no CUDA device");
+    h->last_launches = 0;
+    if (n == 0) return 0;
+    DevCtx& d = *h->devs[0];
+    if (int rc = vcm_plan(h, d, P, sym, std::max(h->cfg.max_batch, 1))) return rc;
+    for (int k = 0; k < kSlots; ++k)
+        if (int rc = vcm_reserve(d.slot[k], P, true)) return rc;
+    const bool pin_in = is_pinned(in);
+    const bool pin_out = (!bb || is_pinned(bb)) && (!res || is_pinned(res));
+    const std::vector<int64_t>& in_off = sym ? P.sym_off : P.llr_off;
+    const size_t unit = sym ? 8 : 1;
+    int which = 0, rc = 0, launches = 0;
+    HostSlotsAbort abort_guard{d};
+    for (const VcmChunk& c : P.chunks) {
+        Slot& s = d.slot[which];
+        which ^= 1;
+        const int m = c.f1 - c.f0;
+        if ((rc = finish_slot(h, s))) return rc;
+        const size_t in_bytes = (size_t)(in_off[c.f1] - in_off[c.f0]) * unit;
+        const uint8_t* src = static_cast<const uint8_t*>(in) + (size_t)in_off[c.f0] * unit;
+        if (!pin_in && in_bytes) {
+            memcpy(s.h_in.p, src, in_bytes);
+            src = s.h_in.p;
+        }
+        if (in_bytes) CU(cudaMemcpyAsync(s.vin.p, src, in_bytes, cudaMemcpyHostToDevice, s.stream));
+        if (sym || !c.fast) {
+            memcpy(s.h_vmeta.p, &P.rec[c.f0], (size_t)m * sizeof(VcmFrame));
+            CU(cudaMemcpyAsync(s.vmeta.p, s.h_vmeta.p, (size_t)m * sizeof(VcmFrame), cudaMemcpyHostToDevice, s.stream));
+        }
+        rc = vcm_chunk(h, d, s, P, c, sym, s.vin.p, in_off[c.f0], s.vmeta.p, bb ? s.vbb.p : nullptr, P.bb_off[c.f0],
+                       res ? s.vres.p : nullptr, s.stream, &launches);
+        if (rc) return rc;
+        const size_t out_bytes = (size_t)(P.bb_off[c.f1] - P.bb_off[c.f0]);
+        s.user_bb = bb ? bb + P.bb_off[c.f0] : nullptr;
+        s.user_res = res ? res + c.f0 : nullptr;
+        s.staged_out = !pin_out;
+        if (bb && out_bytes) CU(cudaMemcpyAsync(pin_out ? s.user_bb : s.h_bb.p, s.vbb.p, out_bytes, cudaMemcpyDeviceToHost, s.stream));
+        if (res)
+            CU(cudaMemcpyAsync(pin_out ? (void*)s.user_res : (void*)s.h_res.p, s.vres.p, (size_t)m * sizeof(dvbs2fec_result),
+                               cudaMemcpyDeviceToHost, s.stream));
+        CU(cudaEventRecord(s.done, s.stream));
+        s.tag_base = (uint64_t)c.f0;
+        s.pending = m;
+        s.bb_bytes = out_bytes;
+    }
+    for (int k = 0; k < kSlots; ++k)
+        if ((rc = finish_slot(h, d.slot[k]))) return rc;
+    abort_guard.armed = false;
+    h->last_launches = launches;
+    return 0;
+}
+
+// device buffers: the device entry point's slot, lock and event chaining (dvbs2fec_decode_batch_device)
+int vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const void* d_in, bool sym, uint8_t* d_bb,
+               dvbs2fec_result* d_res, void* cuda_stream) {
+    if (!h) return fail(DVBS2FEC_EINVAL, "handle is NULL");
+    VcmPlan P;
+    if (int rc = vcm_parse(n, desc, P)) return rc;
+    if (!d_in && (sym ? P.sym_off[n] : P.llr_off[n]) > 0) return fail(DVBS2FEC_EINVAL, "input is NULL");
+    if (h->devs.empty()) return fail(DVBS2FEC_ENODEV, "no CUDA device");
+    DevCtx& d = *h->devs[0];
+    Slot& s = d.slot[2 * kSlots];
+    std::lock_guard<std::mutex> serial(d.dev_mu);
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    h->last_launches = 0;
+    if (n == 0) return 0;
+    if (int rc = vcm_plan(h, d, P, sym, std::max(h->cfg.max_batch, 1))) return rc;
+    // the records go out of a page-locked buffer that the previous call's copy may still be reading
+    if (s.vmeta_copying) CU(cudaEventSynchronize(s.armed));
+    s.vmeta_copying = false;
+    if (int rc = vcm_reserve(s, P, false)) return rc;
+    if (d.dev_used) CU(cudaStreamWaitEvent(st, s.done, 0));
+    bool need_rec = sym;
+    for (const VcmChunk& c : P.chunks) need_rec |= !c.fast;
+    if (need_rec) {
+        memcpy(s.h_vmeta.p, P.rec.data(), (size_t)n * sizeof(VcmFrame));
+        CU(cudaMemcpyAsync(s.vmeta.p, s.h_vmeta.p, (size_t)n * sizeof(VcmFrame), cudaMemcpyHostToDevice, st));
+        CU(cudaEventRecord(s.armed, st));
+        s.vmeta_copying = true;
+    }
+    int rc = 0;
+    for (size_t k = 0; k < P.chunks.size() && !rc; ++k) {
+        const VcmChunk& c = P.chunks[k];
+        rc = vcm_chunk(h, d, s, P, c, sym, d_in, 0, s.vmeta.p + c.f0, d_bb, 0, d_res ? d_res + c.f0 : nullptr, st,
+                       &h->last_launches);
+    }
+    CU(cudaEventRecord(s.done, st));
+    d.dev_used = true;
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -798,6 +1205,7 @@ void dvbs2fec_destroy(dvbs2fec_handle* h) {
             s.bb.release(); s.res.release(); s.workspace.release(); s.counter.release();
             s.h_in.release(); s.h_bb.release(); s.h_res.release();
             s.arrived.release(); s.arrived_vals.release();
+            s.vin.release(); s.vbb.release(); s.vres.release(); s.vmeta.release(); s.h_vmeta.release();
             s.ts.release(); s.ts_len.release();
             if (s.done) cudaEventDestroy(s.done);
             if (s.armed) cudaEventDestroy(s.armed);
@@ -807,6 +1215,7 @@ void dvbs2fec_destroy(dvbs2fec_handle* h) {
         for (auto& kv : d.codes) kv.second.row_level.release();
         for (auto& kv : d.bch) { kv.second.crc.release(); kv.second.basis.release(); }
         for (auto& kv : d.luts) kv.second.release();
+        d.vcm_demap.release();
         for (int i = 0; i < 2; ++i) { d.gf_log[i].release(); d.gf_exp[i].release(); }
         d.prbs.release();
         d.pl_rn.release();
@@ -1090,6 +1499,31 @@ int dvbs2fec_decode_plframes_device(dvbs2fec_handle* h, const float* d_plframes,
     CU(cudaEventRecord(s.done, st));
     d.dev_used = true;
     return rc;
+}
+
+int dvbs2fec_vcm_layout(int n, const int32_t* desc, int64_t* sym_off, int64_t* llr_off, int64_t* bb_off) {
+    VcmPlan P;
+    if (int rc = vcm_parse(n, desc, P)) return rc;
+    if (sym_off) std::copy(P.sym_off.begin(), P.sym_off.end(), sym_off);
+    if (llr_off) std::copy(P.llr_off.begin(), P.llr_off.end(), llr_off);
+    if (bb_off) std::copy(P.bb_off.begin(), P.bb_off.end(), bb_off);
+    return 0;
+}
+int dvbs2fec_decode_vcm(dvbs2fec_handle* h, int n, const int32_t* desc, const int8_t* llr, uint8_t* bb_out,
+                        dvbs2fec_result* results) {
+    return vcm_host(h, n, desc, llr, false, bb_out, results);
+}
+int dvbs2fec_decode_plframes_vcm(dvbs2fec_handle* h, int n, const int32_t* desc, const float* plframes, uint8_t* bb_out,
+                                 dvbs2fec_result* results) {
+    return vcm_host(h, n, desc, plframes, true, bb_out, results);
+}
+int dvbs2fec_decode_vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const int8_t* d_llr, uint8_t* d_bb_out,
+                               dvbs2fec_result* d_results, void* cuda_stream) {
+    return vcm_device(h, n, desc, d_llr, false, d_bb_out, d_results, cuda_stream);
+}
+int dvbs2fec_decode_plframes_vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const float* d_plframes,
+                                        uint8_t* d_bb_out, dvbs2fec_result* d_results, void* cuda_stream) {
+    return vcm_device(h, n, desc, d_plframes, true, d_bb_out, d_results, cuda_stream);
 }
 
 // Copy into a staging batch with non-temporal stores: the CPU never reads these bytes again (the copy engine does), so
