@@ -122,13 +122,14 @@ struct dvbs2fec_plsync {
     Buf<PlHdrState> hst;
     Buf<PlHdrResult> hres;
     Buf<PlTables> tab;
-    Buf<uint8_t> rn;
+    Buf<uint8_t> rn;           // the coarse FED's PL scrambling sequence, of Gold code rn_codenum
     int rn_codenum = -2;
     PlSyncState h_st{};
     // S2PLLBlock (K8)
     Buf<PllState> pst;
     Buf<float> perr, pll_state;
     Buf<float2> pll_in, pll_out;
+    Buf<uint8_t> pll_rn;       // the loop's own sequence: a FED call with another code must not change what a queued loop reads
     Buf<uint8_t> pll_jobs;
     PllArgs pll{};            // configuration part; buffers are filled in per call
     bool pll_ready = false;
@@ -174,7 +175,8 @@ void dvbs2fec_plsync_destroy(dvbs2fec_plsync* p) {
     p->work[0].release(); p->work[1].release(); p->out.release(); p->frames_in.release(); p->hdr_out.release();
     p->metric.release(); p->fed_out.release(); p->starts.release(); p->st.release(); p->hst.release(); p->hres.release();
     p->tab.release(); p->rn.release();
-    p->pst.release(); p->perr.release(); p->pll_state.release(); p->pll_in.release(); p->pll_out.release(); p->pll_jobs.release();
+    p->pst.release(); p->perr.release(); p->pll_state.release(); p->pll_in.release(); p->pll_out.release(); p->pll_rn.release();
+    p->pll_jobs.release();
     delete p;
 }
 
@@ -381,9 +383,14 @@ int dvbs2fec_pll_set_params(dvbs2fec_plsync* p, float loop_bw, int modcod, int s
     if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
     ModcodCfg cfg;
     if (!modcod_config(modcod, shortframes != 0, pilots != 0, &cfg)) return api_fail(DVBS2FEC_EINVAL, "modcod outside 1..28");
+    if (codenum < 0 || codenum > 262141) return api_fail(DVBS2FEC_EINVAL, "Gold code number outside 0..262141");
     CU(cudaSetDevice(p->device));
-    int rc = fed_tables(p, 1, codenum);   // the loop descrambles every payload symbol, pilots or not
-    if (rc) return rc;
+    {   // the loop descrambles every payload symbol, pilots or not
+        const std::vector<uint8_t> rn = pl_scrambling_rn(codenum, 131072);
+        CU(p->pll_rn.reserve(rn.size()));
+        CU(cudaMemcpy(p->pll_rn.p, rn.data(), rn.size(), cudaMemcpyHostToDevice));
+        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    }
     // PhaseControlLoop<float>::criticallyDamped(loop_bw, alpha, beta) (dvbs2_pll.cpp:10)
     PllState s{};
     CU(cudaMemcpy(&s, p->pst.p, sizeof s, cudaMemcpyDeviceToHost));
@@ -424,7 +431,7 @@ int dvbs2fec_pll_set_params(dvbs2fec_plsync* p, float loop_bw, int modcod, int s
         CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
         a.perr_lut = p->perr.p;
     }
-    a.rn = p->rn.p;
+    a.rn = p->pll_rn.p;
     a.tab = p->tab.p;
     a.st = p->pst.p;
     p->pll_ready = true;
