@@ -276,10 +276,8 @@ int prepare_ldpc(DevCtx& d, const LdpcCode& c, const uint32_t* links, LdpcDev& L
     L.N = c.N; L.K = c.K; L.R = c.R; L.q = c.q;
     L.ngroups = c.K / kGroup;
     L.max_cnt = c.max_cnt;
-    L.v2 = ldpc_use_v2(c.index);
-    L.lanes2 = L.v2 && ldpc_use_lanes2(c.index) && ldpc_slot_groups_for(c.max_cnt, true) > 0;
+    L.lanes2 = ldpc_use_lanes2(c.index) && ldpc_slot_groups_for(c.max_cnt, true) > 0;
     L.sg = ldpc_slot_groups_for(c.max_cnt, L.lanes2);
-    L.chains = !L.v2 && ldpc_chains_pay_off(c.index);
     L.occ3 = ldpc_ctas_wanted3(c.index);
     if (!L.sg) return fail(DVBS2FEC_EINVAL, "no LDPC kernel for %d links per row", c.max_cnt);
     L.links = links;

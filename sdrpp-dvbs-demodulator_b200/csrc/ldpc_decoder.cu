@@ -1,4 +1,4 @@
-// K2 host side -- see ldpc_decoder.cuh for the interface and ldpc_v2.cuh / ldpc_kernels.cuh for the kernels.
+// K2 host side -- see ldpc_decoder.cuh for the interface and ldpc_v2.cuh / ldpc_v2l.cuh for the kernels.
 // Reference semantics: SURVEY.md spec S-LDPC (layered_decoder.hh:23-74,121-133; algorithms.hh:235-256,261-276;
 // bbframe_ldpc.cpp:123-139).
 #include "ldpc_decoder.cuh"
@@ -14,11 +14,8 @@ namespace s2 {
 
 // Everything a launch needs that depends only on the configured code: built by ldpc_prepare, read by ldpc_launch.
 struct LdpcPlan {
-    bool v2 = false;
-    int threads = kLdpcThreads;
-    KernelFn fn1[2] = {nullptr, nullptr};    // [streamed]
-    KernelFn2 fn2[2] = {nullptr, nullptr};
-    LdpcParams p1;
+    int threads = 0;
+    KernelFn2 fn2[2] = {nullptr, nullptr};   // [streamed]
     LdpcParams2 p2;
     size_t smem = 0;
 };
@@ -30,14 +27,6 @@ int env_int(const char* name, int dflt) {
     return e ? atoi(e) : dflt;
 }
 
-const Variant* pick(int max_cnt) {
-    const Variant* parts[4] = {kLdpcVariantsA, kLdpcVariantsB, kLdpcVariantsC, kLdpcVariantsD};
-    const int counts[4] = {kLdpcVariantsA_n, kLdpcVariantsB_n, kLdpcVariantsC_n, kLdpcVariantsD_n};
-    for (int k = 0; k < 4; ++k)
-        for (int i = 0; i < counts[k]; ++i)
-            if (parts[k][i].cnt >= max_cnt) return &parts[k][i];
-    return nullptr;
-}
 const Variant2* pick2(int max_cnt) {
     const Variant2* parts[4] = {kLdpc2VariantsA, kLdpc2VariantsB, kLdpc2VariantsC, kLdpc2VariantsD};
     const int counts[4] = {kLdpc2VariantsA_n, kLdpc2VariantsB_n, kLdpc2VariantsC_n, kLdpc2VariantsD_n};
@@ -58,12 +47,6 @@ bool is_uniform(const LdpcDev& c, int cnt) {
     bool uniform = cnt == c.max_cnt;
     for (int i = 0; i < c.q && uniform; ++i) uniform = (c.layer_off[i + 1] - c.layer_off[i]) == cnt;
     return uniform;
-}
-KernelFn pick_fn(const LdpcDev& c, bool streamed) {
-    const Variant* v = pick(c.max_cnt);
-    if (!v) return nullptr;
-    const int ch = c.chains ? 1 : 0, oc = c.occ3 ? 1 : 0;
-    return (is_uniform(c, v->cnt) && v->uniform[0][0][0]) ? v->uniform[streamed][ch][oc] : v->ragged[streamed][ch][oc];
 }
 KernelFn2 pick_fn2(const LdpcDev& c, bool streamed) {
     if (c.lanes2) {
@@ -122,51 +105,7 @@ void plan_barriers(const LdpcDev& c, uint8_t* layer_sync) {
     if (!any) layer_sync[0] = 1;            // pty[q-1][j-1]: stored in layer 0, read (by thread j-1) in layer q-1 / prefetched in q-2
 }
 
-// Chained layers (first-generation kernel): exactly one 360-bit group is hit by exactly two links of the layer (they
-// are adjacent, links are sorted by group).  X is the one whose bit the EARLIER row of a pair owns: row j's X bit is
-// row j+d's Y bit with d = (shift_Y - shift_X) mod 360 <= 180.
-void plan_chains(const LdpcDev& c, uint16_t* layer_chain) {
-    // a chained layer costs about two extra passes over the rows; below this many levels the level loop is cheaper
-    static const int min_levels = env_int("DVBS2FEC_CHAIN_MINLEV", 8);
-    for (int i = 0; i < c.q; ++i) {
-        layer_chain[i] = 0;
-        if (!c.chains || (int)c.layer_nlev[i] < min_levels) continue;
-        int pairs = 0, first = -1;
-        bool simple = true;
-        for (int k = c.layer_off[i]; k + 1 < c.layer_off[i + 1]; ++k) {
-            if ((c.links[k] >> 16) != (c.links[k + 1] >> 16)) continue;
-            if (k + 2 < c.layer_off[i + 1] && (c.links[k + 2] >> 16) == (c.links[k] >> 16)) simple = false;   // three in a group
-            ++pairs;
-            first = k - c.layer_off[i];
-        }
-        if (!simple || pairs != 1 || first > 30) continue;
-        const int s0 = (int)(c.links[c.layer_off[i] + first] & 0xFFFFu), s1 = (int)(c.links[c.layer_off[i] + first + 1] & 0xFFFFu);
-        int d = ((s1 - s0) % 360 + 360) % 360, orient = 0;   // X = first, Y = first + 1
-        if (d > 180) {
-            d = 360 - d;
-            orient = 1;                                      // X = first + 1, Y = first
-        }
-        if (d == 0) continue;
-        layer_chain[i] = (uint16_t)(0x8000u | (unsigned)d << 6 | (unsigned)orient << 5 | (unsigned)first);
-    }
-}
-
 }  // namespace
-
-// Codes for which the three-phase treatment of chained layers beats the level-by-level one (first-generation kernel).
-// Measured with tools/modcod_sweep.py (2048 normal / 8192 short frames, fixed noise) against the same kernel without it:
-// n1/3 -9 %, n2/3 -3..-6 %, n3/4 -12 %, n8/9 -20 %, s2/5 -12 %, s1/2 -3 %, s2/3 -9 % time (s3/4 -10 %, but it
-// gains more from a second CTA with the lean row update, which has no chained mode); within +-2 %
-// or slower for the others (few layers with many levels, or their other conflicted layers dominate; for n1/2
-// the co-resident CTA already hides the level steps at full load).  Only layers with at least eight levels are
-// chained: the three phases cost about two extra passes over the rows.  Index = code table order B1..B11, C1..C10.
-bool ldpc_chains_pay_off(int code_index) {
-    static const bool table[21] = {false, true,  false, false, false, true,  true,  false, false, true,  false,
-                                   false, false, true,  true,  false, true,  false, false, false, false};
-    static const int force = env_int("DVBS2FEC_LDPC_CHAINS", -1);
-    if (force >= 0) return force != 0;
-    return code_index >= 0 && code_index < 21 && table[code_index];
-}
 
 // Codes that run faster with one more resident CTA per SM than the default and the register allocation squeezed
 // accordingly (three CTAs / 56 registers for CNT <= 9, two CTAs / 80 registers above): their shared memory
@@ -179,21 +118,11 @@ bool ldpc_ctas_wanted3(int code_index) {
     return code_index >= 0 && code_index < 21 && table[code_index];
 }
 
-// Codes served by the second-generation kernel.  DVBS2FEC_LDPC_V2=0|1 overrides for every code (re-measuring).
-bool ldpc_use_v2(int code_index) {
-    static const bool table[21] = {true, true, true, true, true, true, true, true, true, true, true,
-                                   true, true, true, true, true, true, true, true, true, true};
-    static const int force = env_int("DVBS2FEC_LDPC_V2", -1);
-    if (force >= 0) return force != 0;
-    return code_index >= 0 && code_index < 21 && table[code_index];
-}
-
-int ldpc_slot_groups(int max_cnt) {
-    const Variant* v = pick(max_cnt);
-    return v ? (v->cnt + 2 + 7) / 8 : 0;
-}
 int ldpc_slot_groups_for(int max_cnt, bool lanes2) {
-    if (!lanes2) return ldpc_slot_groups(max_cnt);
+    if (!lanes2) {
+        const Variant2* v = pick2(max_cnt);
+        return v ? (v->cnt + 2 + 7) / 8 : 0;
+    }
     if (!pickl(max_cnt)) return 0;
     const int dh = (max_cnt + 1) / 2 + 1;     // slots per half row
     return 2 * ((dh + 7) / 8);
@@ -218,51 +147,29 @@ int ldpc_prepare(LdpcDev& c) {
     const int nlinks = c.layer_off[c.q];
     if (nlinks > kMaxLinks) return (int)cudaErrorInvalidValue;
     LdpcPlan* pl = new LdpcPlan();
-    pl->v2 = c.v2;
-    cudaError_t e = cudaSuccess;
-    if (c.v2) {
-        pl->fn2[0] = pick_fn2(c, false);
-        pl->fn2[1] = pick_fn2(c, true);
-        pl->threads = c.lanes2 ? 720 : 360;   // v2::kLdpcThreads2 / v2::kThreads
-        if (!pl->fn2[0] || !pl->fn2[1] || ldpc_slot_groups_for(c.max_cnt, c.lanes2) != c.sg) {
-            delete pl;
-            return (int)cudaErrorInvalidValue;
-        }
-        LdpcParams2& p = pl->p2;
-        memset(&p, 0, sizeof(p));
-        p.N = c.N; p.K = c.K; p.R = c.R; p.q = c.q; p.ngroups = c.ngroups; p.sg = c.sg;
-        p.ws_stride = ldpc_workspace_bytes(c);
-        p.row_level = c.row_level;
-        p.wait_budget = (long long)env_int("DVBS2FEC_STREAM_WAIT_S", 20) * 2000000000ll;
-        for (int i = 0; i <= c.q; ++i) p.layer_off[i] = (uint16_t)c.layer_off[i];
-        for (int i = 0; i < c.q; ++i) p.layer_nlev[i] = c.layer_nlev[i];
-        plan_barriers(c, p.layer_sync);
-        for (int i = 0; i < nlinks; ++i) {
-            const uint32_t g = c.links[i] >> 16, sh = c.links[i] & 0xFFFFu;
-            p.link_group[i] = (uint8_t)g;
-            p.link_add[i] = (uint16_t)(720u - 2u * sh);
-        }
-        for (int st = 0; st < 2 && e == cudaSuccess; ++st) e = allow_max_smem(pl->fn2[st]);
-    } else {
-        const Variant* v = pick(c.max_cnt);
-        pl->fn1[0] = pick_fn(c, false);
-        pl->fn1[1] = pick_fn(c, true);
-        if (!v || !pl->fn1[0] || !pl->fn1[1] || (v->cnt + 2 + 7) / 8 != c.sg) {
-            delete pl;
-            return (int)cudaErrorInvalidValue;
-        }
-        LdpcParams& p = pl->p1;
-        memset(&p, 0, sizeof(p));
-        p.N = c.N; p.K = c.K; p.R = c.R; p.q = c.q; p.ngroups = c.ngroups; p.sg = c.sg;
-        p.ws_stride = ldpc_workspace_bytes(c);
-        p.row_level = c.row_level;
-        for (int i = 0; i <= c.q; ++i) p.layer_off[i] = (uint16_t)c.layer_off[i];
-        for (int i = 0; i < c.q; ++i) p.layer_nlev[i] = c.layer_nlev[i];
-        plan_barriers(c, p.layer_sync);
-        for (int i = 0; i < nlinks; ++i) p.links[i] = c.links[i];
-        plan_chains(c, p.layer_chain);
-        for (int st = 0; st < 2 && e == cudaSuccess; ++st) e = allow_max_smem(pl->fn1[st]);
+    pl->fn2[0] = pick_fn2(c, false);
+    pl->fn2[1] = pick_fn2(c, true);
+    pl->threads = c.lanes2 ? 720 : 360;   // v2::kLdpcThreads2 / v2::kThreads
+    if (!pl->fn2[0] || !pl->fn2[1] || ldpc_slot_groups_for(c.max_cnt, c.lanes2) != c.sg) {
+        delete pl;
+        return (int)cudaErrorInvalidValue;
     }
+    LdpcParams2& p = pl->p2;
+    memset(&p, 0, sizeof(p));
+    p.N = c.N; p.K = c.K; p.R = c.R; p.q = c.q; p.ngroups = c.ngroups; p.sg = c.sg;
+    p.ws_stride = ldpc_workspace_bytes(c);
+    p.row_level = c.row_level;
+    p.wait_budget = (long long)env_int("DVBS2FEC_STREAM_WAIT_S", 20) * 2000000000ll;
+    for (int i = 0; i <= c.q; ++i) p.layer_off[i] = (uint16_t)c.layer_off[i];
+    for (int i = 0; i < c.q; ++i) p.layer_nlev[i] = c.layer_nlev[i];
+    plan_barriers(c, p.layer_sync);
+    for (int i = 0; i < nlinks; ++i) {
+        const uint32_t g = c.links[i] >> 16, sh = c.links[i] & 0xFFFFu;
+        p.link_group[i] = (uint8_t)g;
+        p.link_add[i] = (uint16_t)(720u - 2u * sh);
+    }
+    cudaError_t e = cudaSuccess;
+    for (int st = 0; st < 2 && e == cudaSuccess; ++st) e = allow_max_smem(pl->fn2[st]);
     if (e != cudaSuccess) {
         delete pl;
         return (int)e;
@@ -280,10 +187,7 @@ void ldpc_release(LdpcDev& c) {
 int ldpc_max_ctas_per_sm(const LdpcDev& c) {
     if (!c.plan) return 0;
     int n = 0;
-    if (c.plan->v2)
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, c.plan->fn2[0], c.plan->threads, c.plan->smem);
-    else
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, c.plan->fn1[0], kLdpcThreads, c.plan->smem);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, c.plan->fn2[0], c.plan->threads, c.plan->smem);
     return n;
 }
 
@@ -291,19 +195,11 @@ int ldpc_launch(const LdpcArgs& a, int grid, cudaStream_t stream) {
     const LdpcPlan* pl = a.code.plan;
     if (!pl) return (int)cudaErrorInvalidValue;
     const int st = a.arrived ? 1 : 0;
-    if (pl->v2) {
-        LdpcParams2 p = pl->p2;
-        p.nframes = a.nframes; p.max_trials = a.max_trials; p.hard_stride = a.hard_stride;
-        p.llr_in = a.llr_in; p.hard_out = a.hard_out; p.iters_out = a.iters_out; p.llr_out = a.llr_out;
-        p.workspace = a.workspace; p.work_counter = a.work_counter; p.arrived = a.arrived;
-        pl->fn2[st]<<<grid, pl->threads, pl->smem, stream>>>(p);
-    } else {
-        LdpcParams p = pl->p1;
-        p.nframes = a.nframes; p.max_trials = a.max_trials; p.hard_stride = a.hard_stride;
-        p.llr_in = a.llr_in; p.hard_out = a.hard_out; p.iters_out = a.iters_out; p.llr_out = a.llr_out;
-        p.workspace = a.workspace; p.work_counter = a.work_counter; p.arrived = a.arrived;
-        pl->fn1[st]<<<grid, kLdpcThreads, pl->smem, stream>>>(p);
-    }
+    LdpcParams2 p = pl->p2;
+    p.nframes = a.nframes; p.max_trials = a.max_trials; p.hard_stride = a.hard_stride;
+    p.llr_in = a.llr_in; p.hard_out = a.hard_out; p.iters_out = a.iters_out; p.llr_out = a.llr_out;
+    p.workspace = a.workspace; p.work_counter = a.work_counter; p.arrived = a.arrived;
+    pl->fn2[st]<<<grid, pl->threads, pl->smem, stream>>>(p);
     return (int)cudaGetLastError();
 }
 

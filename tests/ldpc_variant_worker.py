@@ -1,7 +1,7 @@
 """Helpers of tests/test_gpu_ldpc_variants.py, and the subprocess that decodes under one set of LDPC overrides.
 
-The kernel-choice overrides (DVBS2FEC_LDPC_LANES2, _OCC3, _V2, _CHAINS, DVBS2FEC_CHAIN_MINLEV) are read once per
-process, so every environment of the variant matrix runs in a process of its own:
+The kernel-choice overrides (DVBS2FEC_LDPC_LANES2, DVBS2FEC_LDPC_OCC3) are read once per process, so every
+environment of the variant matrix runs in a process of its own:
 
     python tests/ldpc_variant_worker.py ORACLE.npz REPORT.json
 
@@ -54,8 +54,8 @@ CODE_LINKS = {
     (1, 0): (2, False), (1, 1): (3, True), (1, 2): (4, True), (1, 3): (5, False), (1, 4): (9, True), (1, 5): (8, True),
     (1, 6): (11, False), (1, 7): (11, False), (1, 8): (17, False), (1, 10): (25, True),
 }
-# compiled instantiations, cnt -> forms ("U" every layer has cnt links, "R" ragged): ldpc_inst_*.cu and
-# ldpc2_inst_*.cu (one thread per row) list the same set, ldpc2l_inst_*.cu (two threads per row) its own
+# compiled instantiations, cnt -> forms ("U" every layer has cnt links, "R" ragged): ldpc2_inst_*.cu (one thread per
+# row) and ldpc2l_inst_*.cu (two threads per row)
 ONE_LANE = {2: "UR", 3: "U", 4: "U", 5: "UR", 8: "U", 9: "U", 11: "R", 12: "U", 16: "U", 17: "R", 20: "U", 25: "U", 28: "U"}
 TWO_LANES = {8: "U", 9: "U", 11: "R", 12: "U", 16: "U", 17: "R", 20: "U", 25: "U", 28: "U"}
 
@@ -65,7 +65,7 @@ def has_two_lanes(code):
 
 
 def selected_shape(code, lanes2):
-    """(CNT, uniform form) that pick / pickl and is_uniform (ldpc_decoder.cu) choose for the code"""
+    """(CNT, uniform form) that pick2 / pickl and is_uniform (ldpc_decoder.cu) choose for the code"""
     max_cnt, uniform = CODE_LINKS[code]
     table = TWO_LANES if lanes2 else ONE_LANE
     cnt = max_cnt if lanes2 else min(c for c in table if c >= max_cnt)
@@ -78,15 +78,13 @@ def occupancy(cnt, occ3):
     return (3 if cnt <= 9 else 2) if occ3 else (2 if cnt <= 9 else 1)
 
 
-def instantiation(code, v2, lanes2, occ3, chains, streamed):
+def instantiation(code, lanes2, occ3, streamed):
     """the kernel a code launches, as parse_kernel spells it"""
-    lanes2 = v2 and lanes2 and has_two_lanes(code)
+    lanes2 = lanes2 and has_two_lanes(code)
     cnt, use_u = selected_shape(code, lanes2)
     if lanes2:
         return ("ldpc_v2l_kernel", cnt, not use_u, streamed)
-    if v2:
-        return ("ldpc_v2_kernel", cnt, not use_u, streamed, occupancy(cnt, occ3))
-    return ("ldpc_pair_kernel", cnt, use_u, streamed, chains, occupancy(cnt, occ3))
+    return ("ldpc_v2_kernel", cnt, not use_u, streamed, occupancy(cnt, occ3))
 
 
 def reachable_instantiations():
@@ -95,10 +93,8 @@ def reachable_instantiations():
     for code in CODE_LINKS:
         for st in (False, True):
             for occ3 in (False, True):
-                out.add(instantiation(code, True, False, occ3, False, st))
-                out.add(instantiation(code, True, True, occ3, False, st))
-                for ch in (False, True):
-                    out.add(instantiation(code, False, False, occ3, ch, st))
+                out.add(instantiation(code, False, occ3, st))
+                out.add(instantiation(code, True, occ3, st))
     return out
 
 
@@ -107,18 +103,15 @@ def compiled_instantiations():
     for st in (False, True):
         for cnt, forms in ONE_LANE.items():
             for f in forms:
-                rg = f == "R"
                 for occ3 in (False, True):
-                    out.add(("ldpc_v2_kernel", cnt, rg, st, occupancy(cnt, occ3)))
-                    for ch in (False, True):
-                        out.add(("ldpc_pair_kernel", cnt, not rg, st, ch, occupancy(cnt, occ3)))
+                    out.add(("ldpc_v2_kernel", cnt, f == "R", st, occupancy(cnt, occ3)))
         for cnt, forms in TWO_LANES.items():
             for f in forms:
                 out.add(("ldpc_v2l_kernel", cnt, f == "R", st))
     return out
 
 
-_KERNEL_RE = re.compile(r"\b(ldpc_pair_kernel|ldpc_v2l_kernel|ldpc_v2_kernel)<([^<>]*)>")
+_KERNEL_RE = re.compile(r"\b(ldpc_v2l_kernel|ldpc_v2_kernel)<([^<>]*)>")
 
 
 def parse_kernel(name):

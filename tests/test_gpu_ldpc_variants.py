@@ -1,12 +1,12 @@
 """Every LDPC kernel variant against the CPU oracle, on all 21 codes, at batch sizes where every CTA of the
 persistent grid decodes several frame pairs.  Needs a B200.
 
-ldpc_prepare picks one kernel per code from a matrix of instantiations (one or two threads per row, first or second
-generation, uniform or ragged, streamed or not, 2 or 3 CTAs per SM); three performance tables choose the cell, and
-process-wide overrides flip them.  Each environment of ENVS runs in its own subprocess (the overrides are read once
-per process): ldpc_variant_worker.py decodes a batch tiled from M oracle frames per code through four entry points
-and compares every position with the oracle.  The profiler's kernel names prove which instantiation ran, and the
-union over the matrix must contain every instantiation some code can select.
+ldpc_prepare picks one kernel per code from a matrix of instantiations (one or two threads per row, uniform or ragged,
+streamed or not, 2 or 3 CTAs per SM); two performance tables choose the cell, and process-wide overrides flip them.
+Each environment of ENVS runs in its own subprocess (the overrides are read once per process): ldpc_variant_worker.py
+decodes a batch tiled from M oracle frames per code through four entry points and compares every position with the
+oracle.  The profiler's kernel names prove which instantiation ran, and the union over the matrix must contain every
+instantiation some code can select.
 
 Also here: BCH on all 21 codes, with errors on the edges of the syndrome stage's per-lane byte chunks."""
 import json
@@ -25,18 +25,12 @@ from orclib import ALL_CODES, code_params
 
 pytestmark = pytest.mark.gpu
 
-V2, LANES2, OCC3, CHAINS, MINLEV = ("DVBS2FEC_LDPC_V2", "DVBS2FEC_LDPC_LANES2", "DVBS2FEC_LDPC_OCC3", "DVBS2FEC_LDPC_CHAINS",
-                                    "DVBS2FEC_CHAIN_MINLEV")
+LANES2, OCC3 = "DVBS2FEC_LDPC_LANES2", "DVBS2FEC_LDPC_OCC3"
 ENVS = {
     "default": {},
     "lanes2": {LANES2: "1"},
     "one-lane-occ2": {LANES2: "0", OCC3: "0"},
     "one-lane-occ3": {LANES2: "0", OCC3: "1"},
-    "gen1": {V2: "0", CHAINS: "0", OCC3: "0"},
-    "gen1-all-chains-occ3": {V2: "0", CHAINS: "1", MINLEV: "2", OCC3: "1"},   # every layer plan_chains accepts
-    # the other two (chains, occupancy) pairs of the first-generation kernel, so that every instantiation runs
-    "gen1-chains-occ2": {V2: "0", CHAINS: "1", OCC3: "0"},
-    "gen1-occ3": {V2: "0", CHAINS: "0", OCC3: "1"},
 }
 PATHS = ("ldpc_decode", "ldpc_decode_max_trials_1", "ldpc_decode_max_trials_3", "decode_batch", "decode_batch_max_batch_255",
          "decode_batch_device")
@@ -129,14 +123,11 @@ def test_variant_bit_exact(run_env, env_name):
         fam, cnt = k1[0], k1[1]
         two = W.has_two_lanes(code)
         want_cnt, want_u = W.selected_shape(code, fam == "ldpc_v2l_kernel")
-        assert cnt == want_cnt and (k1[2] == want_u if fam == "ldpc_pair_kernel" else k1[2] != want_u), (code, k1)
+        assert cnt == want_cnt and k1[2] != want_u, (code, k1)
         if env.get(LANES2) == "1":
             assert fam == ("ldpc_v2l_kernel" if two else "ldpc_v2_kernel"), (code, k1)
         if env.get(LANES2) == "0":
             assert fam != "ldpc_v2l_kernel", (code, k1)
-        if env.get(V2) == "0":
-            assert fam == "ldpc_pair_kernel", (code, k1)
-            assert k1[4] == (env[CHAINS] == "1"), (code, k1)            # CHAINS
         if OCC3 in env and fam != "ldpc_v2l_kernel":
             assert k1[-1] == W.occupancy(cnt, env[OCC3] == "1"), (code, k1)
         # the streamed launch's grid: every CTA takes at least four pairs from the work counter

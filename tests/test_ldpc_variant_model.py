@@ -58,8 +58,6 @@ def _macro_list(pattern, macro_re):
 
 
 def test_instantiation_tables_match_the_sources():
-    one = _macro_list("ldpc_inst_*.cu", r"\bV([UBR])\((\d+)\)")
-    assert one == W.ONE_LANE
     assert _macro_list("ldpc2_inst_*.cu", r"\bV2([UBR])\((\d+)\)") == W.ONE_LANE
     assert _macro_list("ldpc2l_inst_*.cu", r"\bV2L([UR])\((\d+)\)") == W.TWO_LANES
 
@@ -68,12 +66,10 @@ def test_every_compiled_instantiation_is_reachable():
     """each code selects exactly one instantiation for a setting of the overrides; none is compiled for nothing"""
     reach = W.reachable_instantiations()
     assert reach == W.compiled_instantiations()
-    assert len(reach) == 198
+    assert len(reach) == 78
 
 
 def test_kernel_names_parse():
     assert W.parse_kernel("void s2::v2::ldpc_v2_kernel<9, false, true, 3>(s2::LdpcParams2)") == ("ldpc_v2_kernel", 9, False, True, 3)
     assert W.parse_kernel("void s2::v2::ldpc_v2l_kernel<17, true, false>(s2::LdpcParams2)") == ("ldpc_v2l_kernel", 17, True, False)
-    assert W.parse_kernel("void s2::(anonymous namespace)::ldpc_pair_kernel<5, false, true, true, 2>(s2::LdpcParams)") == \
-        ("ldpc_pair_kernel", 5, False, True, True, 2)
     assert W.parse_kernel("void s2::bch_kernel(s2::BchArgs)") is None
