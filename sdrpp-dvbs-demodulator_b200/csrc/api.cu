@@ -23,6 +23,7 @@
 #include <cuda_runtime.h>
 #include <emmintrin.h>
 
+#include "abi_util.h"
 #include "bch_decoder.cuh"
 #include "demapper.cuh"
 #include "host_tables.h"
@@ -34,73 +35,25 @@
 using namespace s2;
 
 namespace {
-
 thread_local char g_err[512] = "";
-int fail(int code, const char* fmt, ...) {
+}  // namespace
+
+int s2::fail(int code, const char* fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
     vsnprintf(g_err, sizeof(g_err), fmt, ap);
     va_end(ap);
     return code;
 }
-}  // namespace
-namespace s2 {
-// for the C-ABI entry points that live in other translation units (pl_api.cu)
-int api_fail(int code, const char* msg) {
-    snprintf(g_err, sizeof(g_err), "%s", msg);
-    return code;
-}
-}  // namespace s2
+
 namespace {
-#define CU(call)                                                                              \
-    do {                                                                                      \
-        cudaError_t e_ = (call);                                                              \
-        if (e_ != cudaSuccess)                                                                \
-            return fail(DVBS2FEC_ECUDA, "%s: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
 
 constexpr int kStages = 4; // page-locked staging batches per handle (frame queue)
 constexpr int kPiece = 256; // frames per piece of a streamed input copy
 constexpr int kSlots = 2;  // double buffering per device: copy of batch k+1 overlaps kernels of batch k
 
-template <typename T>
-struct DevBuf {
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-template <typename T>
-struct PinBuf {
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMallocHost(&p, n * sizeof(T));
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
+// what a decode call gets per frame
+enum class Input { llr, sym, idx };   // LLRs, PLFRAME symbols, LUT coordinates of the payload symbols
 
 struct Slot {
     cudaStream_t stream = nullptr;
@@ -138,22 +91,20 @@ struct Slot {
     int pending = 0;
     size_t bb_bytes = 0;
     bool staged_out = true;
-    uint64_t tag_base = 0;
 };
 
-struct CodeDev {  // per (device, LDPC code)
-    DevBuf<uint8_t> row_level;
-};
 struct BchTabDev {
     DevBuf<uint16_t> crc, basis;
 };
 
-struct CodeTables {  // what the kernels of one LDPC code need; ldpc.links points into links
+struct CodeTables {  // what the kernels of one LDPC code need on one device; ldpc.links points into links
     LdpcDev ldpc{};
     BchDev bch{};
     int grid = 0;
     int hard_stride = 0;
     std::vector<uint32_t> links;
+    DevBuf<uint8_t> row_level;
+    ~CodeTables() { ldpc_release(ldpc); }
 };
 
 struct DevCtx {
@@ -164,24 +115,34 @@ struct DevCtx {
     Slot slot[2 * kSlots + 1];
     std::mutex dev_mu;
     bool dev_used = false;
-    std::map<int, CodeDev> codes;
+    // prepared codes by code index (prepare_code); entries stay where they are while others are added
+    std::map<int, CodeTables> codes;
     std::map<int, BchTabDev> bch;           // key m*100+t
     DevBuf<uint16_t> gf_log[2], gf_exp[2];  // [0]: m=14, [1]: m=16
     DevBuf<uint8_t> prbs;
     DevBuf<uint8_t> pl_rn;                  // PL scrambling sequence of the handle's Gold code (empty: off)
     std::map<int, DevBuf<uint32_t>> luts;   // key modcod constellation/gamma: modcod number
-    // current configuration
-    LdpcDev ldpc{};
-    BchDev bchd{};
+    // current configuration; the queue worker reaches the code only through cur
+    const CodeTables* cur = nullptr;
     DemapDev demap{};
-    int grid = 0;
-    // VCM calls: prepared codes by code index, demap records by (modcod, short, pilots) -- see vcm.cuh
-    std::map<int, CodeTables> vcm_codes;
+    // VCM calls: demap records by (modcod, short, pilots) -- see vcm.cuh
     DevBuf<DemapDev> vcm_demap;
     bool vcm_demap_ok[kVcmConfigs] = {};
-    ~DevCtx() {
-        ldpc_release(ldpc);
-        for (auto& kv : vcm_codes) ldpc_release(kv.second.ldpc);
+    ~DevCtx() {   // the buffers free themselves after this, with the device current
+        cudaSetDevice(device);
+        for (int k = 0; k < 2 * kSlots + 1; ++k) {
+            Slot& s = slot[k];
+            if (s.copy && !(k >= 1 && k < kSlots)) {   // (slots 1..kSlots-1 borrow slot 0's)
+                cudaStreamSynchronize(s.copy);
+                cudaStreamDestroy(s.copy);
+            }
+            if (s.stream) {
+                cudaStreamSynchronize(s.stream);
+                cudaStreamDestroy(s.stream);
+            }
+            if (s.done) cudaEventDestroy(s.done);
+            if (s.armed) cudaEventDestroy(s.armed);
+        }
     }
 };
 
@@ -205,6 +166,13 @@ struct dvbs2fec_ts_parser {
     DevBuf<GseDesc> g_desc;
     DevBuf<GseOut> g_out;
     DevBuf<uint32_t> g_crc0, g_xpow;
+    ~dvbs2fec_ts_parser() {
+        cudaSetDevice(device);
+        if (stream) {
+            cudaStreamSynchronize(stream);
+            cudaStreamDestroy(stream);
+        }
+    }
 };
 
 struct dvbs2fec_handle {
@@ -213,7 +181,6 @@ struct dvbs2fec_handle {
     ModcodCfg mc{};
     const LdpcCode* code = nullptr;
     int max_trials = 25;
-    int hard_stride = 0;
     int plsyms = 0;
     int last_launches = 0;
     int pl_codenum = -1;                // Gold code of the PL descrambler in K1, -1 = inputs are descrambled
@@ -226,8 +193,6 @@ struct dvbs2fec_handle {
     struct Span { int kind; cudaEvent_t a, b; };
     std::vector<Span> spans;
     std::mutex span_mu;
-    // host copies of the layer tables referenced by LdpcDev (host pointers)
-    std::vector<uint32_t> h_links;
     // ---- queue
     std::mutex mu;
     std::mutex submit_mu;               // serialises producers (the reference has one per instance)
@@ -247,7 +212,7 @@ struct dvbs2fec_handle {
         bool has_ts = false;
         std::vector<uint64_t> tags;
         int n = 0, taken = 0, cap = 0;
-        int kind = 0;                      // 0 LLRs, 1 PLFRAME symbols, 2 LUT coordinates
+        Input kind = Input::llr;
         int rc = 0;
         size_t kb = 0, in_bytes = 0;
         std::atomic<int> outstanding{0};   // device shares still running
@@ -259,20 +224,37 @@ struct dvbs2fec_handle {
     std::deque<int> st_free, st_ready, st_inflight, st_done;
     int st_fill = -1;
     uint64_t launch_seq = 0;
+    ~dvbs2fec_handle() {
+        {
+            std::unique_lock<std::mutex> lk(mu);
+            stop = true;
+            cv_work.notify_all();
+        }
+        if (worker.joinable()) worker.join();
+        for (auto& d : devs) {   // work enqueued on caller-owned streams by the device entry point, before anything goes
+            cudaSetDevice(d->device);
+            cudaDeviceSynchronize();
+        }
+        dvbs2fec_ts_destroy(ts);
+        if (ts_done) cudaEventDestroy(ts_done);
+        for (auto& sp : spans) {
+            cudaEventDestroy(sp.a);
+            cudaEventDestroy(sp.b);
+        }
+    }
 };
 
 static int ts_args(dvbs2fec_ts_parser* p, const uint8_t* d_bb, int cnt, uint8_t* d_out, int out_cap, int* d_produced, TsArgs* out);
 
 namespace {
 
-// LDPC code c on device d into L (ldpc_prepare) and its grid; links = host link words of c, kept alive by the caller
-int prepare_ldpc(DevCtx& d, const LdpcCode& c, const uint32_t* links, LdpcDev& L, int& grid) {
-    CodeDev& cd = d.codes[c.index];
-    if (!cd.row_level.p) {
-        CU(cd.row_level.reserve(c.row_level.size()));
-        CU(cudaMemcpy(cd.row_level.p, c.row_level.data(), c.row_level.size(), cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
-    }
+// LDPC plan, grid, hard stride and link words of code c on device d into T
+int prepare_ldpc(DevCtx& d, const LdpcCode& c, CodeTables& T) {
+    CU(T.row_level.reserve(c.row_level.size()));
+    CU(upload(T.row_level.p, c.row_level.data(), c.row_level.size()));
+    for (const LayerLink& l : c.links) T.links.push_back(((uint32_t)l.group << 16) | l.shift);
+    T.hard_stride = ((c.K / 8) + 15) & ~15;
+    LdpcDev& L = T.ldpc;
     L.N = c.N; L.K = c.K; L.R = c.R; L.q = c.q;
     L.ngroups = c.K / kGroup;
     L.max_cnt = c.max_cnt;
@@ -280,15 +262,15 @@ int prepare_ldpc(DevCtx& d, const LdpcCode& c, const uint32_t* links, LdpcDev& L
     L.sg = ldpc_slot_groups_for(c.max_cnt, L.lanes2);
     L.occ3 = ldpc_ctas_wanted3(c.index);
     if (!L.sg) return fail(DVBS2FEC_EINVAL, "no LDPC kernel for %d links per row", c.max_cnt);
-    L.links = links;
+    L.links = T.links.data();
     L.layer_off = c.layer_off.data();
     L.layer_nlev = c.layer_nlev.data();
-    L.row_level = cd.row_level.p;
+    L.row_level = T.row_level.p;
     if (int e = ldpc_prepare(L)) return fail(DVBS2FEC_ECUDA, "LDPC kernel set-up: %s", cudaGetErrorString((cudaError_t)e));
     int per_sm = ldpc_max_ctas_per_sm(L);
     if (per_sm <= 0) return fail(DVBS2FEC_ENODEV, "LDPC kernel does not fit on device %d (%s)", d.device,
                                  cudaGetErrorString(cudaGetLastError()));
-    grid = d.sms * per_sm;
+    T.grid = d.sms * per_sm;
     return 0;
 }
 
@@ -299,31 +281,44 @@ int prepare_bch(DevCtx& d, const LdpcCode& c, BchDev& B) {
     if (!d.gf_log[fi].p) {
         CU(d.gf_log[fi].reserve(gf.log.size()));
         CU(d.gf_exp[fi].reserve(gf.exp.size()));
-        CU(cudaMemcpy(d.gf_log[fi].p, gf.log.data(), gf.log.size() * 2, cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
-        CU(cudaMemcpy(d.gf_exp[fi].p, gf.exp.data(), gf.exp.size() * 2, cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+        CU(upload(d.gf_log[fi].p, gf.log.data(), gf.log.size() * 2));
+        CU(upload(d.gf_exp[fi].p, gf.exp.data(), gf.exp.size() * 2));
     }
     BchTabDev& bt = d.bch[m * 100 + t];
     if (!bt.crc.p) {
         const BchHost& bh = bch_host(m, t);
         CU(bt.crc.reserve(bh.crc.size()));
         CU(bt.basis.reserve(bh.basis.size()));
-        CU(cudaMemcpy(bt.crc.p, bh.crc.data(), bh.crc.size() * 2, cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
-        CU(cudaMemcpy(bt.basis.p, bh.basis.data(), bh.basis.size() * 2, cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+        CU(upload(bt.crc.p, bh.crc.data(), bh.crc.size() * 2));
+        CU(upload(bt.basis.p, bh.basis.data(), bh.basis.size() * 2));
     }
     if (!d.prbs.p) {
         const auto& seq = bb_prbs();
         CU(d.prbs.reserve(seq.size()));
-        CU(cudaMemcpy(d.prbs.p, seq.data(), seq.size(), cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+        CU(upload(d.prbs.p, seq.data(), seq.size()));
     }
     B.gf.m = m; B.gf.N = gf.N; B.gf.log = d.gf_log[fi].p; B.gf.exp = d.gf_exp[fi].p;
     B.t = t; B.nbch = c.K; B.kbch = c.kbch;
     B.prefix = gf.N - c.K;
     B.crc = bt.crc.p; B.basis = bt.basis.p; B.prbs = d.prbs.p;
+    return 0;
+}
+
+// Code ci on device d, prepared on first use (LDPC plan and grid, BCH record, hard stride, link words) -- the one
+// store of prepared codes for the single-MODCOD configuration and VCM calls alike
+int prepare_code(DevCtx& d, int ci, const CodeTables** out) {
+    auto it = d.codes.find(ci);
+    if (it == d.codes.end()) {
+        it = d.codes.try_emplace(ci).first;
+        const LdpcCode& c = ldpc_code(ci);
+        int rc = prepare_ldpc(d, c, it->second);
+        if (!rc) rc = prepare_bch(d, c, it->second.bch);
+        if (rc) {
+            d.codes.erase(it);
+            return rc;
+        }
+    }
+    *out = &it->second;
     return 0;
 }
 
@@ -350,8 +345,7 @@ int prepare_demap(DevCtx& d, const ModcodCfg& mc, const LdpcCode& c, int plsyms,
         if (!lut.p) {
             std::vector<uint32_t> tab = demap_lut(ch);
             CU(lut.reserve(tab.size()));
-            CU(cudaMemcpy(lut.p, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice));
-            CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+            CU(upload(lut.p, tab.data(), tab.size() * 4));
         }
         D.lut = lut.p;
     }
@@ -360,29 +354,31 @@ int prepare_demap(DevCtx& d, const ModcodCfg& mc, const LdpcCode& c, int plsyms,
 
 int setup_device_tables(dvbs2fec_handle* h, DevCtx& d) {
     CU(cudaSetDevice(d.device));
-    const LdpcCode& c = *h->code;
-    if (int rc = prepare_ldpc(d, c, h->h_links.data(), d.ldpc, d.grid)) return rc;
-    if (int rc = prepare_bch(d, c, d.bchd)) return rc;
-    return prepare_demap(d, h->mc, c, h->plsyms, h->pl_codenum >= 0 ? d.pl_rn.p : nullptr, d.demap);
+    if (int rc = prepare_code(d, h->code->index, &d.cur)) return rc;
+    return prepare_demap(d, h->mc, *h->code, h->plsyms, h->pl_codenum >= 0 ? d.pl_rn.p : nullptr, d.demap);
 }
 
-// kind of input: 0 = LLRs, 1 = PLFRAME symbols, 2 = LUT coordinates of the payload symbols
-size_t input_frame_bytes(const dvbs2fec_handle* h, int kind) {
-    return kind == 1 ? (size_t)h->plsyms * 8 : kind == 2 ? (size_t)(h->code->N / h->mc.bits) * 2 : (size_t)h->code->N;
+size_t input_frame_bytes(const dvbs2fec_handle* h, Input kind) {
+    return kind == Input::sym ? (size_t)h->plsyms * 8 : kind == Input::idx ? (size_t)(h->code->N / h->mc.bits) * 2 : (size_t)h->code->N;
 }
 
-int reserve_slot(dvbs2fec_handle* h, DevCtx& d, Slot& s, int nframes, int kind, bool host_staging) {
+// where a batch of input of this kind goes in slot s
+void* slot_input(Slot& s, Input kind) {
+    return kind == Input::sym ? (void*)s.sym.p : kind == Input::idx ? (void*)s.idx.p : (void*)s.llr.p;
+}
+
+int reserve_slot(dvbs2fec_handle* h, DevCtx& d, Slot& s, int nframes, Input kind, bool host_staging) {
     const LdpcCode& c = *h->code;
     CU(cudaSetDevice(d.device));
     CU(s.llr.reserve((size_t)nframes * c.N));
-    if (kind == 1) CU(s.sym.reserve((size_t)nframes * h->plsyms * 2));
-    if (kind == 2) CU(s.idx.reserve((size_t)nframes * input_frame_bytes(h, 2)));
-    CU(s.hard.reserve((size_t)nframes * h->hard_stride));
+    if (kind == Input::sym) CU(s.sym.reserve((size_t)nframes * h->plsyms * 2));
+    if (kind == Input::idx) CU(s.idx.reserve((size_t)nframes * input_frame_bytes(h, Input::idx)));
+    CU(s.hard.reserve((size_t)nframes * d.cur->hard_stride));
     CU(s.iters.reserve(nframes));
     CU(s.corr.reserve(nframes));
     CU(s.bb.reserve((size_t)nframes * (c.kbch / 8)));
     CU(s.res.reserve(nframes));
-    CU(s.workspace.reserve((size_t)d.grid * ldpc_workspace_bytes(d.ldpc)));
+    CU(s.workspace.reserve((size_t)d.cur->grid * ldpc_workspace_bytes(d.cur->ldpc)));
     CU(s.counter.reserve(1));
     if (host_staging) {
         size_t in_bytes = (size_t)nframes * input_frame_bytes(h, kind);
@@ -414,57 +410,78 @@ struct SpanMark {
     }
 };
 
-// enqueue demap (optional) + LDPC + BCH/descramble for n frames already on the device
-int enqueue_chain(dvbs2fec_handle* h, DevCtx& d, Slot& s, const float* d_sym, const int8_t* d_llr, int n,
-                  uint8_t* d_bb, dvbs2fec_result* d_res, cudaStream_t st, int* launches, uint64_t tag_base = 0,
-                  const unsigned int* arrived = nullptr, const uint8_t* d_idx = nullptr) {
-    const int8_t* llr = d_llr;
-    SpanMark mark{h, st};
-    if (d_sym || d_idx) {
-        mark(0, true);
-        int e = d_sym ? demap_launch(d.demap, d_sym, n, s.llr.p, st) : demap_idx_launch(d.demap, d_idx, n, s.llr.p, st);
-        mark(0, false);
-        if (e) return fail(DVBS2FEC_ECUDA, "demap launch: %s", cudaGetErrorString((cudaError_t)e));
-        llr = s.llr.p;
-        ++*launches;
-    }
-    CU(cudaMemsetAsync(s.counter.p, 0, sizeof(unsigned int), st));
+// The argument blocks of LDPC and BCH for n frames of code T in slot s: the fields that depend on the code and the slot.
+// The frames' hard decisions start at byte hard_off of s.hard, their iteration counts at entry `at` of s.iters, and
+// LDPC hands them out through work counter k (a VCM chunk places the frames of each code so).
+LdpcArgs ldpc_args(const dvbs2fec_handle* h, const CodeTables& T, const Slot& s, const int8_t* llr, int n,
+                   size_t hard_off = 0, int at = 0, int k = 0) {
     LdpcArgs la{};
-    la.code = d.ldpc;
+    la.code = T.ldpc;
     la.llr_in = llr;
     la.nframes = n;
     la.max_trials = h->max_trials;
-    la.hard_out = s.hard.p;
-    la.hard_stride = h->hard_stride;
-    la.iters_out = s.iters.p;
-    la.llr_out = nullptr;
+    la.hard_out = s.hard.p + hard_off;
+    la.hard_stride = T.hard_stride;
+    la.iters_out = s.iters.p + at;
     la.workspace = s.workspace.p;
-    la.work_counter = s.counter.p;
+    la.work_counter = s.counter.p + k;
+    return la;
+}
+BchArgs bch_args(const CodeTables& T, const Slot& s, int n, size_t hard_off = 0, int at = 0) {
+    BchArgs ba{};
+    ba.code = T.bch;
+    ba.hard = s.hard.p + hard_off;
+    ba.hard_stride = T.hard_stride;
+    ba.nframes = n;
+    ba.ldpc_iters = s.iters.p + at;
+    ba.descramble = 1;
+    return ba;
+}
+int ldpc_grid(const CodeTables& T, int n) { return std::min(T.grid, (n + 1) / 2); }
+
+// LDPC then BCH/descramble on st for n frames of code T, placed in slot s as ldpc_args says: BBFRAMEs to bb, records
+// (tags tag_base + i) to res
+int enqueue_ldpc_bch(dvbs2fec_handle* h, const CodeTables& T, Slot& s, cudaStream_t st, int* launches, const int8_t* llr,
+                     int n, const unsigned int* arrived, uint8_t* bb, dvbs2fec_result* res, unsigned long long tag_base,
+                     size_t hard_off = 0, int at = 0, int k = 0) {
+    SpanMark mark{h, st};
+    CU(cudaMemsetAsync(s.counter.p + k, 0, sizeof(unsigned int), st));
+    LdpcArgs la = ldpc_args(h, T, s, llr, n, hard_off, at, k);
     la.arrived = arrived;
-    int grid = std::min(d.grid, (n + 1) / 2);
     mark(1, true);
-    int e = ldpc_launch(la, grid, st);
+    int e = ldpc_launch(la, ldpc_grid(T, n), st);
     mark(1, false);
     if (e) return fail(DVBS2FEC_ECUDA, "ldpc launch: %s", cudaGetErrorString((cudaError_t)e));
     ++*launches;
-    BchArgs ba{};
-    ba.code = d.bchd;
-    ba.hard = s.hard.p;
-    ba.hard_stride = h->hard_stride;
-    ba.nframes = n;
-    ba.ldpc_iters = s.iters.p;
-    ba.tags = nullptr;
+    BchArgs ba = bch_args(T, s, n, hard_off, at);
     ba.tag_base = tag_base;
-    ba.bb_out = d_bb;
-    ba.results = d_res;
-    ba.corr_out = nullptr;
-    ba.descramble = 1;
+    ba.bb_out = bb;
+    ba.results = res;
     mark(2, true);
     e = bch_launch(ba, st);
     mark(2, false);
     if (e) return fail(DVBS2FEC_ECUDA, "bch launch: %s", cudaGetErrorString((cudaError_t)e));
     ++*launches;
     return 0;
+}
+
+// enqueue demap (symbol and coordinate input) + LDPC + BCH/descramble for n frames of the current code already on
+// the device
+int enqueue_chain(dvbs2fec_handle* h, DevCtx& d, Slot& s, Input kind, const void* in, int n, uint8_t* d_bb,
+                  dvbs2fec_result* d_res, cudaStream_t st, int* launches, uint64_t tag_base,
+                  const unsigned int* arrived = nullptr) {
+    const int8_t* llr = static_cast<const int8_t*>(in);
+    if (kind != Input::llr) {
+        SpanMark mark{h, st};
+        mark(0, true);
+        int e = kind == Input::sym ? demap_launch(d.demap, static_cast<const float*>(in), n, s.llr.p, st)
+                                   : demap_idx_launch(d.demap, static_cast<const uint8_t*>(in), n, s.llr.p, st);
+        mark(0, false);
+        if (e) return fail(DVBS2FEC_ECUDA, "demap launch: %s", cudaGetErrorString((cudaError_t)e));
+        llr = s.llr.p;
+        ++*launches;
+    }
+    return enqueue_ldpc_bch(h, *d.cur, s, st, launches, llr, n, arrived, d_bb, d_res, tag_base);
 }
 
 // Streamed LLR input.  arm: zero the arrival word on the copy stream and make the compute stream wait for that,
@@ -516,6 +533,24 @@ int finish_slot(dvbs2fec_handle* h, Slot& s) {
     return 0;
 }
 
+// The end of a chunk of a synchronous call: its outputs (bb_bytes of BBFRAMEs, m records) go to the caller, straight
+// into page-locked caller memory or else through the slot's staging (finish_slot copies them out), and the slot is
+// pending until `done`.
+int chunk_out(Slot& s, uint8_t* user_bb, const uint8_t* d_bb, size_t bb_bytes, dvbs2fec_result* user_res,
+              const dvbs2fec_result* d_res, int m, bool pin_out) {
+    s.user_bb = user_bb;
+    s.user_res = user_res;
+    s.staged_out = !pin_out;
+    if (user_bb && bb_bytes) CU(cudaMemcpyAsync(pin_out ? user_bb : s.h_bb.p, d_bb, bb_bytes, cudaMemcpyDeviceToHost, s.stream));
+    if (user_res)
+        CU(cudaMemcpyAsync(pin_out ? (void*)user_res : (void*)s.h_res.p, d_res, (size_t)m * sizeof(dvbs2fec_result),
+                           cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaEventRecord(s.done, s.stream));
+    s.pending = m;
+    s.bb_bytes = bb_bytes;
+    return 0;
+}
+
 // Error exit of the synchronous entry points: nothing asynchronous may outlive the call -- copies into the caller's
 // buffers that were already enqueued are waited for, and no slot keeps a pointer to them (a later call would copy into
 // freed memory).
@@ -540,15 +575,14 @@ struct HostSlotsAbort {
 };
 
 // frames [0, n) of one device's share, host buffers in and out
-int run_device_share(dvbs2fec_handle* h, DevCtx& d, const int8_t* llr, const float* sym, const uint8_t* idx, int n, uint8_t* bb,
+int run_device_share(dvbs2fec_handle* h, DevCtx& d, Input kind, const void* input, int n, uint8_t* bb,
                      dvbs2fec_result* res, uint64_t tag0, int* launches) {
     if (n <= 0) return 0;
     CU(cudaSetDevice(d.device));
     const LdpcCode& c = *h->code;
     const size_t kb = c.kbch / 8;
-    const int kind = sym ? 1 : idx ? 2 : 0;
     const size_t in_frame_bytes = input_frame_bytes(h, kind);
-    const uint8_t* in = sym ? reinterpret_cast<const uint8_t*>(sym) : idx ? idx : reinterpret_cast<const uint8_t*>(llr);
+    const uint8_t* in = static_cast<const uint8_t*>(input);
     const int chunk = std::min(h->cfg.max_batch, n);
     for (int k = 0; k < kSlots; ++k) {
         int rc = reserve_slot(h, d, d.slot[k], chunk, kind, true);
@@ -564,33 +598,22 @@ int run_device_share(dvbs2fec_handle* h, DevCtx& d, const int8_t* llr, const flo
         const int m = std::min(chunk, n - f0);
         if ((rc = finish_slot(h, s))) return rc;
         const uint8_t* src = in + (size_t)f0 * in_frame_bytes;
-        if (kind == 0) {   // LLR input: the kernel starts on the first piece
+        void* dst = slot_input(s, kind);
+        if (kind == Input::llr) {   // the kernel starts on the first piece
             if ((rc = arm_streamed_input(s, m))) return rc;
             if ((rc = feed_streamed_input(s, src, m, in_frame_bytes, pin_in))) return rc;
-            rc = enqueue_chain(h, d, s, nullptr, s.llr.p, m, s.bb.p, s.res.p, s.stream, launches, tag0 + f0, s.arrived.p);
-            if (rc) return rc;
+            rc = enqueue_chain(h, d, s, kind, dst, m, s.bb.p, s.res.p, s.stream, launches, tag0 + f0, s.arrived.p);
         } else {
             if (!pin_in) {
                 memcpy(s.h_in.p, src, (size_t)m * in_frame_bytes);
                 src = s.h_in.p;
             }
-            void* dst = kind == 1 ? (void*)s.sym.p : (void*)s.idx.p;
             CU(cudaMemcpyAsync(dst, src, (size_t)m * in_frame_bytes, cudaMemcpyHostToDevice, s.stream));
-            rc = enqueue_chain(h, d, s, kind == 1 ? s.sym.p : nullptr, nullptr, m, s.bb.p, s.res.p, s.stream, launches, tag0 + f0, nullptr,
-                               kind == 2 ? s.idx.p : nullptr);
-            if (rc) return rc;
+            rc = enqueue_chain(h, d, s, kind, dst, m, s.bb.p, s.res.p, s.stream, launches, tag0 + f0);
         }
-        s.user_bb = bb ? bb + (size_t)f0 * kb : nullptr;
-        s.user_res = res ? res + f0 : nullptr;
-        s.staged_out = !pin_out;
-        if (bb) CU(cudaMemcpyAsync(pin_out ? s.user_bb : s.h_bb.p, s.bb.p, (size_t)m * kb, cudaMemcpyDeviceToHost, s.stream));
-        if (res)
-            CU(cudaMemcpyAsync(pin_out ? (void*)s.user_res : (void*)s.h_res.p, s.res.p, (size_t)m * sizeof(dvbs2fec_result),
-                               cudaMemcpyDeviceToHost, s.stream));
-        CU(cudaEventRecord(s.done, s.stream));
-        s.tag_base = tag0 + f0;
-        s.pending = m;
-        s.bb_bytes = (size_t)m * kb;
+        if (rc) return rc;
+        rc = chunk_out(s, bb ? bb + (size_t)f0 * kb : nullptr, s.bb.p, (size_t)m * kb, res ? res + f0 : nullptr, s.res.p, m, pin_out);
+        if (rc) return rc;
     }
     for (int k = 0; k < kSlots; ++k)
         if ((rc = finish_slot(h, d.slot[k]))) return rc;
@@ -598,19 +621,18 @@ int run_device_share(dvbs2fec_handle* h, DevCtx& d, const int8_t* llr, const flo
     return 0;
 }
 
-int decode_host(dvbs2fec_handle* h, const int8_t* llr, const float* sym, int n, uint8_t* bb, dvbs2fec_result* res,
-                const uint8_t* idx = nullptr) {
+int decode_host(dvbs2fec_handle* h, Input kind, const void* in, int n, uint8_t* bb, dvbs2fec_result* res) {
     if (!h || !h->configured) return fail(DVBS2FEC_EINVAL, "set_modcod has not been called");
-    if (n < 0 || (!llr && !sym && !idx)) return fail(DVBS2FEC_EINVAL, "bad arguments");
-    if (idx && h->mc.constellation == APSK32) return fail(DVBS2FEC_EINVAL, "32APSK has no LUT in the reference: send symbols");
+    if (n < 0 || !in) return fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (kind == Input::idx && h->mc.constellation == APSK32) return fail(DVBS2FEC_EINVAL, "32APSK has no LUT in the reference: send symbols");
     if (h->devs.empty()) return fail(DVBS2FEC_ENODEV, "no CUDA device");
     const int nd = (int)h->devs.size();
     const size_t kb = h->code->kbch / 8;
-    const size_t in_stride = sym ? (size_t)h->plsyms * 2 : idx ? input_frame_bytes(h, 2) : (size_t)h->code->N;
+    const size_t in_stride = input_frame_bytes(h, kind);
     h->last_launches = 0;
     if (nd == 1) {
         int launches = 0;
-        int rc = run_device_share(h, *h->devs[0], llr, sym, idx, n, bb, res, 0, &launches);
+        int rc = run_device_share(h, *h->devs[0], kind, in, n, bb, res, 0, &launches);
         h->last_launches = launches;
         return rc;
     }
@@ -622,8 +644,7 @@ int decode_host(dvbs2fec_handle* h, const int8_t* llr, const float* sym, int n, 
     for (int k = 0; k < nd; ++k) {
         int f0 = std::min(n, k * per), f1 = std::min(n, f0 + per);
         th.emplace_back([=, &rcs, &ln, &errs] {
-            rcs[k] = run_device_share(h, *h->devs[k], llr ? llr + (size_t)f0 * in_stride : nullptr,
-                                      sym ? sym + (size_t)f0 * in_stride : nullptr, idx ? idx + (size_t)f0 * in_stride : nullptr, f1 - f0,
+            rcs[k] = run_device_share(h, *h->devs[k], kind, static_cast<const uint8_t*>(in) + (size_t)f0 * in_stride, f1 - f0,
                                       bb ? bb + (size_t)f0 * kb : nullptr, res ? res + f0 : nullptr, (uint64_t)f0, &ln[k]);
             if (rcs[k]) errs[k] = g_err;
         });
@@ -667,10 +688,9 @@ void launch_stage(dvbs2fec_handle* h, int st, int which) {
             // beside them) the copy of one batch already overlaps the kernels of another, and a kernel that
             // starts early and waits for streamed input would only hold SMs that a neighbour could use
             // (measured: 8 handles at max_batch 4096, 588 k frames/s plain vs 405 k streamed)
-            void* dst = S.kind == 1 ? (void*)s.sym.p : S.kind == 2 ? (void*)s.idx.p : (void*)s.llr.p;
+            void* dst = slot_input(s, S.kind);
             CU(cudaMemcpyAsync(dst, S.in.p + (size_t)f0 * S.in_bytes, (size_t)m * S.in_bytes, cudaMemcpyHostToDevice, s.stream));
-            rc = enqueue_chain(h, d, s, S.kind == 1 ? s.sym.p : nullptr, S.kind == 0 ? s.llr.p : nullptr, m, s.bb.p, s.res.p, s.stream,
-                               &h->last_launches, (uint64_t)f0, nullptr, S.kind == 2 ? s.idx.p : nullptr);
+            rc = enqueue_chain(h, d, s, S.kind, dst, m, s.bb.p, s.res.p, s.stream, &h->last_launches, (uint64_t)f0);
             if (rc) return rc;
             CU(cudaMemcpyAsync(S.bb.p + (size_t)f0 * S.kb, s.bb.p, (size_t)m * S.kb, cudaMemcpyDeviceToHost, s.stream));
             CU(cudaMemcpyAsync(S.res.p + f0, s.res.p, (size_t)m * sizeof(dvbs2fec_result), cudaMemcpyDeviceToHost, s.stream));
@@ -809,9 +829,7 @@ int vcm_parse(int n, const int32_t* desc, VcmPlan& P) {
                 return fail(DVBS2FEC_EINVAL, "frame %d: MODCOD %d with %s frames has no LDPC code", i, modcod,
                             sh ? "short" : "normal");
             const LdpcCode& c = ldpc_code(mc.code);
-            const int nsym = c.N / mc.bits;
-            f = VcmDesc{modcod * 4 + sh * 2 + pi, mc.code, 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0), nsym, c.N,
-                        c.kbch / 8};
+            f = VcmDesc{modcod * 4 + sh * 2 + pi, mc.code, plframe_symbols(mc), c.N / mc.bits, c.N, c.kbch / 8};
         }
         P.sym_off[i + 1] = P.sym_off[i] + f.plsyms;
         P.llr_off[i + 1] = P.llr_off[i] + f.N;
@@ -830,21 +848,9 @@ int vcm_plan(dvbs2fec_handle* h, DevCtx& d, VcmPlan& P, bool sym, int chunk) {
         if (f.code >= 0) code_seen[f.code] = cfg_seen[f.cfg] = true;
     for (int ci = 0; ci < kNumCodes; ++ci) {
         if (!code_seen[ci]) continue;
-        if (!d.vcm_codes.count(ci)) {
-            const LdpcCode& c = ldpc_code(ci);
-            CodeTables& T = d.vcm_codes[ci];
-            for (const LayerLink& l : c.links) T.links.push_back(((uint32_t)l.group << 16) | l.shift);
-            T.hard_stride = ((c.K / 8) + 15) & ~15;
-            int rc = prepare_ldpc(d, c, T.links.data(), T.ldpc, T.grid);
-            if (!rc) rc = prepare_bch(d, c, T.bch);
-            if (rc) {
-                ldpc_release(T.ldpc);
-                d.vcm_codes.erase(ci);
-                return rc;
-            }
-        }
-        const CodeTables& T = d.vcm_codes[ci];
-        P.workspace = std::max(P.workspace, (size_t)T.grid * ldpc_workspace_bytes(T.ldpc));
+        const CodeTables* T = nullptr;
+        if (int rc = prepare_code(d, ci, &T)) return rc;
+        P.workspace = std::max(P.workspace, (size_t)T->grid * ldpc_workspace_bytes(T->ldpc));
     }
     if (sym) {
         CU(d.vcm_demap.reserve(kVcmConfigs));
@@ -852,12 +858,9 @@ int vcm_plan(dvbs2fec_handle* h, DevCtx& d, VcmPlan& P, bool sym, int chunk) {
             if (!cfg_seen[cfg] || d.vcm_demap_ok[cfg]) continue;
             ModcodCfg mc;
             modcod_config(cfg / 4, (cfg & 2) != 0, (cfg & 1) != 0, &mc);
-            const LdpcCode& c = ldpc_code(mc.code);
-            const int nsym = c.N / mc.bits;
             DemapDev D{};
-            if (int rc = prepare_demap(d, mc, c, 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0), nullptr, D)) return rc;
-            CU(cudaMemcpy(d.vcm_demap.p + cfg, &D, sizeof D, cudaMemcpyHostToDevice));
-            CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+            if (int rc = prepare_demap(d, mc, ldpc_code(mc.code), plframe_symbols(mc), nullptr, D)) return rc;
+            CU(upload(d.vcm_demap.p + cfg, &D, sizeof D));
             d.vcm_demap_ok[cfg] = true;
         }
     }
@@ -892,7 +895,7 @@ int vcm_plan(dvbs2fec_handle* h, DevCtx& d, VcmPlan& P, bool sym, int chunk) {
             G.hard_off = ho;
             G.bb_off = bo;
             lo += align256((size_t)G.cnt * lc.N);
-            ho += (size_t)G.cnt * d.vcm_codes[G.code].hard_stride;
+            ho += (size_t)G.cnt * d.codes.at(G.code).hard_stride;
             bo += align256((size_t)G.cnt * (lc.kbch / 8));
             p += G.cnt;
         }
@@ -977,46 +980,15 @@ int vcm_chunk(dvbs2fec_handle* h, DevCtx& d, Slot& s, const VcmPlan& P, const Vc
             llr = static_cast<const int8_t*>(in) + (P.llr_off[c.f0] - in_shift);
         }
         if (e) return fail(DVBS2FEC_ECUDA, "VCM demap / gather launch: %s", cudaGetErrorString((cudaError_t)e));
-        CU(cudaMemsetAsync(s.counter.p, 0, c.groups.size() * sizeof(unsigned int), st));
     }
     for (size_t g = 0; g < c.groups.size(); ++g) {
         const VcmGroup& G = c.groups[g];
-        const CodeTables& T = d.vcm_codes.at(G.code);
-        LdpcArgs la{};
-        la.code = T.ldpc;
-        la.llr_in = llr + G.llr_off;
-        la.nframes = G.cnt;
-        la.max_trials = h->max_trials;
-        la.hard_out = s.hard.p + G.hard_off;
-        la.hard_stride = T.hard_stride;
-        la.iters_out = s.iters.p + G.p0;
-        la.workspace = s.workspace.p;
-        la.work_counter = s.counter.p + g;
-        mark(1, true);
-        int e = ldpc_launch(la, std::min(T.grid, (G.cnt + 1) / 2), st);
-        mark(1, false);
-        if (e) return fail(DVBS2FEC_ECUDA, "ldpc launch: %s", cudaGetErrorString((cudaError_t)e));
-        ++*launches;
-        BchArgs ba{};
-        ba.code = T.bch;
-        ba.hard = s.hard.p + G.hard_off;
-        ba.hard_stride = T.hard_stride;
-        ba.nframes = G.cnt;
-        ba.ldpc_iters = s.iters.p + G.p0;
-        ba.descramble = 1;
-        if (c.fast) {   // input order: straight into the caller's buffers
-            ba.tag_base = (unsigned long long)c.f0;
-            ba.bb_out = bb_out ? bb_out + (P.bb_off[c.f0] - bb_shift) : nullptr;
-            ba.results = res_out;
-        } else {
-            ba.bb_out = s.bb.p + G.bb_off;
-            ba.results = s.res.p + G.p0;
-        }
-        mark(2, true);
-        e = bch_launch(ba, st);
-        mark(2, false);
-        if (e) return fail(DVBS2FEC_ECUDA, "bch launch: %s", cudaGetErrorString((cudaError_t)e));
-        ++*launches;
+        // a fast chunk is in input order: straight into the caller's buffers
+        uint8_t* bb = c.fast ? (bb_out ? bb_out + (P.bb_off[c.f0] - bb_shift) : nullptr) : s.bb.p + G.bb_off;
+        dvbs2fec_result* res = c.fast ? res_out : s.res.p + G.p0;
+        int rc = enqueue_ldpc_bch(h, d.codes.at(G.code), s, st, launches, llr + G.llr_off, G.cnt, nullptr, bb, res,
+                                  c.fast ? (unsigned long long)c.f0 : 0, G.hard_off, G.p0, (int)g);
+        if (rc) return rc;
     }
     if (!c.fast) {
         mark(2, true);
@@ -1066,18 +1038,9 @@ int vcm_host(dvbs2fec_handle* h, int n, const int32_t* desc, const void* in, boo
         rc = vcm_chunk(h, d, s, P, c, sym, s.vin.p, in_off[c.f0], s.vmeta.p, bb ? s.vbb.p : nullptr, P.bb_off[c.f0],
                        res ? s.vres.p : nullptr, s.stream, &launches);
         if (rc) return rc;
-        const size_t out_bytes = (size_t)(P.bb_off[c.f1] - P.bb_off[c.f0]);
-        s.user_bb = bb ? bb + P.bb_off[c.f0] : nullptr;
-        s.user_res = res ? res + c.f0 : nullptr;
-        s.staged_out = !pin_out;
-        if (bb && out_bytes) CU(cudaMemcpyAsync(pin_out ? s.user_bb : s.h_bb.p, s.vbb.p, out_bytes, cudaMemcpyDeviceToHost, s.stream));
-        if (res)
-            CU(cudaMemcpyAsync(pin_out ? (void*)s.user_res : (void*)s.h_res.p, s.vres.p, (size_t)m * sizeof(dvbs2fec_result),
-                               cudaMemcpyDeviceToHost, s.stream));
-        CU(cudaEventRecord(s.done, s.stream));
-        s.tag_base = (uint64_t)c.f0;
-        s.pending = m;
-        s.bb_bytes = out_bytes;
+        rc = chunk_out(s, bb ? bb + P.bb_off[c.f0] : nullptr, s.vbb.p, (size_t)(P.bb_off[c.f1] - P.bb_off[c.f0]),
+                       res ? res + c.f0 : nullptr, s.vres.p, m, pin_out);
+        if (rc) return rc;
     }
     for (int k = 0; k < kSlots; ++k)
         if ((rc = finish_slot(h, d.slot[k]))) return rc;
@@ -1086,7 +1049,27 @@ int vcm_host(dvbs2fec_handle* h, int n, const int32_t* desc, const void* in, boo
     return 0;
 }
 
-// device buffers: the device entry point's slot, lock and event chaining (dvbs2fec_decode_batch_device)
+// The bracket of the device entry points.  They have their own slot (LDPC workspace, hard decisions, work counter),
+// never shared with the synchronous entry points.  Calls may come on different streams: each one waits for the
+// previous user of the slot (begin) before it touches it, so they are serialised on the device (not on the host) and
+// none of them can race on it, and marks its own end (end) after its last enqueue, also when it fails part-way.
+struct DeviceCall {
+    DevCtx& d;
+    cudaStream_t st;
+    Slot& s = d.slot[2 * kSlots];
+    std::lock_guard<std::mutex> serial{d.dev_mu};
+    int begin() {
+        if (d.dev_used) CU(cudaStreamWaitEvent(st, s.done, 0));
+        return 0;
+    }
+    int end(int rc) {
+        CU(cudaEventRecord(s.done, st));
+        d.dev_used = true;
+        return rc;
+    }
+};
+
+// device buffers, through the device entry points' bracket
 int vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const void* d_in, bool sym, uint8_t* d_bb,
                dvbs2fec_result* d_res, void* cuda_stream) {
     if (!h) return fail(DVBS2FEC_EINVAL, "handle is NULL");
@@ -1095,9 +1078,9 @@ int vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const void* d_in,
     if (!d_in && (sym ? P.sym_off[n] : P.llr_off[n]) > 0) return fail(DVBS2FEC_EINVAL, "input is NULL");
     if (h->devs.empty()) return fail(DVBS2FEC_ENODEV, "no CUDA device");
     DevCtx& d = *h->devs[0];
-    Slot& s = d.slot[2 * kSlots];
-    std::lock_guard<std::mutex> serial(d.dev_mu);
-    cudaStream_t st = (cudaStream_t)cuda_stream;
+    DeviceCall call{d, (cudaStream_t)cuda_stream};
+    Slot& s = call.s;
+    cudaStream_t st = call.st;
     h->last_launches = 0;
     if (n == 0) return 0;
     if (int rc = vcm_plan(h, d, P, sym, std::max(h->cfg.max_batch, 1))) return rc;
@@ -1105,7 +1088,7 @@ int vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const void* d_in,
     if (s.vmeta_copying) CU(cudaEventSynchronize(s.armed));
     s.vmeta_copying = false;
     if (int rc = vcm_reserve(s, P, false)) return rc;
-    if (d.dev_used) CU(cudaStreamWaitEvent(st, s.done, 0));
+    if (int rc = call.begin()) return rc;
     bool need_rec = sym;
     for (const VcmChunk& c : P.chunks) need_rec |= !c.fast;
     if (need_rec) {
@@ -1120,9 +1103,28 @@ int vcm_device(dvbs2fec_handle* h, int n, const int32_t* desc, const void* d_in,
         rc = vcm_chunk(h, d, s, P, c, sym, d_in, 0, s.vmeta.p + c.f0, d_bb, 0, d_res ? d_res + c.f0 : nullptr, st,
                        &h->last_launches);
     }
-    CU(cudaEventRecord(s.done, st));
-    d.dev_used = true;
-    return rc;
+    return call.end(rc);
+}
+
+// frames of the current configuration in device buffers, enqueued on the caller's stream chunk by chunk
+int decode_device(dvbs2fec_handle* h, Input kind, const void* d_in, int n, uint8_t* d_bb, dvbs2fec_result* d_res,
+                  void* cuda_stream) {
+    if (!h || !h->configured || !d_in || n < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
+    DevCtx& d = *h->devs[0];
+    DeviceCall call{d, (cudaStream_t)cuda_stream};
+    if (int rc = call.begin()) return rc;
+    const int chunk = std::min(n, std::max(h->cfg.max_batch, 1));
+    int rc = reserve_slot(h, d, call.s, chunk, Input::llr, false);
+    if (rc) return rc;
+    const size_t kb = h->code->kbch / 8, in_bytes = input_frame_bytes(h, kind);
+    h->last_launches = 0;
+    for (int f0 = 0; f0 < n && !rc; f0 += chunk) {
+        int m = std::min(chunk, n - f0);
+        rc = enqueue_chain(h, d, call.s, kind, static_cast<const uint8_t*>(d_in) + (size_t)f0 * in_bytes, m,
+                           d_bb ? d_bb + (size_t)f0 * kb : nullptr, d_res ? d_res + f0 : nullptr, call.st, &h->last_launches,
+                           (uint64_t)f0);
+    }
+    return call.end(rc);
 }
 
 }  // namespace
@@ -1185,54 +1187,7 @@ int dvbs2fec_create(const dvbs2fec_config* cfg, dvbs2fec_handle** out) {
     return 0;
 }
 
-void dvbs2fec_destroy(dvbs2fec_handle* h) {
-    if (!h) return;
-    {
-        std::unique_lock<std::mutex> lk(h->mu);
-        h->stop = true;
-        h->cv_work.notify_all();
-    }
-    if (h->worker.joinable()) h->worker.join();
-    for (auto& dp : h->devs) {
-        DevCtx& d = *dp;
-        cudaSetDevice(d.device);
-        cudaDeviceSynchronize();   // work enqueued on caller-owned streams by the device entry point
-        for (int k = 0; k < 2 * kSlots + 1; ++k) {
-            Slot& s = d.slot[k];   // (everything on the device has finished: cudaDeviceSynchronize above)
-            s.llr.release(); s.sym.release(); s.idx.release(); s.hard.release(); s.iters.release(); s.corr.release();
-            s.bb.release(); s.res.release(); s.workspace.release(); s.counter.release();
-            s.h_in.release(); s.h_bb.release(); s.h_res.release();
-            s.arrived.release(); s.arrived_vals.release();
-            s.vin.release(); s.vbb.release(); s.vres.release(); s.vmeta.release(); s.h_vmeta.release();
-            s.ts.release(); s.ts_len.release();
-            if (s.done) cudaEventDestroy(s.done);
-            if (s.armed) cudaEventDestroy(s.armed);
-            if (s.copy && !(k >= 1 && k < kSlots)) cudaStreamDestroy(s.copy);   // (slots 1..kSlots-1 borrow slot 0's)
-            if (s.stream) cudaStreamDestroy(s.stream);
-        }
-        for (auto& kv : d.codes) kv.second.row_level.release();
-        for (auto& kv : d.bch) { kv.second.crc.release(); kv.second.basis.release(); }
-        for (auto& kv : d.luts) kv.second.release();
-        d.vcm_demap.release();
-        for (int i = 0; i < 2; ++i) { d.gf_log[i].release(); d.gf_exp[i].release(); }
-        d.prbs.release();
-        d.pl_rn.release();
-    }
-    if (h->ts) dvbs2fec_ts_destroy(h->ts);
-    if (h->ts_done) cudaEventDestroy(h->ts_done);
-    for (auto& sp : h->spans) {
-        cudaEventDestroy(sp.a);
-        cudaEventDestroy(sp.b);
-    }
-    for (auto& S : h->stages) {
-        S.in.release();
-        S.bb.release();
-        S.res.release();
-        S.ts.release();
-        S.ts_len.release();
-    }
-    delete h;
-}
+void dvbs2fec_destroy(dvbs2fec_handle* h) { delete h; }
 
 int dvbs2fec_set_modcod(dvbs2fec_handle* h, int modcod, int shortframes, int pilots, int max_trials) {
     if (!h) return fail(DVBS2FEC_EINVAL, "handle is NULL");
@@ -1246,11 +1201,7 @@ int dvbs2fec_set_modcod(dvbs2fec_handle* h, int modcod, int shortframes, int pil
     h->mc = mc;
     h->code = &ldpc_code(mc.code);
     if (max_trials > 0) h->max_trials = max_trials;
-    h->hard_stride = ((h->code->K / 8) + 15) & ~15;
-    const int nsym = h->code->N / mc.bits;
-    h->plsyms = 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0);
-    h->h_links.clear();
-    for (const LayerLink& l : h->code->links) h->h_links.push_back(((uint32_t)l.group << 16) | l.shift);
+    h->plsyms = plframe_symbols(mc);
     for (auto& d : h->devs) {
         int rc = setup_device_tables(h, *d);
         if (rc) return rc;
@@ -1275,8 +1226,7 @@ int dvbs2fec_set_pl_scrambling(dvbs2fec_handle* h, int codenum) {
             // longest PLFRAME payload: 64800 / 2 symbols + 22 pilot blocks of 36
             std::vector<uint8_t> rn = pl_scrambling_rn(codenum, 32400 + 36 * 22 + 8);
             CU(d.pl_rn.reserve(rn.size()));
-            CU(cudaMemcpy(d.pl_rn.p, rn.data(), rn.size(), cudaMemcpyHostToDevice));
-            CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+            CU(upload(d.pl_rn.p, rn.data(), rn.size()));
         }
         d.demap.rn = codenum >= 0 ? d.pl_rn.p : nullptr;
     }
@@ -1324,7 +1274,7 @@ int dvbs2fec_bb_to_soft(dvbs2fec_handle* h, const float* plframes, int n, int8_t
     if (n == 0) return 0;
     DevCtx& d = *h->devs[0];
     Slot& s = d.slot[0];
-    int rc = reserve_slot(h, d, s, n, 1, false);
+    int rc = reserve_slot(h, d, s, n, Input::sym, false);
     if (rc) return rc;
     CU(cudaMemcpyAsync(s.sym.p, plframes, (size_t)n * h->plsyms * 8, cudaMemcpyHostToDevice, s.stream));
     int e = demap_launch(d.demap, s.sym.p, n, s.llr.p, s.stream);
@@ -1339,24 +1289,15 @@ int dvbs2fec_ldpc_decode(dvbs2fec_handle* h, int8_t* frames, int n, int max_tria
     if (n == 0) return 0;
     DevCtx& d = *h->devs[0];
     Slot& s = d.slot[0];
-    int rc = reserve_slot(h, d, s, n, 0, false);
+    int rc = reserve_slot(h, d, s, n, Input::llr, false);
     if (rc) return rc;
     const size_t bytes = (size_t)n * h->code->N;
     CU(cudaMemcpyAsync(s.llr.p, frames, bytes, cudaMemcpyHostToDevice, s.stream));
     CU(cudaMemsetAsync(s.counter.p, 0, sizeof(unsigned int), s.stream));
-    LdpcArgs la{};
-    la.code = d.ldpc;
-    la.llr_in = s.llr.p;
-    la.nframes = n;
-    la.max_trials = max_trials > 0 ? max_trials : h->max_trials;
-    la.hard_out = s.hard.p;
-    la.hard_stride = h->hard_stride;
-    la.iters_out = s.iters.p;
+    LdpcArgs la = ldpc_args(h, *d.cur, s, s.llr.p, n);
+    if (max_trials > 0) la.max_trials = max_trials;
     la.llr_out = s.llr.p;  // in place, like BBFrameLDPC::decode
-    la.workspace = s.workspace.p;
-    la.work_counter = s.counter.p;
-    la.arrived = nullptr;
-    int e = ldpc_launch(la, std::min(d.grid, (n + 1) / 2), s.stream);
+    int e = ldpc_launch(la, ldpc_grid(*d.cur, n), s.stream);
     if (e) return fail(DVBS2FEC_ECUDA, "ldpc launch: %s", cudaGetErrorString((cudaError_t)e));
     CU(cudaMemcpyAsync(frames, s.llr.p, bytes, cudaMemcpyDeviceToHost, s.stream));
     if (iters) CU(cudaMemcpyAsync(iters, s.iters.p, (size_t)n * 2, cudaMemcpyDeviceToHost, s.stream));
@@ -1369,20 +1310,17 @@ int dvbs2fec_bch_decode(dvbs2fec_handle* h, uint8_t* frames, int n, int16_t* cor
     if (n == 0) return 0;
     DevCtx& d = *h->devs[0];
     Slot& s = d.slot[0];
-    int rc = reserve_slot(h, d, s, n, 0, false);
+    int rc = reserve_slot(h, d, s, n, Input::llr, false);
     if (rc) return rc;
-    const size_t nb = h->code->K / 8;
-    CU(cudaMemsetAsync(s.hard.p, 0, (size_t)n * h->hard_stride, s.stream));
-    CU(cudaMemcpy2DAsync(s.hard.p, h->hard_stride, frames, nb, nb, n, cudaMemcpyHostToDevice, s.stream));
-    BchArgs ba{};
-    ba.code = d.bchd;
-    ba.hard = s.hard.p;
-    ba.hard_stride = h->hard_stride;
-    ba.nframes = n;
+    const size_t nb = h->code->K / 8, stride = d.cur->hard_stride;
+    CU(cudaMemsetAsync(s.hard.p, 0, (size_t)n * stride, s.stream));
+    CU(cudaMemcpy2DAsync(s.hard.p, stride, frames, nb, nb, n, cudaMemcpyHostToDevice, s.stream));
+    BchArgs ba = bch_args(*d.cur, s, n);
     ba.corr_out = s.corr.p;
+    ba.descramble = 0;
     int e = bch_launch(ba, s.stream);
     if (e) return fail(DVBS2FEC_ECUDA, "bch launch: %s", cudaGetErrorString((cudaError_t)e));
-    CU(cudaMemcpy2DAsync(frames, nb, s.hard.p, h->hard_stride, nb, n, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpy2DAsync(frames, nb, s.hard.p, stride, nb, n, cudaMemcpyDeviceToHost, s.stream));
     if (corrections) CU(cudaMemcpyAsync(corrections, s.corr.p, (size_t)n * 2, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaStreamSynchronize(s.stream));
     return 0;
@@ -1404,11 +1342,11 @@ int dvbs2fec_descramble(dvbs2fec_handle* h, uint8_t* frames, int stride, int n) 
 }
 
 int dvbs2fec_decode_batch(dvbs2fec_handle* h, const int8_t* llr, int n, uint8_t* bb_out, dvbs2fec_result* results) {
-    return decode_host(h, llr, nullptr, n, bb_out, results);
+    return decode_host(h, Input::llr, llr, n, bb_out, results);
 }
 int dvbs2fec_decode_plframes(dvbs2fec_handle* h, const float* plframes, int n, uint8_t* bb_out,
                              dvbs2fec_result* results) {
-    return decode_host(h, nullptr, plframes, n, bb_out, results);
+    return decode_host(h, Input::sym, plframes, n, bb_out, results);
 }
 
 int dvbs2fec_quantize_plframes(const dvbs2fec_handle* h, const float* plframes, int n, uint8_t* idx_out) {
@@ -1445,58 +1383,19 @@ int dvbs2fec_quantize_plframes(const dvbs2fec_handle* h, const float* plframes, 
 }
 
 int dvbs2fec_decode_plframes_idx(dvbs2fec_handle* h, const uint8_t* idx, int n, uint8_t* bb_out, dvbs2fec_result* results) {
-    return decode_host(h, nullptr, nullptr, n, bb_out, results, idx);
+    return decode_host(h, Input::idx, idx, n, bb_out, results);
 }
 
 int dvbs2fec_decode_batch_device(dvbs2fec_handle* h, const int8_t* d_llr, int n, uint8_t* d_bb_out,
                                  dvbs2fec_result* d_results, void* cuda_stream) {
-    if (!h || !h->configured || !d_llr || n < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
-    DevCtx& d = *h->devs[0];
-    // Own scratch (LDPC workspace, hard decisions, work counter), never shared with the synchronous entry points.
-    // Calls may come on different streams: each one waits for the previous user of the scratch, so they are
-    // serialised on the device (not on the host) and none of them can race on it.
-    Slot& s = d.slot[2 * kSlots];
-    std::lock_guard<std::mutex> serial(d.dev_mu);
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    if (d.dev_used) CU(cudaStreamWaitEvent(st, s.done, 0));
-    const int chunk = std::min(n, std::max(h->cfg.max_batch, 1));
-    int rc = reserve_slot(h, d, s, chunk, 0, false);
-    if (rc) return rc;
-    const size_t kb = h->code->kbch / 8;
-    h->last_launches = 0;
-    for (int f0 = 0; f0 < n && !rc; f0 += chunk) {
-        int m = std::min(chunk, n - f0);
-        rc = enqueue_chain(h, d, s, nullptr, d_llr + (size_t)f0 * h->code->N, m, d_bb_out ? d_bb_out + (size_t)f0 * kb : nullptr,
-                           d_results ? d_results + f0 : nullptr, st, &h->last_launches, (uint64_t)f0);
-    }
-    CU(cudaEventRecord(s.done, st));
-    d.dev_used = true;
-    return rc;
+    return decode_device(h, Input::llr, d_llr, n, d_bb_out, d_results, cuda_stream);
 }
 
 // PLFRAME symbols already on the device (e.g. what dvbs2fec_pll_process_device left there): demapper, LDPC, BCH and
 // descrambler enqueued on the caller's stream, nothing crosses PCIe.  Shares the device entry point's scratch.
 int dvbs2fec_decode_plframes_device(dvbs2fec_handle* h, const float* d_plframes, int n, uint8_t* d_bb_out,
                                     dvbs2fec_result* d_results, void* cuda_stream) {
-    if (!h || !h->configured || !d_plframes || n < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
-    DevCtx& d = *h->devs[0];
-    Slot& s = d.slot[2 * kSlots];
-    std::lock_guard<std::mutex> serial(d.dev_mu);
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    if (d.dev_used) CU(cudaStreamWaitEvent(st, s.done, 0));
-    const int chunk = std::min(n, std::max(h->cfg.max_batch, 1));
-    int rc = reserve_slot(h, d, s, chunk, 0, false);
-    if (rc) return rc;
-    const size_t kb = h->code->kbch / 8;
-    h->last_launches = 0;
-    for (int f0 = 0; f0 < n && !rc; f0 += chunk) {
-        int m = std::min(chunk, n - f0);
-        rc = enqueue_chain(h, d, s, d_plframes + (size_t)f0 * h->plsyms * 2, nullptr, m, d_bb_out ? d_bb_out + (size_t)f0 * kb : nullptr,
-                           d_results ? d_results + f0 : nullptr, st, &h->last_launches, (uint64_t)f0);
-    }
-    CU(cudaEventRecord(s.done, st));
-    d.dev_used = true;
-    return rc;
+    return decode_device(h, Input::sym, d_plframes, n, d_bb_out, d_results, cuda_stream);
 }
 
 int dvbs2fec_vcm_layout(int n, const int32_t* desc, int64_t* sym_off, int64_t* llr_off, int64_t* bb_off) {
@@ -1550,7 +1449,7 @@ static void stream_copy(void* dst_v, const void* src_v, size_t n) {
 
 // The slot of the next frame in the staging batch being filled (opening a batch if need be).  Called with h->mu held
 // through `lk`, which is dropped while page-locked memory is allocated.
-static int acquire_slot(dvbs2fec_handle* h, std::unique_lock<std::mutex>& lk, int kind, uint8_t** slot) {
+static int acquire_slot(dvbs2fec_handle* h, std::unique_lock<std::mutex>& lk, Input kind, uint8_t** slot) {
     if (!h->worker.joinable()) h->worker = std::thread(worker_main, h);
     if (h->st_fill >= 0 && h->stages[h->st_fill].n > 0 && h->stages[h->st_fill].kind != kind) {
         h->st_ready.push_back(h->st_fill);   // a batch holds one kind of input: close the pending one
@@ -1606,23 +1505,22 @@ static void commit_slot(dvbs2fec_handle* h, uint64_t tag) {
     }
 }
 
-static int submit_common(dvbs2fec_handle* h, const int8_t* llr, const float* sym, uint64_t tag, const uint8_t* idx = nullptr) {
+static int submit_common(dvbs2fec_handle* h, Input kind, const void* frame, uint64_t tag) {
     if (!h || !h->configured) return fail(DVBS2FEC_EINVAL, "set_modcod has not been called");
     std::lock_guard<std::mutex> producer(h->submit_mu);
     std::unique_lock<std::mutex> lk(h->mu);
     if (h->acquired) return fail(DVBS2FEC_EINVAL, "a frame acquired with dvbs2fec_acquire_* has not been committed");
     uint8_t* slot = nullptr;
-    const int kind = sym ? 1 : idx ? 2 : 0;
     int rc = acquire_slot(h, lk, kind, &slot);
     if (rc) return rc;
-    stream_copy(slot, sym ? (const void*)sym : idx ? (const void*)idx : (const void*)llr, h->stages[h->st_fill].in_bytes);
+    stream_copy(slot, frame, h->stages[h->st_fill].in_bytes);
     commit_slot(h, tag);
     return 0;
 }
 
-static int acquire_common(dvbs2fec_handle* h, int kind, void** slot) {
+static int acquire_common(dvbs2fec_handle* h, Input kind, void** slot) {
     if (!h || !h->configured || !slot) return fail(DVBS2FEC_EINVAL, "bad arguments");
-    if (kind == 2 && h->mc.constellation == APSK32) return fail(DVBS2FEC_EINVAL, "32APSK has no LUT in the reference: send symbols");
+    if (kind == Input::idx && h->mc.constellation == APSK32) return fail(DVBS2FEC_EINVAL, "32APSK has no LUT in the reference: send symbols");
     std::lock_guard<std::mutex> producer(h->submit_mu);
     std::unique_lock<std::mutex> lk(h->mu);
     if (h->acquired) return fail(DVBS2FEC_EINVAL, "the previous frame has not been committed");
@@ -1636,23 +1534,23 @@ static int acquire_common(dvbs2fec_handle* h, int kind, void** slot) {
 
 int dvbs2fec_submit_llr(dvbs2fec_handle* h, const int8_t* llr, uint64_t tag) {
     if (!llr) return fail(DVBS2FEC_EINVAL, "llr is NULL");
-    return submit_common(h, llr, nullptr, tag);
+    return submit_common(h, Input::llr, llr, tag);
 }
 int dvbs2fec_submit_plframe(dvbs2fec_handle* h, const float* plframe, int nsym, uint64_t tag) {
     if (!plframe || !h || !h->configured || nsym != h->plsyms)
         return fail(DVBS2FEC_EINVAL, "plframe must hold dvbs2fec_plframe_symbols() complex samples");
-    return submit_common(h, nullptr, plframe, tag);
+    return submit_common(h, Input::sym, plframe, tag);
 }
 
 int dvbs2fec_submit_plframe_idx(dvbs2fec_handle* h, const uint8_t* idx, uint64_t tag) {
     if (!idx || !h || !h->configured) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (h->mc.constellation == APSK32) return fail(DVBS2FEC_EINVAL, "32APSK has no LUT in the reference: send symbols");
-    return submit_common(h, nullptr, nullptr, tag, idx);
+    return submit_common(h, Input::idx, idx, tag);
 }
 
-int dvbs2fec_acquire_llr(dvbs2fec_handle* h, int8_t** slot) { return acquire_common(h, 0, reinterpret_cast<void**>(slot)); }
-int dvbs2fec_acquire_plframe(dvbs2fec_handle* h, float** slot) { return acquire_common(h, 1, reinterpret_cast<void**>(slot)); }
-int dvbs2fec_acquire_plframe_idx(dvbs2fec_handle* h, uint8_t** slot) { return acquire_common(h, 2, reinterpret_cast<void**>(slot)); }
+int dvbs2fec_acquire_llr(dvbs2fec_handle* h, int8_t** slot) { return acquire_common(h, Input::llr, reinterpret_cast<void**>(slot)); }
+int dvbs2fec_acquire_plframe(dvbs2fec_handle* h, float** slot) { return acquire_common(h, Input::sym, reinterpret_cast<void**>(slot)); }
+int dvbs2fec_acquire_plframe_idx(dvbs2fec_handle* h, uint8_t** slot) { return acquire_common(h, Input::idx, reinterpret_cast<void**>(slot)); }
 int dvbs2fec_commit(dvbs2fec_handle* h, uint64_t tag) {
     if (!h || !h->configured) return fail(DVBS2FEC_EINVAL, "bad arguments");
     std::lock_guard<std::mutex> producer(h->submit_mu);
@@ -1664,16 +1562,31 @@ int dvbs2fec_commit(dvbs2fec_handle* h, uint64_t tag) {
     return 0;
 }
 
+// collect: wait up to timeout_us (< 0: for ever) for a finished stage (h->mu held through lk)
+static void wait_for_done(dvbs2fec_handle* h, std::unique_lock<std::mutex>& lk, int timeout_us) {
+    if (!h->st_done.empty() || timeout_us == 0) return;
+    auto ready = [h] { return !h->st_done.empty(); };
+    if (timeout_us < 0)
+        h->cv_done.wait(lk, ready);
+    else
+        h->cv_done.wait_for(lk, std::chrono::microseconds(timeout_us), ready);
+}
+// the record of frame i of a finished stage; a stage that failed to launch has decoded nothing
+static dvbs2fec_result stage_record(const dvbs2fec_handle::Stage& S, int i) {
+    dvbs2fec_result r = S.res.p[i];
+    r.tag = S.tags[i];
+    if (S.rc) {
+        r.ldpc_iters = -1;
+        r.bch_corr = -1;
+        r.flags = DVBS2FEC_FLAG_LDPC_FAIL | DVBS2FEC_FLAG_BCH_FAIL;
+    }
+    return r;
+}
+
 int dvbs2fec_collect(dvbs2fec_handle* h, uint8_t* bb_out, dvbs2fec_result* results, int max, int timeout_us) {
     if (!h || !h->configured || max < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
     std::unique_lock<std::mutex> lk(h->mu);
-    if (h->st_done.empty() && timeout_us != 0) {
-        auto ready = [h] { return !h->st_done.empty(); };
-        if (timeout_us < 0)
-            h->cv_done.wait(lk, ready);
-        else
-            h->cv_done.wait_for(lk, std::chrono::microseconds(timeout_us), ready);
-    }
+    wait_for_done(h, lk, timeout_us);
     int n = 0;
     const size_t kb = h->code->kbch / 8;
     while (n < max && !h->st_done.empty()) {
@@ -1686,16 +1599,7 @@ int dvbs2fec_collect(dvbs2fec_handle* h, uint8_t* bb_out, dvbs2fec_result* resul
                 for (int i = 0; i < k; ++i) memcpy(bb_out + (size_t)(n + i) * kb, S.bb.p + (size_t)(S.taken + i) * S.kb, std::min(kb, S.kb));
         }
         if (results)
-            for (int i = 0; i < k; ++i) {
-                dvbs2fec_result r = S.res.p[S.taken + i];
-                r.tag = S.tags[S.taken + i];
-                if (S.rc) {
-                    r.ldpc_iters = -1;
-                    r.bch_corr = -1;
-                    r.flags = DVBS2FEC_FLAG_LDPC_FAIL | DVBS2FEC_FLAG_BCH_FAIL;
-                }
-                results[n + i] = r;
-            }
+            for (int i = 0; i < k; ++i) results[n + i] = stage_record(S, S.taken + i);
         S.taken += k;
         n += k;
         if (S.taken == S.n) {
@@ -1730,13 +1634,7 @@ int dvbs2fec_collect_ts(dvbs2fec_handle* h, uint8_t* ts_out, int cap, dvbs2fec_r
     if (nresults) *nresults = 0;
     if (!h || !h->configured || !ts_out || cap < 0 || max_results < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
     std::unique_lock<std::mutex> lk(h->mu);
-    if (h->st_done.empty() && timeout_us != 0) {
-        auto ready = [h] { return !h->st_done.empty(); };
-        if (timeout_us < 0)
-            h->cv_done.wait(lk, ready);
-        else
-            h->cv_done.wait_for(lk, std::chrono::microseconds(timeout_us), ready);
-    }
+    wait_for_done(h, lk, timeout_us);
     int bytes = 0, nres = 0;
     while (!h->st_done.empty()) {
         dvbs2fec_handle::Stage& S = h->stages[h->st_done.front()];
@@ -1749,16 +1647,7 @@ int dvbs2fec_collect_ts(dvbs2fec_handle* h, uint8_t* ts_out, int cap, dvbs2fec_r
         if (S.ts_taken < total) break;   // no room for the rest: next call
         if (results) {                   // the batch's records follow its last packets, as many as fit
             const int k = std::min(max_results - nres, S.n - S.res_taken);
-            for (int i = S.res_taken; i < S.res_taken + k; ++i) {
-                dvbs2fec_result r = S.res.p[i];
-                r.tag = S.tags[i];
-                if (S.rc) {
-                    r.ldpc_iters = -1;
-                    r.bch_corr = -1;
-                    r.flags = DVBS2FEC_FLAG_LDPC_FAIL | DVBS2FEC_FLAG_BCH_FAIL;
-                }
-                results[nres++] = r;
-            }
+            for (int i = S.res_taken; i < S.res_taken + k; ++i) results[nres++] = stage_record(S, i);
             S.res_taken += k;
             if (S.res_taken < S.n) break;   // the rest of the records: next call
         }
@@ -1806,24 +1695,7 @@ int dvbs2fec_ts_create(int device, dvbs2fec_ts_parser** out) {
     return 0;
 }
 
-void dvbs2fec_ts_destroy(dvbs2fec_ts_parser* p) {
-    if (!p) return;
-    cudaSetDevice(p->device);
-    if (p->stream) {
-        cudaStreamSynchronize(p->stream);
-        cudaStreamDestroy(p->stream);
-    }
-    p->state.release();
-    p->plan.release();
-    p->meta.release();
-    p->bb.release();
-    p->out.release();
-    p->h_produced.release();
-    p->gstate.release(); p->gbuf.release(); p->g_sync.release(); p->g_doff.release(); p->g_before.release();
-    p->g_nxt.release(); p->g_aux.release(); p->g_aux2.release(); p->g_desc.release(); p->g_out.release();
-    p->g_crc0.release(); p->g_xpow.release();
-    delete p;
-}
+void dvbs2fec_ts_destroy(dvbs2fec_ts_parser* p) { delete p; }
 
 int dvbs2fec_ts_set_frame_size(dvbs2fec_ts_parser* p, int kbch_bits) {
     if (!p || kbch_bits < 88 || kbch_bits > 65535 || kbch_bits % 8) return fail(DVBS2FEC_EINVAL, "bad frame size");
@@ -2016,8 +1888,7 @@ int dvbs2fec_modulate(int modcod, int shortframes, int pilots, const uint8_t* co
     const LdpcCode& c = ldpc_code(mc.code);
     ConstellationHost ch = make_constellation(mc.constellation, mc.g1, mc.g2);
     const int nsym = c.N / mc.bits;
-    const int total = 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0);
-    memset(plframe, 0, (size_t)total * 8);
+    memset(plframe, 0, (size_t)plframe_symbols(mc) * 8);
     std::vector<uint8_t> tx(c.N);
     for (int n = 0; n < c.N; ++n) tx[interleaved_position(mc, n)] = code_bits[n] & 1;
     for (int s = 0; s < nsym; ++s) {
@@ -2033,13 +1904,12 @@ int dvbs2fec_modcod_info(int modcod, int shortframes, int pilots, int* nldpc, in
     if (!modcod_config(modcod, shortframes != 0, pilots != 0, &mc) || mc.code < 0)
         return fail(DVBS2FEC_EINVAL, "unsupported MODCOD/frame size");
     const LdpcCode& c = ldpc_code(mc.code);
-    const int nsym = c.N / mc.bits;
     if (nldpc) *nldpc = c.N;
     if (kldpc) *kldpc = c.K;
     if (kbch) *kbch = c.kbch;
     if (bch_t) *bch_t = c.bch_t;
     if (bits_per_symbol) *bits_per_symbol = mc.bits;
-    if (plframe_symbols) *plframe_symbols = 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0);
+    if (plframe_symbols) *plframe_symbols = s2::plframe_symbols(mc);
     if (links_total) *links_total = c.links_total;
     return 0;
 }

@@ -8,78 +8,43 @@
 #include "../../include/dvbs2fec.h"
 
 #include <algorithm>
-#include <cstdio>
 #include <memory>
 
 #include <cuda_runtime.h>
 
-namespace s2 {
-int api_fail(int code, const char* msg);
-}
-using s2::api_fail;
+#include "abi_util.h"
 
-namespace {
-int failf(int code, const char* what, cudaError_t e) {
-    char buf[300];
-    snprintf(buf, sizeof buf, "%s: %s", what, cudaGetErrorString(e));
-    return api_fail(code, buf);
-}
-#define CU(call)                                                     \
-    do {                                                             \
-        cudaError_t e_ = (call);                                     \
-        if (e_ != cudaSuccess) return failf(DVBS2FEC_ECUDA, #call, e_); \
-    } while (0)
-
-template <typename T>
-cudaError_t reserve(T*& p, size_t& cap, size_t n, bool zero = false) {
-    if (n <= cap) return cudaSuccess;
-    T* q = nullptr;
-    cudaError_t e = cudaMalloc(&q, n * sizeof(T));
-    if (e != cudaSuccess) return e;
-    if (zero) {
-        cudaMemset(q, 0, n * sizeof(T));
-        if (p) cudaMemcpy(q, p, cap * sizeof(T), cudaMemcpyDeviceToDevice);      // grows without forgetting
-        cudaDeviceSynchronize();      // both are asynchronous, and the decoder's stream does not wait for the default stream
-    }
-    if (p) cudaFree(p);
-    p = q;
-    cap = n;
-    return cudaSuccess;
-}
-}  // namespace
+using namespace s2;
 
 struct dvbs2fec_dvbs_demod {
     int device = 0, frame_stride = 204;
     dvbs2fec_dvbs_viterbi* vit = nullptr;
     dvbs2fec_dvbs_deframer* def = nullptr;
     dvbs2fec_dvbs_outer* outer = nullptr;
-    float* d_syms = nullptr; size_t syms_cap = 0;
-    int8_t* d_soft = nullptr; size_t soft_cap = 0;
-    uint8_t* d_bits = nullptr; size_t bits_cap = 0;      // persists: what the decoder leaves unwritten (rate 5/6) is what was there
-    uint8_t* d_frames = nullptr; size_t frames_cap = 0;
-    uint8_t* d_ts = nullptr; size_t ts_cap = 0;
-    int32_t* d_err = nullptr; size_t err_cap = 0;
+    DevBuf<float> d_syms;
+    DevBuf<int8_t> d_soft;
+    DevBuf<uint8_t> d_bits;      // persists: what the decoder leaves unwritten (rate 5/6) is what was there
+    DevBuf<uint8_t> d_frames, d_ts;
+    DevBuf<int32_t> d_err;
     int errors[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     int frames_found = 0, frames_done = 0;
+    ~dvbs2fec_dvbs_demod() {
+        cudaSetDevice(device);
+        dvbs2fec_dvbs_viterbi_destroy(vit);
+        dvbs2fec_dvbs_deframer_destroy(def);
+        dvbs2fec_dvbs_outer_destroy(outer);
+    }
 };
 
 extern "C" {
 
-void dvbs2fec_dvbs_demod_destroy(dvbs2fec_dvbs_demod* p) {
-    if (!p) return;
-    cudaSetDevice(p->device);
-    dvbs2fec_dvbs_viterbi_destroy(p->vit);
-    dvbs2fec_dvbs_deframer_destroy(p->def);
-    dvbs2fec_dvbs_outer_destroy(p->outer);
-    cudaFree(p->d_syms); cudaFree(p->d_soft); cudaFree(p->d_bits); cudaFree(p->d_frames); cudaFree(p->d_ts); cudaFree(p->d_err);
-    delete p;
-}
+void dvbs2fec_dvbs_demod_destroy(dvbs2fec_dvbs_demod* p) { delete p; }
 
 int dvbs2fec_dvbs_demod_create(int device, float ber_threshold, int max_outsync, int frame_stride, dvbs2fec_dvbs_demod** out) {
-    if (!out) return api_fail(DVBS2FEC_EINVAL, "out is NULL");
+    if (!out) return fail(DVBS2FEC_EINVAL, "out is NULL");
     *out = nullptr;
-    if (frame_stride != 204 && frame_stride != 1632) return api_fail(DVBS2FEC_EINVAL, "frame_stride is 204 (as the module) or 1632 (back-to-back frames)");
-    std::unique_ptr<dvbs2fec_dvbs_demod, void (*)(dvbs2fec_dvbs_demod*)> p(new dvbs2fec_dvbs_demod(), dvbs2fec_dvbs_demod_destroy);
+    if (frame_stride != 204 && frame_stride != 1632) return fail(DVBS2FEC_EINVAL, "frame_stride is 204 (as the module) or 1632 (back-to-back frames)");
+    std::unique_ptr<dvbs2fec_dvbs_demod> p(new dvbs2fec_dvbs_demod());
     p->device = device;
     p->frame_stride = frame_stride;
     int rc = dvbs2fec_dvbs_viterbi_create(device, ber_threshold, max_outsync, &p->vit);
@@ -91,13 +56,13 @@ int dvbs2fec_dvbs_demod_create(int device, float ber_threshold, int max_outsync,
 }
 
 int dvbs2fec_dvbs_demod_reset(dvbs2fec_dvbs_demod* p) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     int rc = dvbs2fec_dvbs_viterbi_reset(p->vit);
     if (!rc) rc = dvbs2fec_dvbs_deframer_reset(p->def);
     if (!rc) rc = dvbs2fec_dvbs_outer_reset(p->outer);
     if (rc) return rc;
     CU(cudaSetDevice(p->device));
-    if (p->d_bits) CU(cudaMemset(p->d_bits, 0, p->bits_cap));
+    if (p->d_bits.p) CU(cudaMemset(p->d_bits.p, 0, p->d_bits.cap));
     CU(cudaDeviceSynchronize());
     std::fill(p->errors, p->errors + 8, 0);
     p->frames_found = p->frames_done = 0;
@@ -105,24 +70,26 @@ int dvbs2fec_dvbs_demod_reset(dvbs2fec_dvbs_demod* p) {
 }
 
 int dvbs2fec_dvbs_demod_process(dvbs2fec_dvbs_demod* p, int count, const float* syms, uint8_t* out, int out_cap) {
-    if (!p || count < 0 || out_cap < 0 || (count && !syms) || (out_cap && !out)) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || count < 0 || out_cap < 0 || (count && !syms) || (out_cap && !out)) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!count) return 0;
-    if (count > (1 << 23)) return api_fail(DVBS2FEC_EINVAL, "more than 2^23 symbols in one call");
+    if (count > (1 << 23)) return fail(DVBS2FEC_EINVAL, "more than 2^23 symbols in one call");
     CU(cudaSetDevice(p->device));
     const size_t nsoft_max = (size_t)2 * count + 8192;
-    CU(reserve(p->d_syms, p->syms_cap, (size_t)2 * count));
-    CU(reserve(p->d_soft, p->soft_cap, nsoft_max));
-    CU(reserve(p->d_bits, p->bits_cap, nsoft_max, true));
-    CU(cudaMemcpy(p->d_syms, syms, sizeof(float) * 2 * count, cudaMemcpyHostToDevice));
-    CU(cudaDeviceSynchronize());      // a pageable copy returns once staged; the stages' own streams do not wait for the default stream
-    const int nsoft = dvbs2fec_dvbs_sts_process_device(p->vit, count, p->d_syms, p->d_soft);      // :80
+    CU(p->d_syms.reserve((size_t)2 * count));
+    CU(p->d_soft.reserve(nsoft_max));
+    const size_t had = p->d_bits.cap;      // d_bits grows without forgetting, and from zeros
+    CU(p->d_bits.grow(nsoft_max, had, nullptr));
+    if (p->d_bits.cap > had) CU(cudaMemset(p->d_bits.p + had, 0, p->d_bits.cap - had));
+    CU(cudaMemcpy(p->d_syms.p, syms, sizeof(float) * 2 * count, cudaMemcpyHostToDevice));
+    CU(cudaDeviceSynchronize());      // a pageable copy and a memset return early; the stages' own streams do not wait for the default stream
+    const int nsoft = dvbs2fec_dvbs_sts_process_device(p->vit, count, p->d_syms.p, p->d_soft.p);      // :80
     if (nsoft <= 0) return nsoft;
-    const int nbits = dvbs2fec_dvbs_viterbi_process_device(p->vit, nsoft, p->d_soft, p->d_bits);      // :81
+    const int nbits = dvbs2fec_dvbs_viterbi_process_device(p->vit, nsoft, p->d_soft.p, p->d_bits.p);      // :81
     if (nbits <= 0) return nbits;
     // :82 -- a frame needs 13056 new bits unless sync patterns overlap; room for one frame per 1632 bits and a few more
     const int max_frames = nbits / 1632 + 8;
-    CU(reserve(p->d_frames, p->frames_cap, (size_t)max_frames * 1632));
-    int rc = dvbs2fec_dvbs_deframer_work_device(p->def, p->d_bits, nbits, p->d_frames, max_frames, nullptr, nullptr);
+    CU(p->d_frames.reserve((size_t)max_frames * 1632));
+    int rc = dvbs2fec_dvbs_deframer_work_device(p->def, p->d_bits.p, nbits, p->d_frames.p, max_frames, nullptr, nullptr);
     if (rc) return rc;
     int found = 0;
     const int nframes = dvbs2fec_dvbs_deframer_stats(p->def, nullptr, nullptr, &found);      // synchronises
@@ -130,19 +97,19 @@ int dvbs2fec_dvbs_demod_process(dvbs2fec_dvbs_demod* p, int count, const float* 
     p->frames_found = found;
     p->frames_done = nframes;
     if (!nframes) return 0;
-    if ((long long)nframes * 8 * 188 > out_cap) return api_fail(DVBS2FEC_ENOSPC, "TS output does not fit out_cap");
-    CU(reserve(p->d_ts, p->ts_cap, (size_t)nframes * 8 * 188));
-    CU(reserve(p->d_err, p->err_cap, (size_t)nframes * 8));
-    const int nb = dvbs2fec_dvbs_outer_process_device(p->outer, nframes, p->frame_stride, p->d_frames, p->d_ts, p->d_err, nullptr);      // :85-100
+    if ((long long)nframes * 8 * 188 > out_cap) return fail(DVBS2FEC_ENOSPC, "TS output does not fit out_cap");
+    CU(p->d_ts.reserve((size_t)nframes * 8 * 188));
+    CU(p->d_err.reserve((size_t)nframes * 8));
+    const int nb = dvbs2fec_dvbs_outer_process_device(p->outer, nframes, p->frame_stride, p->d_frames.p, p->d_ts.p, p->d_err.p, nullptr);      // :85-100
     if (nb < 0) return nb;
-    CU(cudaMemcpy(out, p->d_ts, (size_t)nframes * 8 * 188, cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(p->errors, p->d_err + (size_t)(nframes - 1) * 8, sizeof(int) * 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out, p->d_ts.p, (size_t)nframes * 8 * 188, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(p->errors, p->d_err.p + (size_t)(nframes - 1) * 8, sizeof(int) * 8, cudaMemcpyDeviceToHost));
     return nframes * 8 * 188;
 }
 
 int dvbs2fec_dvbs_demod_stats(dvbs2fec_dvbs_demod* p, float* viterbi_ber, int* viterbi_lock, int* viterbi_rate, float* rs_avg, int* deframer_err,
                               int* frames_found, int* frames_done) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     int rc = dvbs2fec_dvbs_viterbi_stats(p->vit, viterbi_ber, viterbi_lock, viterbi_rate, nullptr, nullptr, nullptr);      // :101-113
     if (rc) return rc;
     if (rs_avg) {      // :114 (integer division, as there)

@@ -16,16 +16,14 @@
 // oracle and in the harness around the compiled reference -- it starts from zeros.
 #include "../../include/dvbs2fec.h"
 
-#include <cstdio>
 #include <cstring>
 #include <memory>
 
 #include <cuda_runtime.h>
 
-namespace s2 {
-int api_fail(int code, const char* msg);
-}
-using s2::api_fail;
+#include "abi_util.h"
+
+using namespace s2;
 
 namespace {
 
@@ -148,93 +146,65 @@ __global__ void __launch_bounds__(256) carry_kernel(const uint8_t* __restrict__ 
     if (i < kCarry) next[i] = (uint8_t)stream_bit(hist, in, size, (long long)size + i);
 }
 
-int failf(int code, const char* what, cudaError_t e) {
-    char buf[300];
-    snprintf(buf, sizeof buf, "%s: %s", what, cudaGetErrorString(e));
-    return api_fail(code, buf);
-}
-#define CU(call)                                                     \
-    do {                                                             \
-        cudaError_t e_ = (call);                                     \
-        if (e_ != cudaSuccess) return failf(DVBS2FEC_ECUDA, #call, e_); \
-    } while (0)
-
-template <typename T>
-cudaError_t reserve(T*& p, size_t& cap, size_t n) {
-    if (n <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-    cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-    if (e == cudaSuccess) cap = n;
-    return e;
-}
-
 }  // namespace
 
 struct dvbs2fec_dvbs_deframer {
     int device = 0;
     cudaStream_t stream = nullptr;
-    DeframerState* st = nullptr;
-    uint8_t* hist[2] = {nullptr, nullptr};
+    DevBuf<DeframerState> st;
+    DevBuf<uint8_t> hist[2];
     int cur = 0;
-    uint32_t* W = nullptr; size_t W_cap = 0;
-    uint32_t* blockhits = nullptr; size_t bh_cap = 0;
-    int* counts = nullptr; size_t cnt_cap = 0;
-    uint32_t* hits = nullptr; size_t hits_cap = 0;
-    uint8_t* in = nullptr; size_t in_cap = 0;
-    uint32_t* out = nullptr; size_t out_cap = 0;
+    DevBuf<uint32_t> W, blockhits, hits, out;
+    DevBuf<int> counts;
+    DevBuf<uint8_t> in;
+    ~dvbs2fec_dvbs_deframer() {
+        cudaSetDevice(device);
+        if (stream) {
+            cudaStreamSynchronize(stream);
+            cudaStreamDestroy(stream);
+        }
+    }
 };
 
 extern "C" {
 
 int dvbs2fec_dvbs_deframer_reset(dvbs2fec_dvbs_deframer* p) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
-    CU(cudaMemset(p->st, 0, sizeof(DeframerState)));
-    CU(cudaMemset(p->hist[0], 0, kWindow));
-    CU(cudaMemset(p->hist[1], 0, kWindow));
+    CU(cudaMemset(p->st.p, 0, sizeof(DeframerState)));
+    CU(cudaMemset(p->hist[0].p, 0, kWindow));
+    CU(cudaMemset(p->hist[1].p, 0, kWindow));
     CU(cudaDeviceSynchronize());      // device memsets are asynchronous, and the callers' streams do not wait for the default stream
     p->cur = 0;
     return 0;
 }
 
 int dvbs2fec_dvbs_deframer_create(int device, dvbs2fec_dvbs_deframer** out) {
-    if (!out) return api_fail(DVBS2FEC_EINVAL, "out is NULL");
+    if (!out) return fail(DVBS2FEC_EINVAL, "out is NULL");
     *out = nullptr;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return api_fail(DVBS2FEC_ENODEV, "no CUDA device");
-    if (device < 0 || device >= ndev) return api_fail(DVBS2FEC_EINVAL, "device out of range");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(DVBS2FEC_ENODEV, "no CUDA device");
+    if (device < 0 || device >= ndev) return fail(DVBS2FEC_EINVAL, "device out of range");
     std::unique_ptr<dvbs2fec_dvbs_deframer> p(new dvbs2fec_dvbs_deframer());
     p->device = device;
     CU(cudaSetDevice(device));
     CU(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
-    CU(cudaMalloc(&p->st, sizeof(DeframerState)));
-    CU(cudaMalloc(&p->hist[0], kWindow));
-    CU(cudaMalloc(&p->hist[1], kWindow));
+    CU(p->st.reserve(1));
+    CU(p->hist[0].reserve(kWindow));
+    CU(p->hist[1].reserve(kWindow));
     int rc = dvbs2fec_dvbs_deframer_reset(p.get());
     if (rc) return rc;
     *out = p.release();
     return 0;
 }
 
-void dvbs2fec_dvbs_deframer_destroy(dvbs2fec_dvbs_deframer* p) {
-    if (!p) return;
-    cudaSetDevice(p->device);
-    if (p->stream) {
-        cudaStreamSynchronize(p->stream);
-        cudaStreamDestroy(p->stream);
-    }
-    cudaFree(p->st); cudaFree(p->hist[0]); cudaFree(p->hist[1]); cudaFree(p->W); cudaFree(p->blockhits); cudaFree(p->counts);
-    cudaFree(p->hits); cudaFree(p->in); cudaFree(p->out);
-    delete p;
-}
+void dvbs2fec_dvbs_deframer_destroy(dvbs2fec_dvbs_deframer* p) { delete p; }
 
 int dvbs2fec_dvbs_deframer_work_device(dvbs2fec_dvbs_deframer* p, const uint8_t* d_bits, int size, uint8_t* d_frames, int max_frames,
                                        int32_t* d_nframes, void* stream) {
-    if (!p || size < 0 || max_frames < 0 || (size && !d_bits) || (max_frames && !d_frames)) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
-    if (size >= (1 << 24)) return api_fail(DVBS2FEC_EINVAL, "more than 2^24 - 1 bits in one call");
-    if ((reinterpret_cast<uintptr_t>(d_frames) & 3u) != 0) return api_fail(DVBS2FEC_EINVAL, "frame buffer must be 4-byte aligned");
+    if (!p || size < 0 || max_frames < 0 || (size && !d_bits) || (max_frames && !d_frames)) return fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (size >= (1 << 24)) return fail(DVBS2FEC_EINVAL, "more than 2^24 - 1 bits in one call");
+    if ((reinterpret_cast<uintptr_t>(d_frames) & 3u) != 0) return fail(DVBS2FEC_EINVAL, "frame buffer must be 4-byte aligned");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (!size) {
@@ -242,49 +212,49 @@ int dvbs2fec_dvbs_deframer_work_device(dvbs2fec_dvbs_deframer* p, const uint8_t*
         return 0;
     }
     const int nwords = (kCarry + size + 31) / 32 + 2, nblocks = (size + kDetect - 1) / kDetect;
-    if ((size_t)nwords > p->W_cap || (size_t)nblocks > p->cnt_cap || (size_t)max_frames + 1 > p->hits_cap) {
+    if ((size_t)nwords > p->W.cap || (size_t)nblocks > p->counts.cap || (size_t)max_frames + 1 > p->hits.cap) {
         CU(cudaStreamSynchronize(st));
-        CU(reserve(p->W, p->W_cap, (size_t)nwords));
-        CU(reserve(p->blockhits, p->bh_cap, (size_t)nblocks * kDetect));
-        CU(reserve(p->counts, p->cnt_cap, (size_t)nblocks));
-        CU(reserve(p->hits, p->hits_cap, (size_t)max_frames + 1));
+        CU(p->W.reserve((size_t)nwords));
+        CU(p->blockhits.reserve((size_t)nblocks * kDetect));
+        CU(p->counts.reserve((size_t)nblocks));
+        CU(p->hits.reserve((size_t)max_frames + 1));
     }
-    const uint8_t* hist = p->hist[p->cur];
-    pack_kernel<<<(nwords + 255) / 256, 256, 0, st>>>(hist, d_bits, size, p->W, nwords);
-    detect_kernel<<<nblocks, kDetect, 0, st>>>(p->W, size, p->blockhits, p->counts);
-    collect_kernel<<<1, 1024, 0, st>>>(p->blockhits, p->counts, nblocks, max_frames, p->hits, p->st, d_nframes);
-    if (max_frames) frames_kernel<<<max_frames, 416, 0, st>>>(p->W, p->hits, p->st, reinterpret_cast<uint32_t*>(d_frames));
-    carry_kernel<<<(kCarry + 255) / 256, 256, 0, st>>>(hist, d_bits, size, p->hist[p->cur ^ 1]);
+    const uint8_t* hist = p->hist[p->cur].p;
+    pack_kernel<<<(nwords + 255) / 256, 256, 0, st>>>(hist, d_bits, size, p->W.p, nwords);
+    detect_kernel<<<nblocks, kDetect, 0, st>>>(p->W.p, size, p->blockhits.p, p->counts.p);
+    collect_kernel<<<1, 1024, 0, st>>>(p->blockhits.p, p->counts.p, nblocks, max_frames, p->hits.p, p->st.p, d_nframes);
+    if (max_frames) frames_kernel<<<max_frames, 416, 0, st>>>(p->W.p, p->hits.p, p->st.p, reinterpret_cast<uint32_t*>(d_frames));
+    carry_kernel<<<(kCarry + 255) / 256, 256, 0, st>>>(hist, d_bits, size, p->hist[p->cur ^ 1].p);
     CU(cudaGetLastError());
     p->cur ^= 1;
     return 0;
 }
 
 int dvbs2fec_dvbs_deframer_work(dvbs2fec_dvbs_deframer* p, const uint8_t* bits, int size, uint8_t* frames, int max_frames) {
-    if (!p || size < 0 || max_frames < 0 || (size && !bits) || (max_frames && !frames)) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || size < 0 || max_frames < 0 || (size && !bits) || (max_frames && !frames)) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!size) return 0;
     CU(cudaSetDevice(p->device));
     // a frame cannot follow another in less than one bit; the caller's limit bounds what is written
-    CU(reserve(p->in, p->in_cap, (size_t)size));
-    CU(reserve(p->out, p->out_cap, (size_t)max_frames * 408 + 1));
-    CU(cudaMemcpyAsync(p->in, bits, (size_t)size, cudaMemcpyHostToDevice, p->stream));
-    int rc = dvbs2fec_dvbs_deframer_work_device(p, p->in, size, reinterpret_cast<uint8_t*>(p->out), max_frames, nullptr, p->stream);
+    CU(p->in.reserve((size_t)size));
+    CU(p->out.reserve((size_t)max_frames * 408 + 1));
+    CU(cudaMemcpyAsync(p->in.p, bits, (size_t)size, cudaMemcpyHostToDevice, p->stream));
+    int rc = dvbs2fec_dvbs_deframer_work_device(p, p->in.p, size, reinterpret_cast<uint8_t*>(p->out.p), max_frames, nullptr, p->stream);
     if (rc) return rc;
     DeframerState s;
-    CU(cudaMemcpyAsync(&s, p->st, sizeof s, cudaMemcpyDeviceToHost, p->stream));
+    CU(cudaMemcpyAsync(&s, p->st.p, sizeof s, cudaMemcpyDeviceToHost, p->stream));
     CU(cudaStreamSynchronize(p->stream));
     if (s.written) {
-        CU(cudaMemcpyAsync(frames, p->out, (size_t)s.written * 1632, cudaMemcpyDeviceToHost, p->stream));
+        CU(cudaMemcpyAsync(frames, p->out.p, (size_t)s.written * 1632, cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
     }
     return s.written;
 }
 
 int dvbs2fec_dvbs_deframer_stats(dvbs2fec_dvbs_deframer* p, int* errors_nor, int* errors_inv, int* found) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     DeframerState s;
-    CU(cudaMemcpy(&s, p->st, sizeof s, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&s, p->st.p, sizeof s, cudaMemcpyDeviceToHost));
     if (errors_nor) *errors_nor = s.errors_nor;
     if (errors_inv) *errors_inv = s.errors_inv;
     if (found) *found = s.nframes;

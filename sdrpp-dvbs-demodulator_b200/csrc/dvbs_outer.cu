@@ -24,17 +24,15 @@
 // tests/test_dvbs_oracle.py pins to the compiled reference).
 #include "../../include/dvbs2fec.h"
 
-#include <cstdio>
 #include <cstring>
 #include <memory>
 #include <vector>
 
 #include <cuda_runtime.h>
 
-namespace s2 {
-int api_fail(int code, const char* msg);
-}
-using s2::api_fail;
+#include "abi_util.h"
+
+using namespace s2;
 
 namespace {
 
@@ -314,37 +312,6 @@ __global__ void commit_kernel(OuterState* st) {
     st->prbs_off = st->prbs_next;
 }
 
-template <typename T>
-struct DevBuf {
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-
-int failf(int code, const char* what, cudaError_t e) {
-    char buf[300];
-    snprintf(buf, sizeof buf, "%s: %s", what, cudaGetErrorString(e));
-    return api_fail(code, buf);
-}
-#define CU(call)                                                     \
-    do {                                                             \
-        cudaError_t e_ = (call);                                     \
-        if (e_ != cudaSuccess) return failf(DVBS2FEC_ECUDA, #call, e_); \
-    } while (0)
-
 }  // namespace
 
 struct dvbs2fec_dvbs_outer {
@@ -355,28 +322,34 @@ struct dvbs2fec_dvbs_outer {
     DevBuf<uint8_t> prbs, D, dec, ok, in, out;
     DevBuf<int> src, eff;
     DevBuf<int32_t> err;
+    ~dvbs2fec_dvbs_outer() {
+        cudaSetDevice(device);
+        if (stream) {
+            cudaStreamSynchronize(stream);
+            cudaStreamDestroy(stream);
+        }
+    }
 };
 
 extern "C" {
 
 int dvbs2fec_dvbs_outer_reset(dvbs2fec_dvbs_outer* p) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     OuterState s;
     memset(&s, 0, sizeof s);            // FIFOs and obuffer zeroed (dvbs_interleaving.h:30-40, dvbs_reedsolomon.h:20-22), reg = 0
     s.prbs_off = -1;
     s.prbs_next = -1;
-    CU(cudaMemcpy(p->st.p, &s, sizeof s, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->st.p, &s, sizeof s));
     return 0;
 }
 
 int dvbs2fec_dvbs_outer_create(int device, dvbs2fec_dvbs_outer** out) {
-    if (!out) return api_fail(DVBS2FEC_EINVAL, "out is NULL");
+    if (!out) return fail(DVBS2FEC_EINVAL, "out is NULL");
     *out = nullptr;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return api_fail(DVBS2FEC_ENODEV, "no CUDA device");
-    if (device < 0 || device >= ndev) return api_fail(DVBS2FEC_EINVAL, "device out of range");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(DVBS2FEC_ENODEV, "no CUDA device");
+    if (device < 0 || device >= ndev) return fail(DVBS2FEC_EINVAL, "device out of range");
     std::unique_ptr<dvbs2fec_dvbs_outer> p(new dvbs2fec_dvbs_outer());
     p->device = device;
     CU(cudaSetDevice(device));
@@ -395,8 +368,7 @@ int dvbs2fec_dvbs_outer_create(int device, dvbs2fec_dvbs_outer** out) {
         g.exp[i] = (uint8_t)e;
         if (i < 256) g.log[e] = (uint8_t)i;
     }
-    CU(cudaMemcpy(p->gf.p, &g, sizeof g, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->gf.p, &g, sizeof g));
     // one period of the dispersal generator from its load value 0xa9 (dvbs_scrambling.h:16-28): entry o = the byte
     // prbs(8) returns after o clocks
     std::vector<uint8_t> bits(kPeriod + 8), tab(kPeriod + 1);
@@ -411,31 +383,20 @@ int dvbs2fec_dvbs_outer_create(int device, dvbs2fec_dvbs_outer** out) {
         for (int k = 0; k < 8; ++k) b = (b << 1) | bits[(size_t)(o + k)];
         tab[(size_t)o] = (uint8_t)b;
     }
-    CU(cudaMemcpy(p->prbs.p, tab.data(), kPeriod, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->prbs.p, tab.data(), kPeriod));
     int rc = dvbs2fec_dvbs_outer_reset(p.get());
     if (rc) return rc;
     *out = p.release();
     return 0;
 }
 
-void dvbs2fec_dvbs_outer_destroy(dvbs2fec_dvbs_outer* p) {
-    if (!p) return;
-    cudaSetDevice(p->device);
-    if (p->stream) {
-        cudaStreamSynchronize(p->stream);
-        cudaStreamDestroy(p->stream);
-    }
-    p->st.release(); p->gf.release(); p->prbs.release(); p->D.release(); p->dec.release(); p->ok.release();
-    p->in.release(); p->out.release(); p->src.release(); p->eff.release(); p->err.release();
-    delete p;
-}
+void dvbs2fec_dvbs_outer_destroy(dvbs2fec_dvbs_outer* p) { delete p; }
 
 int dvbs2fec_dvbs_outer_process_device(dvbs2fec_dvbs_outer* p, int nframes, int frame_stride, const uint8_t* d_frames, uint8_t* d_out,
                                        int32_t* d_errors, void* stream) {
-    if (!p || nframes < 0 || frame_stride < 1 || (nframes && (!d_frames || !d_out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || nframes < 0 || frame_stride < 1 || (nframes && (!d_frames || !d_out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!nframes) return 0;
-    if (nframes > (1 << 20)) return api_fail(DVBS2FEC_EINVAL, "more than 2^20 frames in one call");
+    if (nframes > (1 << 20)) return fail(DVBS2FEC_EINVAL, "more than 2^20 frames in one call");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
     const int np = nframes * 8;
@@ -458,7 +419,7 @@ int dvbs2fec_dvbs_outer_process_device(dvbs2fec_dvbs_outer* p, int nframes, int 
 }
 
 int dvbs2fec_dvbs_outer_process(dvbs2fec_dvbs_outer* p, int nframes, int frame_stride, const uint8_t* frames, uint8_t* out, int32_t* errors) {
-    if (!p || nframes < 0 || frame_stride < 1 || (nframes && (!frames || !out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || nframes < 0 || frame_stride < 1 || (nframes && (!frames || !out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!nframes) return 0;
     CU(cudaSetDevice(p->device));
     const size_t in_bytes = (size_t)(nframes - 1) * frame_stride + kFrame, np = (size_t)nframes * 8;

@@ -38,10 +38,10 @@
 
 #include <cuda_runtime.h>
 
-namespace s2 {
-int api_fail(int code, const char* msg);
-}
-using s2::api_fail;
+#include "abi_util.h"
+
+using s2::DevBuf;
+using s2::fail;
 
 namespace {
 
@@ -452,28 +452,6 @@ __global__ void __launch_bounds__(256) sts_kernel(const float* __restrict__ syms
     }
 }
 
-int failf(int code, const char* what, cudaError_t e) {
-    char buf[300];
-    snprintf(buf, sizeof buf, "%s: %s", what, cudaGetErrorString(e));
-    return api_fail(code, buf);
-}
-#define CU(call)                                                     \
-    do {                                                             \
-        cudaError_t e_ = (call);                                     \
-        if (e_ != cudaSuccess) return failf(DVBS2FEC_ECUDA, #call, e_); \
-    } while (0)
-
-template <typename T>
-cudaError_t reserve(T*& p, size_t& cap, size_t n) {
-    if (n <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-    cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-    if (e == cudaSuccess) cap = n;
-    return e;
-}
-
 void build_patterns(Pattern* P) {
     memset(P, 0, sizeof(Pattern) * kPatterns);
     auto fill = [](Pattern& p, int pin, std::initializer_list<std::pair<int, int>> slots) {      // (owner, erasure)
@@ -527,7 +505,7 @@ struct dvbs2fec_dvbs_viterbi {
     int dec_ber_start[5], dec_main_start[5], enc_state[5] = {0, 0, 0, 0, 0}, stale_bit = 0;
     DepuncState dp[5];
     int stale23[2] = {128, 128};
-    int8_t* d_last_search = nullptr;      // first 2048 soft bits of the last block the search ran on
+    DevBuf<int8_t> d_last_search;      // first 2048 soft bits of the last block the search ran on
     int have_last_search = 0;
     int search_batch = 1;
     int max_sync_blocks = kMaxSyncBlocks;      // DVBS2FEC_VIT_MAX_BATCH overrides (tests: batches cut inside a call)
@@ -536,27 +514,32 @@ struct dvbs2fec_dvbs_viterbi {
     SearchLayout lay;
     int search_img_stride = 0, search_steps = 0, search_out = 0;
     // device pools
-    int8_t* d_in = nullptr; size_t in_cap = 0;
-    uint8_t* d_out = nullptr; size_t out_cap = 0;
-    uint8_t* images = nullptr; size_t img_cap = 0;
-    uint2* decpool = nullptr; size_t dec_cap = 0;
-    uint8_t* decoded = nullptr; size_t decd_cap = 0;
-    VTask* tasks = nullptr; size_t task_cap = 0;
-    VResult* res = nullptr; size_t res_cap = 0;
-    ContDesc* desc = nullptr; size_t desc_cap = 0;
-    ContRec* rec = nullptr; size_t rec_cap = 0;
-    EmitDesc* emit = nullptr; size_t emit_cap = 0;
-    int* flag = nullptr;
+    DevBuf<int8_t> d_in;
+    DevBuf<uint8_t> d_out, images, decoded;
+    DevBuf<uint2> decpool;
+    DevBuf<VTask> tasks;
+    DevBuf<VResult> res;
+    DevBuf<ContDesc> desc;
+    DevBuf<ContRec> rec;
+    DevBuf<EmitDesc> emit;
+    DevBuf<int> flag;
     std::vector<VTask> h_tasks;
     std::vector<VResult> h_res;
     std::vector<ContDesc> h_desc;
     std::vector<ContRec> h_rec;
     std::vector<EmitDesc> h_emit;
     // DVBSymToSoftBlock
-    int8_t* sts_carry[2] = {nullptr, nullptr};
+    DevBuf<int8_t> sts_carry[2];
     int sts_cur = 0, sts_fill = 0;
-    float* d_syms = nullptr; size_t syms_cap = 0;
-    int8_t* d_soft = nullptr; size_t soft_cap = 0;
+    DevBuf<float> d_syms;
+    DevBuf<int8_t> d_soft;
+    ~dvbs2fec_dvbs_viterbi() {
+        cudaSetDevice(device);
+        if (stream) {
+            cudaStreamSynchronize(stream);
+            cudaStreamDestroy(stream);
+        }
+    }
 };
 
 namespace {
@@ -566,27 +549,27 @@ using Vit = dvbs2fec_dvbs_viterbi;
 // guess, decode, check (repeat what started wrong), BER; results to the host
 int run_tasks(Vit* v, int ntasks) {
     cudaStream_t st = v->stream;
-    CU(reserve(v->tasks, v->task_cap, (size_t)ntasks));
-    CU(reserve(v->res, v->res_cap, (size_t)ntasks));
-    CU(cudaMemcpyAsync(v->tasks, v->h_tasks.data(), sizeof(VTask) * ntasks, cudaMemcpyHostToDevice, st));
+    CU(v->tasks.reserve((size_t)ntasks));
+    CU(v->res.reserve((size_t)ntasks));
+    CU(cudaMemcpyAsync(v->tasks.p, v->h_tasks.data(), sizeof(VTask) * ntasks, cudaMemcpyHostToDevice, st));
     const int grid = (ntasks + 3) / 4;
-    acs_kernel<<<grid, 128, 0, st>>>(v->tasks, v->res, ntasks, 0, v->images, v->decpool, v->decoded, v->flag + 1);
-    acs_kernel<<<grid, 128, 0, st>>>(v->tasks, v->res, ntasks, 1, v->images, v->decpool, v->decoded, v->flag + 1);
+    acs_kernel<<<grid, 128, 0, st>>>(v->tasks.p, v->res.p, ntasks, 0, v->images.p, v->decpool.p, v->decoded.p, v->flag.p + 1);
+    acs_kernel<<<grid, 128, 0, st>>>(v->tasks.p, v->res.p, ntasks, 1, v->images.p, v->decpool.p, v->decoded.p, v->flag.p + 1);
     v->h_res.resize(ntasks);
     v->n_tasks += ntasks;
     for (int pass = 0;; ++pass) {
         int flag = 0;
-        CU(cudaMemsetAsync(v->flag, 0, sizeof(int), st));
-        mark_kernel<<<(ntasks + 255) / 256, 256, 0, st>>>(v->tasks, v->res, ntasks, v->flag);
-        ber_kernel<<<grid, 128, 0, st>>>(v->tasks, v->res, ntasks, v->images, v->decoded);
-        CU(cudaMemcpyAsync(&flag, v->flag, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(v->h_res.data(), v->res, sizeof(VResult) * ntasks, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemsetAsync(v->flag.p, 0, sizeof(int), st));
+        mark_kernel<<<(ntasks + 255) / 256, 256, 0, st>>>(v->tasks.p, v->res.p, ntasks, v->flag.p);
+        ber_kernel<<<grid, 128, 0, st>>>(v->tasks.p, v->res.p, ntasks, v->images.p, v->decoded.p);
+        CU(cudaMemcpyAsync(&flag, v->flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(v->h_res.data(), v->res.p, sizeof(VResult) * ntasks, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         v->n_passes++;
         if (!flag) break;
         v->n_repeated += flag;
-        if (pass > ntasks) return api_fail(DVBS2FEC_ECUDA, "viterbi: start-state check does not settle");
-        acs_kernel<<<grid, 128, 0, st>>>(v->tasks, v->res, ntasks, 2, v->images, v->decpool, v->decoded, v->flag + 1);
+        if (pass > ntasks) return fail(DVBS2FEC_ECUDA, "viterbi: start-state check does not settle");
+        acs_kernel<<<grid, 128, 0, st>>>(v->tasks.p, v->res.p, ntasks, 2, v->images.p, v->decpool.p, v->decoded.p, v->flag.p + 1);
     }
     CU(cudaGetLastError());
     return 0;
@@ -597,10 +580,10 @@ int run_tasks(Vit* v, int ntasks) {
 int run_search(Vit* v, const int8_t* d_in, int n, int* consumed) {
     cudaStream_t st = v->stream;
     const SearchLayout& L = v->lay;
-    CU(reserve(v->images, v->img_cap, (size_t)n * v->search_img_stride));
-    CU(reserve(v->decpool, v->dec_cap, (size_t)n * v->search_steps));
-    CU(reserve(v->decoded, v->decd_cap, (size_t)n * v->search_out));
-    search_image_kernel<<<n, 256, 0, st>>>(d_in, v->d_last_search, v->have_last_search, v->images, (uint32_t)v->search_img_stride);
+    CU(v->images.reserve((size_t)n * v->search_img_stride));
+    CU(v->decpool.reserve((size_t)n * v->search_steps));
+    CU(v->decoded.reserve((size_t)n * v->search_out));
+    search_image_kernel<<<n, 256, 0, st>>>(d_in, v->d_last_search.p, v->have_last_search, v->images.p, (uint32_t)v->search_img_stride);
     v->h_tasks.resize((size_t)n * kSearchTasks);
     int last_of_rate[5];      // task index of the latest candidate of each rate
     for (int r = 0; r < 5; ++r) last_of_rate[r] = -1;
@@ -658,7 +641,7 @@ int run_search(Vit* v, const int8_t* d_in, int n, int* consumed) {
             }
     }
     // b blocks went through the search; the last of them is what ber_depunc_buffer now derives from
-    CU(cudaMemcpyAsync(v->d_last_search, d_in + (size_t)(b - 1) * kBuf, kTest, cudaMemcpyDeviceToDevice, st));
+    CU(cudaMemcpyAsync(v->d_last_search.p, d_in + (size_t)(b - 1) * kBuf, kTest, cudaMemcpyDeviceToDevice, st));
     v->have_last_search = 1;
     *consumed = locked ? b - 1 : b;
     return 0;
@@ -668,9 +651,9 @@ int run_search(Vit* v, const int8_t* d_in, int n, int* consumed) {
 int run_sync(Vit* v, const int8_t* d_in, int n, uint8_t* d_out, long long* oidx, int* accepted) {
     cudaStream_t st = v->stream;
     const int r = v->rate, fs = kFsMain[r], nsteps = fs + 6, nread = 2 * nsteps, stride = pad16(nread), ostride = pad16(fs);
-    CU(reserve(v->images, v->img_cap, (size_t)n * stride));
-    CU(reserve(v->decpool, v->dec_cap, (size_t)n * nsteps));
-    CU(reserve(v->decoded, v->decd_cap, (size_t)n * ostride));
+    CU(v->images.reserve((size_t)n * stride));
+    CU(v->decpool.reserve((size_t)n * nsteps));
+    CU(v->decoded.reserve((size_t)n * ostride));
     const bool cont = r == R23 || r == R56;
     std::vector<DepuncState> after(n);
     std::vector<int> szs(n, kBuf);
@@ -694,13 +677,13 @@ int run_sync(Vit* v, const int8_t* d_in, int n, uint8_t* d_out, long long* oidx,
             if (D.oo % 2 == 1) { szs[k] = D.oo - 1; d.got_extra = 1; }
             after[k] = d;
         }
-        CU(reserve(v->desc, v->desc_cap, (size_t)n));
-        CU(reserve(v->rec, v->rec_cap, (size_t)n));
-        CU(cudaMemcpyAsync(v->desc, v->h_desc.data(), sizeof(ContDesc) * n, cudaMemcpyHostToDevice, st));
+        CU(v->desc.reserve((size_t)n));
+        CU(v->rec.reserve((size_t)n));
+        CU(cudaMemcpyAsync(v->desc.p, v->h_desc.data(), sizeof(ContDesc) * n, cudaMemcpyHostToDevice, st));
     } else if (r == R34) std::fill(szs.begin(), szs.end(), kBuf / 2 * 3);
     else if (r == R78) std::fill(szs.begin(), szs.end(), kBuf / 8 * 14);
-    sync_image_kernel<<<dim3(n, 8), 256, 0, st>>>(d_in, r, v->phase, v->shift, nread, cont ? v->desc : nullptr, cont ? v->rec : nullptr, v->dp[r].buf,
-                                                   v->stale23[0], v->stale23[1], v->images, (uint32_t)stride);
+    sync_image_kernel<<<dim3(n, 8), 256, 0, st>>>(d_in, r, v->phase, v->shift, nread, cont ? v->desc.p : nullptr, cont ? v->rec.p : nullptr, v->dp[r].buf,
+                                                   v->stale23[0], v->stale23[1], v->images.p, (uint32_t)stride);
     v->h_tasks.resize(n);
     for (int k = 0; k < n; ++k) {
         VTask& t = v->h_tasks[k];
@@ -723,7 +706,7 @@ int run_sync(Vit* v, const int8_t* d_in, int n, uint8_t* d_out, long long* oidx,
     if (rc) return rc;
     if (cont) {
         v->h_rec.resize(n);
-        CU(cudaMemcpyAsync(v->h_rec.data(), v->rec, sizeof(ContRec) * n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(v->h_rec.data(), v->rec.p, sizeof(ContRec) * n, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
     }
     v->h_emit.clear();
@@ -751,9 +734,9 @@ int run_sync(Vit* v, const int8_t* d_in, int n, uint8_t* d_out, long long* oidx,
     }
     *accepted = k;
     if (k) {
-        CU(reserve(v->emit, v->emit_cap, (size_t)k));
-        CU(cudaMemcpyAsync(v->emit, v->h_emit.data(), sizeof(EmitDesc) * k, cudaMemcpyHostToDevice, st));
-        emit_kernel<<<k, 256, 0, st>>>(v->emit, v->decoded, d_out);
+        CU(v->emit.reserve((size_t)k));
+        CU(cudaMemcpyAsync(v->emit.p, v->h_emit.data(), sizeof(EmitDesc) * k, cudaMemcpyHostToDevice, st));
+        emit_kernel<<<k, 256, 0, st>>>(v->emit.p, v->decoded.p, d_out);
         CU(cudaStreamSynchronize(st));      // h_emit is reused by the next batch
     }
     CU(cudaGetLastError());
@@ -765,7 +748,7 @@ int run_sync(Vit* v, const int8_t* d_in, int n, uint8_t* d_out, long long* oidx,
 extern "C" {
 
 int dvbs2fec_dvbs_viterbi_reset(dvbs2fec_dvbs_viterbi* v) {
-    if (!v) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!v) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(v->device));
     v->state = v->rate = v->phase = v->shift = v->invalid = 0;
     v->ber = 10;
@@ -785,11 +768,11 @@ int dvbs2fec_dvbs_viterbi_reset(dvbs2fec_dvbs_viterbi* v) {
 }
 
 int dvbs2fec_dvbs_viterbi_create(int device, float ber_threshold, int max_outsync, dvbs2fec_dvbs_viterbi** out) {
-    if (!out) return api_fail(DVBS2FEC_EINVAL, "out is NULL");
+    if (!out) return fail(DVBS2FEC_EINVAL, "out is NULL");
     *out = nullptr;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return api_fail(DVBS2FEC_ENODEV, "no CUDA device");
-    if (device < 0 || device >= ndev) return api_fail(DVBS2FEC_EINVAL, "device out of range");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(DVBS2FEC_ENODEV, "no CUDA device");
+    if (device < 0 || device >= ndev) return fail(DVBS2FEC_EINVAL, "device out of range");
     std::unique_ptr<Vit> v(new Vit());
     v->device = device;
     v->thr = ber_threshold;
@@ -817,34 +800,23 @@ int dvbs2fec_dvbs_viterbi_create(int device, float ber_threshold, int max_outsyn
     v->search_steps = 2 * steps;
     v->search_out = 2 * outb;
     CU(cudaMemcpyToSymbol(cSearch, &L, sizeof L));
-    CU(cudaMalloc(&v->d_last_search, kTest));
-    CU(cudaMalloc(&v->flag, 2 * sizeof(int)));
-    CU(cudaMemset(v->flag, 0, 2 * sizeof(int)));      // [0] tasks that started wrong in this pass, [1] tracebacks that fell back to the walk
+    CU(v->d_last_search.reserve(kTest));
+    CU(v->flag.reserve(2));
+    CU(cudaMemset(v->flag.p, 0, 2 * sizeof(int)));      // [0] tasks that started wrong in this pass, [1] tracebacks that fell back to the walk
     CU(cudaDeviceSynchronize());
-    CU(cudaMalloc(&v->sts_carry[0], kBuf));
-    CU(cudaMalloc(&v->sts_carry[1], kBuf));
+    CU(v->sts_carry[0].reserve(kBuf));
+    CU(v->sts_carry[1].reserve(kBuf));
     int rc = dvbs2fec_dvbs_viterbi_reset(v.get());
     if (rc) return rc;
     *out = v.release();
     return 0;
 }
 
-void dvbs2fec_dvbs_viterbi_destroy(dvbs2fec_dvbs_viterbi* v) {
-    if (!v) return;
-    cudaSetDevice(v->device);
-    if (v->stream) {
-        cudaStreamSynchronize(v->stream);
-        cudaStreamDestroy(v->stream);
-    }
-    cudaFree(v->d_last_search); cudaFree(v->flag); cudaFree(v->sts_carry[0]); cudaFree(v->sts_carry[1]);
-    cudaFree(v->d_in); cudaFree(v->d_out); cudaFree(v->images); cudaFree(v->decpool); cudaFree(v->decoded); cudaFree(v->tasks);
-    cudaFree(v->res); cudaFree(v->desc); cudaFree(v->rec); cudaFree(v->emit); cudaFree(v->d_syms); cudaFree(v->d_soft);
-    delete v;
-}
+void dvbs2fec_dvbs_viterbi_destroy(dvbs2fec_dvbs_viterbi* v) { delete v; }
 
 int dvbs2fec_dvbs_viterbi_process_device(dvbs2fec_dvbs_viterbi* v, int count, const int8_t* d_in, uint8_t* d_out) {
-    if (!v || count < 0 || (count && (!d_in || !d_out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
-    if (count % kBuf) return api_fail(DVBS2FEC_EINVAL, "count must be a multiple of 8192 soft bits (VIT_BUF_SIZE)");
+    if (!v || count < 0 || (count && (!d_in || !d_out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (count % kBuf) return fail(DVBS2FEC_EINVAL, "count must be a multiple of 8192 soft bits (VIT_BUF_SIZE)");
     CU(cudaSetDevice(v->device));
     const int nb = count / kBuf;
     int pos = 0;
@@ -866,29 +838,29 @@ int dvbs2fec_dvbs_viterbi_process_device(dvbs2fec_dvbs_viterbi* v, int count, co
             pos += accepted;
         }
     }
-    if (oidx > 0x7FFFFFFF) return api_fail(DVBS2FEC_EINVAL, "more than 2^31 - 1 output bits in one call");
+    if (oidx > 0x7FFFFFFF) return fail(DVBS2FEC_EINVAL, "more than 2^31 - 1 output bits in one call");
     return (int)oidx;
 }
 
 int dvbs2fec_dvbs_viterbi_process(dvbs2fec_dvbs_viterbi* v, int count, const int8_t* in, uint8_t* out) {
-    if (!v || count < 0 || (count && (!in || !out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
-    if (count % kBuf) return api_fail(DVBS2FEC_EINVAL, "count must be a multiple of 8192 soft bits (VIT_BUF_SIZE)");
+    if (!v || count < 0 || (count && (!in || !out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (count % kBuf) return fail(DVBS2FEC_EINVAL, "count must be a multiple of 8192 soft bits (VIT_BUF_SIZE)");
     if (!count) return 0;
     CU(cudaSetDevice(v->device));
-    CU(reserve(v->d_in, v->in_cap, (size_t)count));
-    CU(reserve(v->d_out, v->out_cap, (size_t)count));
-    CU(cudaMemcpyAsync(v->d_in, in, (size_t)count, cudaMemcpyHostToDevice, v->stream));
+    CU(v->d_in.reserve((size_t)count));
+    CU(v->d_out.reserve((size_t)count));
+    CU(cudaMemcpyAsync(v->d_in.p, in, (size_t)count, cudaMemcpyHostToDevice, v->stream));
     // the bytes the reference leaves unwritten (rate 5/6) keep what the caller's buffer holds
-    CU(cudaMemcpyAsync(v->d_out, out, (size_t)count, cudaMemcpyHostToDevice, v->stream));
-    const int n = dvbs2fec_dvbs_viterbi_process_device(v, count, v->d_in, v->d_out);
+    CU(cudaMemcpyAsync(v->d_out.p, out, (size_t)count, cudaMemcpyHostToDevice, v->stream));
+    const int n = dvbs2fec_dvbs_viterbi_process_device(v, count, v->d_in.p, v->d_out.p);
     if (n <= 0) return n;
-    CU(cudaMemcpyAsync(out, v->d_out, (size_t)n, cudaMemcpyDeviceToHost, v->stream));
+    CU(cudaMemcpyAsync(out, v->d_out.p, (size_t)n, cudaMemcpyDeviceToHost, v->stream));
     CU(cudaStreamSynchronize(v->stream));
     return n;
 }
 
 int dvbs2fec_dvbs_viterbi_stats(dvbs2fec_dvbs_viterbi* v, float* ber, int* state, int* rate, int* phase, int* shift, int* invalid) {
-    if (!v) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!v) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     float b = v->ber;
     if (v->state != 1) {      // Viterbi_DVBS::ber (:282-313): the best candidate of the last search
         b = 10;
@@ -907,11 +879,11 @@ int dvbs2fec_dvbs_viterbi_stats(dvbs2fec_dvbs_viterbi* v, float* ber, int* state
 }
 
 int dvbs2fec_dvbs_viterbi_counters(dvbs2fec_dvbs_viterbi* v, long long* tasks, long long* repeated, long long* passes, long long* walks) {
-    if (!v) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!v) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     if (walks) {
         int w = 0;
         CU(cudaSetDevice(v->device));
-        CU(cudaMemcpy(&w, v->flag + 1, sizeof(int), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(&w, v->flag.p + 1, sizeof(int), cudaMemcpyDeviceToHost));
         *walks = w;
     }
     if (tasks) *tasks = v->n_tasks;
@@ -921,12 +893,12 @@ int dvbs2fec_dvbs_viterbi_counters(dvbs2fec_dvbs_viterbi* v, long long* tasks, l
 }
 
 int dvbs2fec_dvbs_sts_process_device(dvbs2fec_dvbs_viterbi* v, int count, const float* d_syms, int8_t* d_out) {
-    if (!v || count < 0 || (count && (!d_syms || !d_out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!v || count < 0 || (count && (!d_syms || !d_out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!count) return 0;
     CU(cudaSetDevice(v->device));
     const int total = v->sts_fill + 2 * count, nout = total / kBuf * kBuf;
-    sts_kernel<<<std::min((total + 255) / 256, 1184), 256, 0, v->stream>>>(d_syms, 2 * count, v->sts_carry[v->sts_cur], v->sts_fill, nout, d_out,
-                                                                            v->sts_carry[v->sts_cur ^ 1]);
+    sts_kernel<<<std::min((total + 255) / 256, 1184), 256, 0, v->stream>>>(d_syms, 2 * count, v->sts_carry[v->sts_cur].p, v->sts_fill, nout, d_out,
+                                                                            v->sts_carry[v->sts_cur ^ 1].p);
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(v->stream));
     v->sts_cur ^= 1;
@@ -935,15 +907,15 @@ int dvbs2fec_dvbs_sts_process_device(dvbs2fec_dvbs_viterbi* v, int count, const 
 }
 
 int dvbs2fec_dvbs_sts_process(dvbs2fec_dvbs_viterbi* v, int count, const float* syms, int8_t* out) {
-    if (!v || count < 0 || (count && (!syms || !out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!v || count < 0 || (count && (!syms || !out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!count) return 0;
     CU(cudaSetDevice(v->device));
-    CU(reserve(v->d_syms, v->syms_cap, (size_t)2 * count));
-    CU(reserve(v->d_soft, v->soft_cap, (size_t)2 * count + kBuf));
-    CU(cudaMemcpyAsync(v->d_syms, syms, sizeof(float) * 2 * count, cudaMemcpyHostToDevice, v->stream));
-    const int n = dvbs2fec_dvbs_sts_process_device(v, count, v->d_syms, v->d_soft);
+    CU(v->d_syms.reserve((size_t)2 * count));
+    CU(v->d_soft.reserve((size_t)2 * count + kBuf));
+    CU(cudaMemcpyAsync(v->d_syms.p, syms, sizeof(float) * 2 * count, cudaMemcpyHostToDevice, v->stream));
+    const int n = dvbs2fec_dvbs_sts_process_device(v, count, v->d_syms.p, v->d_soft.p);
     if (n <= 0) return n;
-    CU(cudaMemcpyAsync(out, v->d_soft, (size_t)n, cudaMemcpyDeviceToHost, v->stream));
+    CU(cudaMemcpyAsync(out, v->d_soft.p, (size_t)n, cudaMemcpyDeviceToHost, v->stream));
     CU(cudaStreamSynchronize(v->stream));
     return n;
 }

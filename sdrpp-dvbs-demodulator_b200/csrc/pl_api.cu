@@ -4,7 +4,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <memory>
@@ -12,58 +11,13 @@
 
 #include <cuda_runtime.h>
 
+#include "abi_util.h"
 #include "host_tables.h"
 #include "pl_sync.cuh"
 
-namespace s2 {
-int api_fail(int code, const char* msg);
-}
 using namespace s2;
 
 namespace {
-int failf(int code, const char* fmt, const char* a, const char* file, int line) {
-    char buf[400];
-    snprintf(buf, sizeof buf, fmt, a, file, line);
-    return api_fail(code, buf);
-}
-#define CU(call)                                                                                                 \
-    do {                                                                                                         \
-        cudaError_t e_ = (call);                                                                                 \
-        if (e_ != cudaSuccess) return failf(DVBS2FEC_ECUDA, #call ": %s (%s:%d)", cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-
-template <typename T>
-struct Buf {
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-    // grow, keeping the first `keep` elements
-    cudaError_t grow(size_t n, size_t keep, cudaStream_t st) {
-        if (n <= cap) return cudaSuccess;
-        T* q = nullptr;
-        cudaError_t e = cudaMalloc(&q, n * sizeof(T));
-        if (e != cudaSuccess) return e;
-        if (p && keep) e = cudaMemcpyAsync(q, p, keep * sizeof(T), cudaMemcpyDeviceToDevice, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        if (p) cudaFree(p);
-        p = q;
-        cap = n;
-        return e;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
 
 // s2_sof / s2_plscodes (dvbs2/s2_defs.h:16-87) with the reference's float expressions
 void build_tables(PlTables& t) {
@@ -115,35 +69,42 @@ struct dvbs2fec_plsync {
     int cur = 0;               // work buffer holding the carried symbols
     int pend_ub = 0;           // upper bound of the symbols carried over (exact after a synchronous call)
     bool pend_exact = true;
-    Buf<float2> work[2], out, frames_in, hdr_out;
-    Buf<float> metric, fed_out;
-    Buf<int> starts;
-    Buf<PlSyncState> st;
-    Buf<PlHdrState> hst;
-    Buf<PlHdrResult> hres;
-    Buf<PlTables> tab;
-    Buf<uint8_t> rn;           // the coarse FED's PL scrambling sequence, of Gold code rn_codenum
+    DevBuf<float2> work[2], out, frames_in, hdr_out;
+    DevBuf<float> metric, fed_out;
+    DevBuf<int> starts;
+    DevBuf<PlSyncState> st;
+    DevBuf<PlHdrState> hst;
+    DevBuf<PlHdrResult> hres;
+    DevBuf<PlTables> tab;
+    DevBuf<uint8_t> rn;           // the coarse FED's PL scrambling sequence, of Gold code rn_codenum
     int rn_codenum = -2;
     PlSyncState h_st{};
     // S2PLLBlock (K8)
-    Buf<PllState> pst;
-    Buf<float> perr, pll_state;
-    Buf<float2> pll_in, pll_out;
-    Buf<uint8_t> pll_rn;       // the loop's own sequence: a FED call with another code must not change what a queued loop reads
-    Buf<uint8_t> pll_jobs;
+    DevBuf<PllState> pst;
+    DevBuf<float> perr, pll_state;
+    DevBuf<float2> pll_in, pll_out;
+    DevBuf<uint8_t> pll_rn;       // the loop's own sequence: a FED call with another code must not change what a queued loop reads
+    DevBuf<uint8_t> pll_jobs;
     PllArgs pll{};            // configuration part; buffers are filled in per call
     bool pll_ready = false;
     int pll_sequential = 0;      // 0: pipelined speculative kernel, 1: sequential walk, 2: one-warp speculative kernel
+    ~dvbs2fec_plsync() {
+        cudaSetDevice(device);
+        if (stream) {
+            cudaStreamSynchronize(stream);
+            cudaStreamDestroy(stream);
+        }
+    }
 };
 
 extern "C" {
 
 int dvbs2fec_plsync_create(int device, dvbs2fec_plsync** out) {
-    if (!out) return api_fail(DVBS2FEC_EINVAL, "out is NULL");
+    if (!out) return fail(DVBS2FEC_EINVAL, "out is NULL");
     *out = nullptr;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return api_fail(DVBS2FEC_ENODEV, "no CUDA device");
-    if (device < 0 || device >= ndev) return api_fail(DVBS2FEC_EINVAL, "device out of range");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(DVBS2FEC_ENODEV, "no CUDA device");
+    if (device < 0 || device >= ndev) return fail(DVBS2FEC_EINVAL, "device out of range");
     std::unique_ptr<dvbs2fec_plsync> p(new dvbs2fec_plsync());
     p->device = device;
     if (const char* e = getenv("DVBS2FEC_PLL_MODE")) p->pll_sequential = (atoi(e) == 1 || atoi(e) == 2) ? atoi(e) : 0;      // A/B measurements
@@ -155,8 +116,7 @@ int dvbs2fec_plsync_create(int device, dvbs2fec_plsync** out) {
     CU(p->tab.reserve(1));
     std::unique_ptr<PlTables> t(new PlTables());
     build_tables(*t);
-    CU(cudaMemcpy(p->tab.p, t.get(), sizeof(PlTables), cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->tab.p, t.get(), sizeof(PlTables)));
     CU(cudaMemset(p->hst.p, 0, sizeof(PlHdrState)));
     CU(p->pst.reserve(1));
     CU(cudaMemset(p->pst.p, 0, sizeof(PllState)));
@@ -165,30 +125,17 @@ int dvbs2fec_plsync_create(int device, dvbs2fec_plsync** out) {
     return 0;
 }
 
-void dvbs2fec_plsync_destroy(dvbs2fec_plsync* p) {
-    if (!p) return;
-    cudaSetDevice(p->device);
-    if (p->stream) {
-        cudaStreamSynchronize(p->stream);
-        cudaStreamDestroy(p->stream);
-    }
-    p->work[0].release(); p->work[1].release(); p->out.release(); p->frames_in.release(); p->hdr_out.release();
-    p->metric.release(); p->fed_out.release(); p->starts.release(); p->st.release(); p->hst.release(); p->hres.release();
-    p->tab.release(); p->rn.release();
-    p->pst.release(); p->perr.release(); p->pll_state.release(); p->pll_in.release(); p->pll_out.release(); p->pll_rn.release();
-    p->pll_jobs.release();
-    delete p;
-}
+void dvbs2fec_plsync_destroy(dvbs2fec_plsync* p) { delete p; }
 
 int dvbs2fec_plsync_set_params(dvbs2fec_plsync* p, int slot_num, int pilots) {
-    if (!p || slot_num < 1 || slot_num > 4096) return api_fail(DVBS2FEC_EINVAL, "bad slot count");
+    if (!p || slot_num < 1 || slot_num > 4096) return fail(DVBS2FEC_EINVAL, "bad slot count");
     CU(cudaSetDevice(p->device));
     p->rfs = raw_frame_size(slot_num, pilots);
     return dvbs2fec_plsync_reset(p);
 }
 
 int dvbs2fec_plsync_reset(dvbs2fec_plsync* p) {
-    if (!p || !p->rfs) return api_fail(DVBS2FEC_EINVAL, "set_params has not been called");
+    if (!p || !p->rfs) return fail(DVBS2FEC_EINVAL, "set_params has not been called");
     CU(cudaSetDevice(p->device));
     // reset() (dvbs2_pl_sync.cpp:37-45) clears the gathering state; the public members keep their values
     PlSyncState s = p->h_st;
@@ -221,14 +168,14 @@ static int plsync_run(dvbs2fec_plsync* p, int count, const float2* d_append, flo
     a.st = p->st.p;
     a.nframes_out = d_nframes;
     int e = plsync_launch(a, p->pend_ub, st);
-    if (e) return api_fail(DVBS2FEC_ECUDA, cudaGetErrorString((cudaError_t)e));
+    if (e) return fail(DVBS2FEC_ECUDA, "%s", cudaGetErrorString((cudaError_t)e));
     p->cur ^= 1;
     return 0;
 }
 
 int dvbs2fec_plsync_process(dvbs2fec_plsync* p, int count, const float* in, float* out) {
-    if (!p || !p->rfs) return api_fail(DVBS2FEC_EINVAL, "set_params has not been called");
-    if (count < 0 || (count && !in) || !out) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs) return fail(DVBS2FEC_EINVAL, "set_params has not been called");
+    if (count < 0 || (count && !in) || !out) return fail(DVBS2FEC_EINVAL, "bad arguments");
     CU(cudaSetDevice(p->device));
     if (!p->pend_exact) {   // device-buffer calls came before: ask the device how many symbols it carries
         CU(cudaDeviceSynchronize());
@@ -257,8 +204,8 @@ int dvbs2fec_plsync_process(dvbs2fec_plsync* p, int count, const float* in, floa
 
 int dvbs2fec_plsync_process_device(dvbs2fec_plsync* p, int count, const float* d_in, float* d_out, int max_frames, int* d_nframes,
                                    void* stream) {
-    if (!p || !p->rfs) return api_fail(DVBS2FEC_EINVAL, "set_params has not been called");
-    if (count < 0 || (count && !d_in) || !d_out || max_frames < 0) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs) return fail(DVBS2FEC_EINVAL, "set_params has not been called");
+    if (count < 0 || (count && !d_in) || !d_out || max_frames < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
     // fewer than two frames are ever carried over: sized for that, the buffers only grow with the caller's block size
@@ -282,7 +229,7 @@ int dvbs2fec_plsync_process_device(dvbs2fec_plsync* p, int count, const float* d
 }
 
 int dvbs2fec_plsync_stats(dvbs2fec_plsync* p, int* current_position, double* best_match, int* pending) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     CU(cudaMemcpy(&p->h_st, p->st.p, sizeof(PlSyncState), cudaMemcpyDeviceToHost));
     if (current_position) *current_position = p->h_st.current_position;
@@ -292,7 +239,7 @@ int dvbs2fec_plsync_stats(dvbs2fec_plsync* p, int* current_position, double* bes
 }
 
 int dvbs2fec_plhdr_set_params(dvbs2fec_plsync* p, float loop_bw) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     // S2PLHDRDemod::init (dvbs2_plhdr_demod.cpp:5-12): criticallyDamped(loop_bw * 0.03f), phase = freq = 0
     PlHdrState s{};
@@ -301,24 +248,23 @@ int dvbs2fec_plhdr_set_params(dvbs2fec_plsync* p, float loop_bw) {
     const float den = (float)(1.0 + 2.0 * damp * bw + bw * bw);
     s.alpha = (4 * damp * bw) / den;
     s.beta = (4 * bw * bw) / den;
-    CU(cudaMemcpy(p->hst.p, &s, sizeof s, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->hst.p, &s, sizeof s));
     return 0;
 }
 
 int dvbs2fec_plhdr_process_device(dvbs2fec_plsync* p, int nframes, const float* d_frames, float* d_headers, int32_t* d_results,
                                   void* stream) {
-    if (!p || !p->rfs || nframes < 0 || (nframes && (!d_frames || !d_headers || !d_results))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs || nframes < 0 || (nframes && (!d_frames || !d_headers || !d_results))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     CU(cudaSetDevice(p->device));
     static_assert(sizeof(PlHdrResult) == 4 * sizeof(int32_t), "result record is four ints");
     int e = plhdr_launch(reinterpret_cast<const float2*>(d_frames), nframes, p->rfs, reinterpret_cast<float2*>(d_headers),
                          reinterpret_cast<PlHdrResult*>(d_results), p->hst.p, p->tab.p, (cudaStream_t)stream);
-    if (e) return api_fail(DVBS2FEC_ECUDA, cudaGetErrorString((cudaError_t)e));
+    if (e) return fail(DVBS2FEC_ECUDA, "%s", cudaGetErrorString((cudaError_t)e));
     return 0;
 }
 
 int dvbs2fec_plhdr_process(dvbs2fec_plsync* p, int nframes, const float* frames, float* headers, int32_t* results, float* loop_state) {
-    if (!p || !p->rfs || nframes < 0 || (nframes && (!frames || !headers || !results))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs || nframes < 0 || (nframes && (!frames || !headers || !results))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     CU(cudaSetDevice(p->device));
     CU(p->frames_in.reserve((size_t)std::max(nframes, 1) * p->rfs));
     CU(p->hdr_out.reserve((size_t)std::max(nframes, 1) * kPlHeader));
@@ -343,11 +289,10 @@ int dvbs2fec_plhdr_process(dvbs2fec_plsync* p, int nframes, const float* frames,
 
 static int fed_tables(dvbs2fec_plsync* p, int pilots, int codenum) {
     if (pilots && p->rn_codenum != codenum) {
-        if (codenum < 0 || codenum > 262141) return api_fail(DVBS2FEC_EINVAL, "Gold code number outside 0..262141");
+        if (codenum < 0 || codenum > 262141) return fail(DVBS2FEC_EINVAL, "Gold code number outside 0..262141");
         std::vector<uint8_t> rn = pl_scrambling_rn(codenum, 131072);
         CU(p->rn.reserve(rn.size()));
-        CU(cudaMemcpy(p->rn.p, rn.data(), rn.size(), cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+        CU(upload(p->rn.p, rn.data(), rn.size()));
         p->rn_codenum = codenum;
     }
     return 0;
@@ -355,17 +300,17 @@ static int fed_tables(dvbs2fec_plsync* p, int pilots, int codenum) {
 
 int dvbs2fec_coarse_fed_device(dvbs2fec_plsync* p, int nframes, const float* d_frames, int pilots, int pls_code, int codenum, float* d_err,
                                void* stream) {
-    if (!p || !p->rfs || nframes < 0 || (nframes && (!d_frames || !d_err))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs || nframes < 0 || (nframes && (!d_frames || !d_err))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     CU(cudaSetDevice(p->device));
     int rc = fed_tables(p, pilots, codenum);
     if (rc) return rc;
     int e = fed_launch(reinterpret_cast<const float2*>(d_frames), nframes, p->rfs, pilots, pls_code, p->rn.p, p->tab.p, d_err, (cudaStream_t)stream);
-    if (e) return api_fail(DVBS2FEC_ECUDA, cudaGetErrorString((cudaError_t)e));
+    if (e) return fail(DVBS2FEC_ECUDA, "%s", cudaGetErrorString((cudaError_t)e));
     return 0;
 }
 
 int dvbs2fec_coarse_fed(dvbs2fec_plsync* p, int nframes, const float* frames, int pilots, int pls_code, int codenum, float* err) {
-    if (!p || !p->rfs || nframes < 0 || (nframes && (!frames || !err))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs || nframes < 0 || (nframes && (!frames || !err))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!nframes) return 0;
     CU(cudaSetDevice(p->device));
     CU(p->frames_in.reserve((size_t)nframes * p->rfs));
@@ -380,16 +325,15 @@ int dvbs2fec_coarse_fed(dvbs2fec_plsync* p, int nframes, const float* frames, in
 
 // ---------------------------------------------------------------------------------------------- S2PLLBlock (K8)
 int dvbs2fec_pll_set_params(dvbs2fec_plsync* p, float loop_bw, int modcod, int shortframes, int pilots, int codenum) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     ModcodCfg cfg;
-    if (!modcod_config(modcod, shortframes != 0, pilots != 0, &cfg)) return api_fail(DVBS2FEC_EINVAL, "modcod outside 1..28");
-    if (codenum < 0 || codenum > 262141) return api_fail(DVBS2FEC_EINVAL, "Gold code number outside 0..262141");
+    if (!modcod_config(modcod, shortframes != 0, pilots != 0, &cfg)) return fail(DVBS2FEC_EINVAL, "modcod outside 1..28");
+    if (codenum < 0 || codenum > 262141) return fail(DVBS2FEC_EINVAL, "Gold code number outside 0..262141");
     CU(cudaSetDevice(p->device));
     {   // the loop descrambles every payload symbol, pilots or not
         const std::vector<uint8_t> rn = pl_scrambling_rn(codenum, 131072);
         CU(p->pll_rn.reserve(rn.size()));
-        CU(cudaMemcpy(p->pll_rn.p, rn.data(), rn.size(), cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+        CU(upload(p->pll_rn.p, rn.data(), rn.size()));
     }
     // PhaseControlLoop<float>::criticallyDamped(loop_bw, alpha, beta) (dvbs2_pll.cpp:10)
     PllState s{};
@@ -399,8 +343,7 @@ int dvbs2fec_pll_set_params(dvbs2fec_plsync* p, float loop_bw, int modcod, int s
     const float den = (float)(1.0 + 2.0 * damp * bw + bw * bw);
     s.alpha = (4 * damp * bw) / den;
     s.beta = (4 * bw * bw) / den;
-    CU(cudaMemcpy(p->pst.p, &s, sizeof s, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->pst.p, &s, sizeof s));
     PllArgs& a = p->pll;
     a = PllArgs{};
     a.pilot_cnt = 0;
@@ -427,8 +370,7 @@ int dvbs2fec_pll_set_params(dvbs2fec_plsync* p, float loop_bw, int modcod, int s
     if (cfg.constellation != APSK32) {   // the reference has no table for 32APSK (constellation.cpp:294,319-321)
         const std::vector<float> lut = demap_phase_lut(c);
         CU(p->perr.reserve(lut.size()));
-        CU(cudaMemcpy(p->perr.p, lut.data(), lut.size() * sizeof(float), cudaMemcpyHostToDevice));
-        CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+        CU(upload(p->perr.p, lut.data(), lut.size() * sizeof(float)));
         a.perr_lut = p->perr.p;
     }
     a.rn = p->pll_rn.p;
@@ -439,31 +381,29 @@ int dvbs2fec_pll_set_params(dvbs2fec_plsync* p, float loop_bw, int modcod, int s
 }
 
 int dvbs2fec_pll_reset(dvbs2fec_plsync* p) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     PllState s{};
     CU(cudaMemcpy(&s, p->pst.p, sizeof s, cudaMemcpyDeviceToHost));
     s.phase = 0;
     s.freq = 0;
-    CU(cudaMemcpy(p->pst.p, &s, sizeof s, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->pst.p, &s, sizeof s));
     return 0;
 }
 
 int dvbs2fec_pll_set_state(dvbs2fec_plsync* p, float phase, float freq) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     PllState s{};
     CU(cudaMemcpy(&s, p->pst.p, sizeof s, cudaMemcpyDeviceToHost));
     s.phase = phase;
     s.freq = freq;
-    CU(cudaMemcpy(p->pst.p, &s, sizeof s, cudaMemcpyHostToDevice));
-    CU(cudaStreamSynchronize(nullptr));      // (a pageable copy returns once staged; non-blocking streams do not wait for the default stream)
+    CU(upload(p->pst.p, &s, sizeof s));
     return 0;
 }
 
 int dvbs2fec_pll_set_sequential(dvbs2fec_plsync* p, int on) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     p->pll_sequential = (on == 1 || on == 2) ? on : 0;
     return 0;
 }
@@ -472,8 +412,8 @@ int dvbs2fec_pll_frame_symbols(const dvbs2fec_plsync* p) { return (p && p->pll_r
 
 int dvbs2fec_pll_process_device(dvbs2fec_plsync* p, int nframes, int frame_stride, const float* d_frames, float* d_out, float* d_state,
                                 void* stream) {
-    if (!p || !p->pll_ready) return api_fail(DVBS2FEC_EINVAL, "dvbs2fec_pll_set_params has not been called");
-    if (nframes < 0 || frame_stride < p->pll.total || (nframes && (!d_frames || !d_out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->pll_ready) return fail(DVBS2FEC_EINVAL, "dvbs2fec_pll_set_params has not been called");
+    if (nframes < 0 || frame_stride < p->pll.total || (nframes && (!d_frames || !d_out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     CU(cudaSetDevice(p->device));
     PllArgs a = p->pll;
     a.frames = reinterpret_cast<const float2*>(d_frames);
@@ -482,13 +422,13 @@ int dvbs2fec_pll_process_device(dvbs2fec_plsync* p, int nframes, int frame_strid
     a.rfs = frame_stride;
     a.state_out = d_state;
     int e = pll_launch(a, p->pll_sequential, (cudaStream_t)stream);
-    if (e) return api_fail(DVBS2FEC_ECUDA, cudaGetErrorString((cudaError_t)e));
+    if (e) return fail(DVBS2FEC_ECUDA, "%s", cudaGetErrorString((cudaError_t)e));
     return 0;
 }
 
 int dvbs2fec_pll_process(dvbs2fec_plsync* p, int nframes, int frame_stride, const float* frames, float* out, float* state) {
-    if (!p || !p->pll_ready) return api_fail(DVBS2FEC_EINVAL, "dvbs2fec_pll_set_params has not been called");
-    if (nframes < 0 || frame_stride < p->pll.total || (nframes && (!frames || !out))) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->pll_ready) return fail(DVBS2FEC_EINVAL, "dvbs2fec_pll_set_params has not been called");
+    if (nframes < 0 || frame_stride < p->pll.total || (nframes && (!frames || !out))) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if (!nframes) return 0;
     CU(cudaSetDevice(p->device));
     const size_t n = (size_t)nframes * frame_stride;
@@ -509,12 +449,12 @@ int dvbs2fec_pll_process(dvbs2fec_plsync* p, int nframes, int frame_stride, cons
 
 int dvbs2fec_pll_process_multi_device(int nstreams, dvbs2fec_plsync* const* objs, int nframes, int frame_stride,
                                       const float* const* d_frames, float* const* d_out, void* stream) {
-    if (nstreams < 1 || nstreams > 4096 || !objs || !d_frames || !d_out || nframes < 0) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (nstreams < 1 || nstreams > 4096 || !objs || !d_frames || !d_out || nframes < 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
     std::vector<PllArgs> jobs((size_t)nstreams);
     for (int k = 0; k < nstreams; ++k) {
         dvbs2fec_plsync* p = objs[k];
         if (!p || !p->pll_ready || p->device != objs[0]->device || frame_stride < p->pll.total || !d_frames[k] || !d_out[k])
-            return api_fail(DVBS2FEC_EINVAL, "stream not configured, on another device, or stride shorter than its frame");
+            return fail(DVBS2FEC_EINVAL, "stream not configured, on another device, or stride shorter than its frame");
         PllArgs a = p->pll;
         a.frames = reinterpret_cast<const float2*>(d_frames[k]);
         a.out = reinterpret_cast<float2*>(d_out[k]);
@@ -533,12 +473,12 @@ int dvbs2fec_pll_process_multi_device(int nstreams, dvbs2fec_plsync* const* objs
     CU(cudaMemcpyAsync(p0->pll_jobs.p, jobs.data(), jobs.size() * sizeof(PllArgs), cudaMemcpyHostToDevice, st));
     CU(cudaStreamSynchronize(st));   // `jobs` is pageable host memory
     int e = pll_launch_multi(reinterpret_cast<const PllArgs*>(p0->pll_jobs.p), nstreams, st);
-    if (e) return api_fail(DVBS2FEC_ECUDA, cudaGetErrorString((cudaError_t)e));
+    if (e) return fail(DVBS2FEC_ECUDA, "%s", cudaGetErrorString((cudaError_t)e));
     return 0;
 }
 
 int dvbs2fec_pll_rounds(dvbs2fec_plsync* p) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     CU(cudaSetDevice(p->device));
     PllState s{};
     CU(cudaMemcpy(&s, p->pst.p, sizeof s, cudaMemcpyDeviceToHost));

@@ -10,39 +10,13 @@
 #include "../../include/dvbs2fec.h"
 
 #include <algorithm>
-#include <cstdio>
 #include <memory>
 
 #include <cuda_runtime.h>
 
-namespace s2 {
-int api_fail(int code, const char* msg);
-}
-using s2::api_fail;
+#include "abi_util.h"
 
-namespace {
-int failf(int code, const char* what, cudaError_t e) {
-    char buf[300];
-    snprintf(buf, sizeof buf, "%s: %s", what, cudaGetErrorString(e));
-    return api_fail(code, buf);
-}
-#define CU(call)                                                     \
-    do {                                                             \
-        cudaError_t e_ = (call);                                     \
-        if (e_ != cudaSuccess) return failf(DVBS2FEC_ECUDA, #call, e_); \
-    } while (0)
-
-template <typename T>
-cudaError_t reserve(T*& p, size_t& cap, size_t n) {
-    if (n <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-    cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-    if (e == cudaSuccess) cap = n;
-    return e;
-}
-}  // namespace
+using namespace s2;
 
 struct dvbs2fec_s2_demod {
     int device = 0;
@@ -51,46 +25,38 @@ struct dvbs2fec_s2_demod {
     dvbs2fec_ts_parser* ts = nullptr;      // BBFRAME -> TS / GSE (K6), for dvbs2fec_s2_demod_process_ts
     cudaStream_t stream = nullptr;
     int modcod = 0, shortframes = 0, pilots = 0, codenum = 0, rfs = 0, kb = 0;
-    float* d_x = nullptr; size_t x_cap = 0;
-    float* d_fr = nullptr; size_t fr_cap = 0;
-    float* d_pl = nullptr; size_t pl_cap = 0;
-    float* d_hsym = nullptr; size_t hsym_cap = 0;
-    uint8_t* d_bb = nullptr; size_t bb_cap = 0;
-    dvbs2fec_result* d_res = nullptr; size_t res_cap = 0;
-    float* d_fed = nullptr; size_t fed_cap = 0;
-    int32_t* d_hdr = nullptr; size_t hdr_cap = 0;
-    uint8_t* d_ts = nullptr; size_t ts_cap = 0;
-    int* d_n = nullptr;
+    DevBuf<float> d_x, d_fr, d_pl, d_hsym, d_fed;
+    DevBuf<uint8_t> d_bb, d_ts;
+    DevBuf<dvbs2fec_result> d_res;
+    DevBuf<int32_t> d_hdr;
+    DevBuf<int> d_n;
     int last_frames = 0;
+    ~dvbs2fec_s2_demod() {
+        cudaSetDevice(device);
+        if (stream) {
+            cudaStreamSynchronize(stream);
+            cudaStreamDestroy(stream);
+        }
+        dvbs2fec_plsync_destroy(pl);
+        dvbs2fec_ts_destroy(ts);
+        dvbs2fec_destroy(fec);
+    }
 };
 
 extern "C" {
 
-void dvbs2fec_s2_demod_destroy(dvbs2fec_s2_demod* p) {
-    if (!p) return;
-    cudaSetDevice(p->device);
-    if (p->stream) {
-        cudaStreamSynchronize(p->stream);
-        cudaStreamDestroy(p->stream);
-    }
-    dvbs2fec_plsync_destroy(p->pl);
-    dvbs2fec_ts_destroy(p->ts);
-    dvbs2fec_destroy(p->fec);
-    cudaFree(p->d_x); cudaFree(p->d_fr); cudaFree(p->d_pl); cudaFree(p->d_hsym); cudaFree(p->d_bb); cudaFree(p->d_res);
-    cudaFree(p->d_fed); cudaFree(p->d_hdr); cudaFree(p->d_ts); cudaFree(p->d_n);
-    delete p;
-}
+void dvbs2fec_s2_demod_destroy(dvbs2fec_s2_demod* p) { delete p; }
 
 int dvbs2fec_s2_demod_create(const dvbs2fec_config* cfg, dvbs2fec_s2_demod** out) {
-    if (!out) return api_fail(DVBS2FEC_EINVAL, "out is NULL");
+    if (!out) return fail(DVBS2FEC_EINVAL, "out is NULL");
     *out = nullptr;
-    std::unique_ptr<dvbs2fec_s2_demod, void (*)(dvbs2fec_s2_demod*)> p(new dvbs2fec_s2_demod(), dvbs2fec_s2_demod_destroy);
+    std::unique_ptr<dvbs2fec_s2_demod> p(new dvbs2fec_s2_demod());
     dvbs2fec_config c{};
     if (cfg) c = *cfg;
-    if (c.n_devices > 1) return api_fail(DVBS2FEC_EINVAL, "one stream of symbols is a recurrence (PL sync, phase loops): one device");
+    if (c.n_devices > 1) return fail(DVBS2FEC_EINVAL, "one stream of symbols is a recurrence (PL sync, phase loops): one device");
     int dev = 0;
     if (c.n_devices == 1) dev = c.devices[0];
-    else if (cudaGetDevice(&dev) != cudaSuccess) return api_fail(DVBS2FEC_ENODEV, "no CUDA device");
+    else if (cudaGetDevice(&dev) != cudaSuccess) return fail(DVBS2FEC_ENODEV, "no CUDA device");
     c.n_devices = 1;
     c.devices[0] = dev;
     if (c.max_batch <= 0) c.max_batch = 1024;
@@ -101,14 +67,14 @@ int dvbs2fec_s2_demod_create(const dvbs2fec_config* cfg, dvbs2fec_s2_demod** out
     if (rc) return rc;
     CU(cudaSetDevice(dev));
     CU(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
-    CU(cudaMalloc(&p->d_n, sizeof(int)));
+    CU(p->d_n.reserve(1));
     *out = p.release();
     return 0;
 }
 
 int dvbs2fec_s2_demod_set_params(dvbs2fec_s2_demod* p, int modcod, int shortframes, int pilots, int max_trials, float pll_loop_bw,
                                  float plhdr_loop_bw, int codenum) {
-    if (!p) return api_fail(DVBS2FEC_EINVAL, "handle is NULL");
+    if (!p) return fail(DVBS2FEC_EINVAL, "handle is NULL");
     int nldpc = 0, bits = 0, plsyms = 0;
     int rc = dvbs2fec_modcod_info(modcod, shortframes, pilots, &nldpc, nullptr, nullptr, nullptr, &bits, &plsyms, nullptr);
     if (rc) return rc;
@@ -125,12 +91,12 @@ int dvbs2fec_s2_demod_set_params(dvbs2fec_s2_demod* p, int modcod, int shortfram
     p->kb = dvbs2fec_kbch(p->fec) / 8;
     rc = dvbs2fec_ts_set_frame_size(p->ts, p->kb * 8);      // BBFrameTSParser::setFrameSize (main.cpp, on a MODCOD change)
     if (rc) return rc;
-    if (p->rfs != plsyms || dvbs2fec_pll_frame_symbols(p->pl) > p->rfs) return api_fail(DVBS2FEC_EINVAL, "frame sizes of the stages disagree");
+    if (p->rfs != plsyms || dvbs2fec_pll_frame_symbols(p->pl) > p->rfs) return fail(DVBS2FEC_EINVAL, "frame sizes of the stages disagree");
     return 0;
 }
 
 int dvbs2fec_s2_demod_reset(dvbs2fec_s2_demod* p) {
-    if (!p || !p->rfs) return api_fail(DVBS2FEC_EINVAL, "set_params has not been called");
+    if (!p || !p->rfs) return fail(DVBS2FEC_EINVAL, "set_params has not been called");
     CU(cudaSetDevice(p->device));
     CU(cudaStreamSynchronize(p->stream));
     int rc = dvbs2fec_plsync_reset(p->pl);
@@ -151,38 +117,38 @@ int stage_to_device(dvbs2fec_s2_demod* p, int count, const float* syms) {
     CU(cudaSetDevice(p->device));
     cudaStream_t st = p->stream;
     const size_t fsz = (size_t)room * p->rfs * 2;
-    CU(reserve(p->d_x, p->x_cap, (size_t)2 * count));
-    CU(reserve(p->d_fr, p->fr_cap, fsz));
-    if (fsz > p->pl_cap) {
-        CU(reserve(p->d_pl, p->pl_cap, fsz));
-        CU(cudaMemsetAsync(p->d_pl, 0, fsz * sizeof(float), st));      // symbols behind the ones the loop handles are never written
+    CU(p->d_x.reserve((size_t)2 * count));
+    CU(p->d_fr.reserve(fsz));
+    if (fsz > p->d_pl.cap) {
+        CU(p->d_pl.reserve(fsz));
+        CU(cudaMemsetAsync(p->d_pl.p, 0, fsz * sizeof(float), st));      // symbols behind the ones the loop handles are never written
     }
-    CU(reserve(p->d_hsym, p->hsym_cap, (size_t)room * 180));
-    CU(reserve(p->d_bb, p->bb_cap, (size_t)room * p->kb));
-    CU(reserve(p->d_res, p->res_cap, (size_t)room));
-    CU(reserve(p->d_fed, p->fed_cap, (size_t)room));
-    CU(reserve(p->d_hdr, p->hdr_cap, (size_t)room * 4));
-    CU(cudaMemcpyAsync(p->d_x, syms, sizeof(float) * 2 * count, cudaMemcpyHostToDevice, st));
-    int rc = dvbs2fec_plsync_process_device(p->pl, count, p->d_x, p->d_fr, room, p->d_n, st);      // :300
+    CU(p->d_hsym.reserve((size_t)room * 180));
+    CU(p->d_bb.reserve((size_t)room * p->kb));
+    CU(p->d_res.reserve((size_t)room));
+    CU(p->d_fed.reserve((size_t)room));
+    CU(p->d_hdr.reserve((size_t)room * 4));
+    CU(cudaMemcpyAsync(p->d_x.p, syms, sizeof(float) * 2 * count, cudaMemcpyHostToDevice, st));
+    int rc = dvbs2fec_plsync_process_device(p->pl, count, p->d_x.p, p->d_fr.p, room, p->d_n.p, st);      // :300
     if (rc) return rc;
     int n = 0;
-    CU(cudaMemcpyAsync(&n, p->d_n, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&n, p->d_n.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (n <= 0) return 0;
     const int pls_code = p->modcod << 2 | p->shortframes << 1 | p->pilots;
-    rc = dvbs2fec_coarse_fed_device(p->pl, n, p->d_fr, p->pilots, pls_code, p->codenum, p->d_fed, st);      // :302
-    if (!rc) rc = dvbs2fec_pll_process_device(p->pl, n, p->rfs, p->d_fr, p->d_pl, nullptr, st);             // :314
-    if (!rc) rc = dvbs2fec_plhdr_process_device(p->pl, n, p->d_fr, p->d_hsym, p->d_hdr, st);                // :315
-    if (!rc) rc = dvbs2fec_decode_plframes_device(p->fec, p->d_pl, n, p->d_bb, p->d_res, st);               // :316, 334-366
+    rc = dvbs2fec_coarse_fed_device(p->pl, n, p->d_fr.p, p->pilots, pls_code, p->codenum, p->d_fed.p, st);      // :302
+    if (!rc) rc = dvbs2fec_pll_process_device(p->pl, n, p->rfs, p->d_fr.p, p->d_pl.p, nullptr, st);             // :314
+    if (!rc) rc = dvbs2fec_plhdr_process_device(p->pl, n, p->d_fr.p, p->d_hsym.p, p->d_hdr.p, st);                // :315
+    if (!rc) rc = dvbs2fec_decode_plframes_device(p->fec, p->d_pl.p, n, p->d_bb.p, p->d_res.p, st);               // :316, 334-366
     if (rc) return rc;
     return n;
 }
 
 int copy_side_outputs(dvbs2fec_s2_demod* p, int n, dvbs2fec_result* results, float* fed_err, int32_t* plhdr) {
     cudaStream_t st = p->stream;
-    if (results) CU(cudaMemcpyAsync(results, p->d_res, sizeof(dvbs2fec_result) * n, cudaMemcpyDeviceToHost, st));
-    if (fed_err) CU(cudaMemcpyAsync(fed_err, p->d_fed, sizeof(float) * n, cudaMemcpyDeviceToHost, st));
-    if (plhdr) CU(cudaMemcpyAsync(plhdr, p->d_hdr, sizeof(int32_t) * 4 * n, cudaMemcpyDeviceToHost, st));
+    if (results) CU(cudaMemcpyAsync(results, p->d_res.p, sizeof(dvbs2fec_result) * n, cudaMemcpyDeviceToHost, st));
+    if (fed_err) CU(cudaMemcpyAsync(fed_err, p->d_fed.p, sizeof(float) * n, cudaMemcpyDeviceToHost, st));
+    if (plhdr) CU(cudaMemcpyAsync(plhdr, p->d_hdr.p, sizeof(int32_t) * 4 * n, cudaMemcpyDeviceToHost, st));
     return 0;
 }
 }  // namespace
@@ -191,14 +157,14 @@ extern "C" {
 
 int dvbs2fec_s2_demod_process(dvbs2fec_s2_demod* p, int count, const float* syms, uint8_t* bb_out, int max_frames, dvbs2fec_result* results,
                               float* fed_err, int32_t* plhdr) {
-    if (!p || !p->rfs) return api_fail(DVBS2FEC_EINVAL, "set_params has not been called");
-    if (count < 0 || (count && !syms) || !bb_out) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
-    if (max_frames < count / p->rfs + 2) return api_fail(DVBS2FEC_EINVAL, "max_frames < count / raw_frame_size + 2 (dvbs2fec_s2_demod_max_frames)");
+    if (!p || !p->rfs) return fail(DVBS2FEC_EINVAL, "set_params has not been called");
+    if (count < 0 || (count && !syms) || !bb_out) return fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (max_frames < count / p->rfs + 2) return fail(DVBS2FEC_EINVAL, "max_frames < count / raw_frame_size + 2 (dvbs2fec_s2_demod_max_frames)");
     if (!count) return 0;
     const int n = stage_to_device(p, count, syms);
     if (n <= 0) return n;
     cudaStream_t st = p->stream;
-    CU(cudaMemcpyAsync(bb_out, p->d_bb, (size_t)n * p->kb, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(bb_out, p->d_bb.p, (size_t)n * p->kb, cudaMemcpyDeviceToHost, st));
     int rc = copy_side_outputs(p, n, results, fed_err, plhdr);
     if (rc) return rc;
     CU(cudaStreamSynchronize(st));
@@ -207,27 +173,27 @@ int dvbs2fec_s2_demod_process(dvbs2fec_s2_demod* p, int count, const float* syms
 
 int dvbs2fec_s2_demod_process_ts(dvbs2fec_s2_demod* p, int count, const float* syms, uint8_t* ts_out, int ts_cap, int max_frames, int* nframes,
                                  dvbs2fec_result* results, float* fed_err, int32_t* plhdr) {
-    if (!p || !p->rfs) return api_fail(DVBS2FEC_EINVAL, "set_params has not been called");
-    if (count < 0 || (count && !syms) || !ts_out || ts_cap <= 0) return api_fail(DVBS2FEC_EINVAL, "bad arguments");
+    if (!p || !p->rfs) return fail(DVBS2FEC_EINVAL, "set_params has not been called");
+    if (count < 0 || (count && !syms) || !ts_out || ts_cap <= 0) return fail(DVBS2FEC_EINVAL, "bad arguments");
     if ((results || fed_err || plhdr) && max_frames < count / p->rfs + 2)
-        return api_fail(DVBS2FEC_EINVAL, "max_frames < count / raw_frame_size + 2 (dvbs2fec_s2_demod_max_frames)");
+        return fail(DVBS2FEC_EINVAL, "max_frames < count / raw_frame_size + 2 (dvbs2fec_s2_demod_max_frames)");
     if (nframes) *nframes = 0;
     if (!count) return 0;
     const int n = stage_to_device(p, count, syms);
     if (n <= 0) return n;
     if (nframes) *nframes = n;
     cudaStream_t st = p->stream;
-    CU(reserve(p->d_ts, p->ts_cap, (size_t)ts_cap));
-    int rc = dvbs2fec_ts_work_device(p->ts, p->d_bb, n, p->d_ts, ts_cap, p->d_n, st);      // main.cpp:538: ts_parser.work(...)
+    CU(p->d_ts.reserve((size_t)ts_cap));
+    int rc = dvbs2fec_ts_work_device(p->ts, p->d_bb.p, n, p->d_ts.p, ts_cap, p->d_n.p, st);      // main.cpp:538: ts_parser.work(...)
     if (rc) return rc;
     int produced = 0;
-    CU(cudaMemcpyAsync(&produced, p->d_n, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&produced, p->d_n.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     rc = copy_side_outputs(p, n, results, fed_err, plhdr);
     if (rc) return rc;
     CU(cudaStreamSynchronize(st));
-    if (produced < 0) return api_fail(produced, "TS / GSE output does not fit ts_cap");
+    if (produced < 0) return fail(produced, "TS / GSE output does not fit ts_cap");
     if (produced) {
-        CU(cudaMemcpyAsync(ts_out, p->d_ts, (size_t)produced, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(ts_out, p->d_ts.p, (size_t)produced, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
     }
     return produced;

@@ -178,4 +178,9 @@ bool modcod_config(int modcod, bool shortframes, bool pilots, ModcodCfg* out) {
     return true;
 }
 
+int plframe_symbols(const ModcodCfg& mc) {
+    const int nsym = mc.slots * 90;
+    return 90 + nsym + (mc.pilots ? 36 * ((nsym - 1) / 1440) : 0);
+}
+
 }  // namespace s2

@@ -32,6 +32,9 @@ struct ModcodCfg {
 };
 // false for modcod outside 1..28 (the reference throws, modcod_to_cfg.cpp:10-11,134-135)
 bool modcod_config(int modcod, bool shortframes, bool pilots, ModcodCfg* out);
+// complex samples of a PLFRAME of this configuration: PLHEADER, payload and (with pilots) a pilot block of 36 after
+// every 16 slots but the last
+int plframe_symbols(const ModcodCfg& mc);
 
 struct LayerLink {
     uint16_t group;  // data-bit group g: bits 360g .. 360g+359
